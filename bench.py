@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""bench.py — one JSON line for the MeShClust2 hot path on B200 (contract in the task prompt / DESIGN.md §Measurement).
+"""bench.py — one JSON line for the MeShClust2 hot path on B200 (DESIGN.md §Measurement).
 
 A step = one pass of the hot path over one batch of synthetic mutated-template DNA:
     K1  k-mer histograms of every sequence (Loader<T>::get_point), then
@@ -11,10 +11,13 @@ N > 1: one process per GPU (torchrun); sequences sharded for K1, histogram shard
 split by folded query-row blocks; total work fixed ("strong" scaling).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg3|cfg2|cfg4|cfg5] [--n-seqs N]
+                  [--dump-outputs DIR]
 
 --workload cfg4 / cfg5 print the same kind of line for BASELINE configs[3] (long records, k=8, uint16) and configs[4]
 (1M x 1 kb candidate scans + one update / merge pass, sharded over the ranks); the default cfg3 run carries both as
-`also_cfg4` / `also_cfg5` blocks so that the driver's own run times them.
+`also_cfg4` / `also_cfg5` blocks so that the default run times them.
+--dump-outputs DIR writes what the last timed step computed as DIR/<name>.npy (dump_outputs; cfg5: dump_scan_outputs), so
+that two builds can be compared output for output on the same seeded inputs.
 """
 import argparse
 import json
@@ -268,8 +271,11 @@ def run_ours(args, rank, world, local_rank):
         ctx = capi.Context(local_rank)
         model = ctx.model_from_file(WEIGHTS)
         peak, peak_src = peaks()
+        dump = {} if args.dump_outputs else None
         blk = cfg5_block(ctx, capi, mdist, torch, comm, model, model.meta["id"], local_rank, peak, n_total=n_total,
-                         n_queries=16 * args.steps)
+                         n_queries=16 * args.steps, dump=dump)
+        if dump is not None:
+            dump_scan_outputs(args.dump_outputs, dump, comm)
         cs = blk["candidate_scan"]
         line = {"metric": METRIC, "value": cs["pairs_per_s"], "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": 4,
                 "ms_per_step": cs["ms_per_query"] * 16, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
@@ -349,6 +355,8 @@ def run_ours(args, rank, world, local_rank):
     for _ in range(args.warmup):
         res = step_resident()
     ms, res, launches, ktime, clocks = timed(step_resident, args.steps, sample_clocks=True)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res, eng, n_total, comm)
     n_scored = res["n_scored"]
     value = n_scored * args.steps / (ms * 1e-3)
     log("[bench] rank %d per-kind device ms per step: %s" % (rank, {kk: round(v[0] / args.steps, 3) for kk, v in ktime.items()}))
@@ -492,6 +500,93 @@ def pin_inputs(capi, enc):
             except capi.Mc2Error as e:          # e.g. a locked-memory limit: the copies still work, just through pageable memory
                 log("[bench] could not page-lock %s: %s" % (key, e))
     return done
+
+
+DUMP_MAX_SURVIVORS = 1 << 21        # three float64 arrays: 48 MiB
+DUMP_HIST_BYTES = 8 << 20           # the float32 histogram sample
+
+
+def _pair_sample(a, b, cap):
+    """The pairs (a[i], b[i]) in (a, b) order: all of them up to cap, above it a fixed sample, the pairs whose splitmix64
+    hash has its top `shift` bits clear, with the smallest shift that brings the expected count to 3/4 of cap.  Whether a
+    pair is kept depends on the pair alone, so two builds that differ in one pair differ in that pair only (unless their
+    pair counts fall on two sides of cap or of a halving step).  Returns (indices into a / b, shift)."""
+    shift = 0
+    while len(a) > cap and (len(a) >> shift) > cap * 3 // 4:
+        shift += 1
+    keep = np.arange(len(a))
+    if shift:
+        with np.errstate(over="ignore"):
+            h = a.astype(np.uint64) * np.uint64(0x9E3779B97F4A7C15) ^ b.astype(np.uint64)
+            h ^= h >> np.uint64(30)
+            h *= np.uint64(0xBF58476D1CE4E5B9)
+            h ^= h >> np.uint64(27)
+            h *= np.uint64(0x94D049BB133111EB)
+            h ^= h >> np.uint64(31)
+        keep = np.flatnonzero((h >> np.uint64(64 - shift)) == 0)
+    return keep[np.lexsort((b[keep], a[keep]))], shift
+
+
+def _save_outputs(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float32 if name == "hist" else np.float64))
+
+
+def dump_outputs(out_dir, res, eng, n_total, comm):
+    """--dump-outputs, all-pairs workloads: what the last timed step computed, as out_dir/<name>.npy, float64 unless noted
+    (56 MiB at most):
+      survivor_q, survivor_d, survivor_score   the survivor pairs of every rank and their scores, in (q, d) order; above
+                                               DUMP_MAX_SURVIVORS pairs the fixed hash sample of _pair_sample
+      counts                                   [pairs scored, pairs close, survivors returned, sample shift]
+      hist_rows, hist (float32), hist_mag, hist_len
+                                               32 fixed seeded runs of consecutive k-mer histogram rows of the step, with
+                                               the rows' magnitudes and lengths
+    Runs before the next step: the survivors are views of buffers the engine reuses."""
+    surv = res["survivors"]
+    qd = surv.array()
+    q, d, score = qd[:, 0], qd[:, 1], surv.scores()
+    if comm.dist is not None:
+        parts = [None] * comm.world
+        comm.dist.all_gather_object(parts, (q, d, score))
+        q, d, score = (np.concatenate([p[i] for p in parts]) for i in range(3))
+    if comm.rank != 0:
+        return
+    order, shift = _pair_sample(q, d, DUMP_MAX_SURVIVORS)
+    want = min(n_total, max(1, DUMP_HIST_BYTES // (4 * eng.N)))
+    run = max(1, want // 32)
+    starts = np.sort(np.random.default_rng(1).choice(n_total // run, want // run, replace=False)) * run
+    got = [eng.full.download(int(a), run) for a in starts]
+    _save_outputs(out_dir, {"survivor_q": q[order], "survivor_d": d[order], "survivor_score": score[order],
+                            "counts": [res["n_scored"], res["n_close"], len(q), shift],
+                            "hist_rows": np.concatenate([np.arange(a, a + run) for a in starts]),
+                            "hist": np.concatenate([g["hist"] for g in got]),
+                            "hist_mag": np.concatenate([g["mag"] for g in got]),
+                            "hist_len": np.concatenate([g["len"] for g in got])})
+    log("[bench] last step's outputs written to %s (%d of %d survivors, %d histogram rows)" % (
+        out_dir, len(order), len(q), len(starts) * run))
+
+
+def dump_scan_outputs(out_dir, dump, comm):
+    """--dump-outputs, cfg5: what the last timed step computed, as out_dir/<name>.npy, all float64 (48 MiB at most):
+      scan_q, scan_best, scan_best_dist, scan_is_min   the step's 16 get_close scans: query row, arg-max row (-1: none), its
+                                                       distance, whether no candidate was close
+      mark_q, mark_candidate                           the (query, candidate) pairs the scans marked close, every rank's, in
+                                                       that order; above DUMP_MAX_SURVIVORS the hash sample of
+                                                       _pair_sample
+      counts                                           [pairs marked, sample shift]
+      update_next, update_n_good, merge_choice         the timed update + merge pass (-1 / 0: none)"""
+    mq, mc = dump.pop("marks")
+    if comm.dist is not None:
+        parts = [None] * comm.world
+        comm.dist.all_gather_object(parts, (mq, mc))
+        mq, mc = np.concatenate([p[0] for p in parts]), np.concatenate([p[1] for p in parts])
+    if comm.rank != 0:
+        return
+    order, shift = _pair_sample(mq, mc, DUMP_MAX_SURVIVORS)
+    dump.update(mark_q=mq[order], mark_candidate=mc[order], counts=[len(mq), shift])
+    _save_outputs(out_dir, dump)
+    log("[bench] last step's outputs written to %s (%d of %d marks)" % (out_dir, len(order), len(mq)))
 
 
 def small_workload(ctx, capi, mdist, torch, model, cutoff, steps=20):
@@ -660,12 +755,13 @@ def cfg4_block(ctx, capi, model, cutoff, peak, probe=None, n=5000):
     return out
 
 
-def cfg5_block(ctx, capi, mdist, torch, comm, model, cutoff, local_rank, peak, n_total=1000000, n_queries=64, delta=5):
+def cfg5_block(ctx, capi, mdist, torch, comm, model, cutoff, local_rank, peak, n_total=1000000, n_queries=64, delta=5, dump=None):
     """BASELINE configs[4] in the same run: 1M x 1 kb (k = 5, uint8) histograms RANGE-PARTITIONED over the ranks (1 GiB in
     all), Trainer::get_close candidate scans of the accumulate stage (the query row broadcast from its owner, every rank
     scanning its shard with mc2_get_close, one triple per rank combined) and one update + merge pass of the update stage at
     --delta 5 over the replicated set (mc2_update_centers / mc2_merge_centers, centers split over the ranks).
-    Histograms are generated directly (template rows + noise), bypassing FASTA, as SURVEY 8(d) allows for pair kernels."""
+    Histograms are generated directly (template rows + noise), bypassing FASTA, as SURVEY 8(d) allows for pair kernels.
+    dump: a dict to receive the results of the last 16 scans and of the update pass (dump_scan_outputs)."""
     world, rank = comm.world, comm.rank
     per, bounds = mdist.shard_bounds(n_total, world)
     lo, hi = bounds[rank]
@@ -691,12 +787,29 @@ def cfg5_block(ctx, capi, mdist, torch, comm, model, cutoff, local_rank, peak, n
     torch.cuda.synchronize()
     t0 = time.perf_counter()
     n_close = 0
+    timed_best = []
     for q in qs:
         r = mdist.candidate_scan(eng, comm, torch, q, n_total, cutoff)
         n_close += int(np.count_nonzero(r["marks_local"]))
+        if dump is not None:
+            timed_best.append((r["best"], r["best_dist"], r["is_min"]))
     torch.cuda.synchronize()
     comm.barrier()
     dt = comm.all_reduce_max(time.perf_counter() - t0, torch, eng.device)
+    if dump is not None:
+        # a scan reuses its mark buffer, so the marks of the last step's scans come from scanning those queries again,
+        # untimed; each repeat must return what the timed scan returned
+        last = qs[-16:]
+        mq, mc = [], []
+        for t, q in enumerate(last):
+            r = mdist.candidate_scan(eng, comm, torch, q, n_total, cutoff)
+            assert (r["best"], r["best_dist"], r["is_min"]) == timed_best[len(qs) - len(last) + t], "get_close scan not repeatable"
+            c = np.flatnonzero(r["marks_local"]) + lo
+            mq.append(np.full(len(c), q))
+            mc.append(c)
+        got = timed_best[len(qs) - len(last):]
+        dump.update(scan_q=last, scan_best=[g[0] for g in got], scan_best_dist=[g[1] for g in got],
+                    scan_is_min=[g[2] for g in got], marks=(np.concatenate(mq), np.concatenate(mc)))
     out["candidate_scan"] = {"queries": n_queries, "candidates_per_query": n_total, "ms_per_query": dt / n_queries * 1e3,
                              "pairs_per_s": n_queries * n_total / dt, "achieved_gbs": n_queries * n_total * 1057 / dt / 1e9,
                              "frac_of_hbm_per_gpu": n_queries * n_total * 1057 / dt / 1e9 / (peak * world),
@@ -734,6 +847,8 @@ def cfg5_block(ctx, capi, mdist, torch, comm, model, cutoff, local_rank, peak, n
         mg = mdist.merge_pass(eng, comm, torch, rows, cm, cl, delta, cutoff)
         torch.cuda.synchronize(); comm.barrier()
         dtu = comm.all_reduce_max(time.perf_counter() - t0, torch, eng.device)
+        if dump is not None:
+            dump.update(update_next=nxt, update_n_good=ng, merge_choice=mg)
         out["update_stage"] = {"centers": int(nc), "delta": delta, "member_pairs": int(off[-1]), "merge_pairs": int(nc * delta),
                                "ms_per_pass": dtu * 1e3, "pairs_per_s": (int(off[-1]) + nc * delta) / dtu,
                                "moved": int(np.count_nonzero(nxt >= 0)), "merged": int(np.count_nonzero(mg > 0))}
@@ -958,7 +1073,13 @@ def main():
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--cpu-hist-sample", type=int, default=100000)
     ap.add_argument("--cpu-pair-sample", type=int, default=20000000)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (--impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs covers the timed device path (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

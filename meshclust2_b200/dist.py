@@ -73,25 +73,31 @@ def rect_row_blocks(n, world, rank):
 
 class Survivors:
     """This rank's survivor pairs of one step, block by block, WITHOUT copying them together: an engine may hand back views
-    of its own (page-locked, per-block) buffers, valid until its next step.  tolist() / array() build the [m, 2] form."""
+    of its own (page-locked, per-block) buffers, valid until its next step.  tolist() / array() build the [m, 2] form;
+    scores() the pairs' scores in the same order, where the engine reported them."""
 
     def __init__(self):
         self.parts = []
 
     def add(self, pairs):
         if isinstance(pairs, tuple):
-            self.parts.append((np.asarray(pairs[0]), np.asarray(pairs[1])))
+            self.parts.append(tuple(np.asarray(p) for p in pairs))
         else:
             pairs = np.asarray(pairs).reshape(-1, 2)
             self.parts.append((pairs[:, 0], pairs[:, 1]))
 
     def __len__(self):
-        return int(sum(len(q) for q, _ in self.parts))
+        return int(sum(len(p[0]) for p in self.parts))
 
     def array(self):
         if not self.parts:
             return np.zeros((0, 2), dtype=np.uint64)
-        return np.stack([np.concatenate([q for q, _ in self.parts]), np.concatenate([d for _, d in self.parts])], axis=1)
+        return np.stack([np.concatenate([p[0] for p in self.parts]), np.concatenate([p[1] for p in self.parts])], axis=1)
+
+    def scores(self):
+        if not self.parts:
+            return np.zeros(0)
+        return np.concatenate([p[2] for p in self.parts])
 
     def tolist(self):
         return self.array().tolist()
@@ -142,7 +148,8 @@ def all_pairs_step(engine, comm, torch, n_total, cutoff, upper_only=True, blocks
     engine.export_local()           -> (bins [per, N] tensor, length [per] int64 tensor, mag [per] int64 tensor) padded
     engine.install_full(bins, length, mag, n_total)   make the gathered set the sweep's database
     engine.use_local_as_full()      single rank: the counted shard is the database (no copy, no collective)
-    engine.sweep(q0, q1, upper_only, cutoff, max_out) -> (n_survivors, n_scored, survivors: array [m,2] or (q[m], d[m]))
+    engine.sweep(q0, q1, upper_only, cutoff, max_out) -> (n_survivors, n_scored, survivors: array [m,2], (q[m], d[m])
+                                    or (q[m], d[m], score[m]))
     Returns dict(n_scored, n_close, survivors (this rank's), blocks)."""
     if comm.world > 1 and hasattr(engine, "count_and_gather_in_place"):
         # the product engine: K1 writes this rank's rows straight into the full set, the all-gathers run in place on it
@@ -495,4 +502,4 @@ class GpuEngine:
         nd = min(len(self.full), getattr(self, "n_total", None) or len(self.full))   # rows past n_total are shard padding
         r = self.ctx.all_pairs(self.model, self.full, self.full, cutoff, q_range=(q0, q1), d_range=(0, nd),
                                upper_only=upper_only, max_out=max_out, out=slots[slot][:3])
-        return r["n_out"], r["n_scored"], (r["q"], r["d"])
+        return r["n_out"], r["n_scored"], (r["q"], r["d"], r["score"])

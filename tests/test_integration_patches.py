@@ -1,6 +1,7 @@
 """CPU: the build-time hunks for the relinked meshclust2 (integration/patch_cluster_factory.py, integration/patch_crunner.py)
 apply to the reference sources where they lie, add only the offers to the batched entry points, and leave every reference line
-in place (the original loops stay as the declined path).  Skipped where /root/reference is absent (the GPU box)."""
+in place (the original loops stay as the declined path).  The hunk tests skip where the reference sources are absent;
+the check that a patch refuses an unexpected source needs none."""
 import difflib
 import os
 import subprocess
@@ -11,7 +12,7 @@ import pytest
 from conftest import ROOT
 
 REF = os.environ.get("MC2_REFERENCE_ROOT", "/root/reference")
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "src", "cluster")), reason="reference sources not present")
+needs_reference = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "src", "cluster")), reason="reference sources not present")
 
 
 def _patched(script, rel, tmp_path):
@@ -24,6 +25,7 @@ def _patched(script, rel, tmp_path):
     return added, removed
 
 
+@needs_reference
 def test_cluster_factory_hunks(tmp_path):
     added, removed = _patched("patch_cluster_factory.py", "ClusterFactory.cpp", tmp_path)
     text = "\n".join(added)
@@ -35,6 +37,7 @@ def test_cluster_factory_hunks(tmp_path):
     assert any(l.strip() == "merge(part, trn, delta, bandwidth);" for l in added)
 
 
+@needs_reference
 def test_crunner_hunks(tmp_path):
     added, removed = _patched("patch_crunner.py", "CRunner.cpp", tmp_path)
     text = "\n".join(added)
