@@ -342,6 +342,22 @@ int mc2_all_pairs(mc2_ctx *ctx, const mc2_model *model, const mc2_hset *set_q, u
 		  uint64_t max_out, uint64_t *out_q, uint64_t *out_d, double *out_score, uint64_t *n_out,
 		  uint64_t *n_scored);
 
+/* Identity search: every (query, database) pair of the two row ranges inside the length window, as mc2_all_pairs
+ * (FC_Runner.cpp:435-444; upper_only: c > r; feature order compute(database c, query r)), scored with a REGRESSION model
+ * (Predictor<T>::similarity = p_predict, Predictor.cpp:284-300: identity = GLM sum clamped to [0, 1]).
+ * Survivors are the pairs with identity >= min_identity (the >= of the reference's --id labels, FeatureSelector.cpp:27):
+ * min_identity <= 0 keeps every in-window pair, a value above 1 keeps none, and fastcar's `sim > 0` is min_identity = the
+ * smallest positive double (4.9406564584124654e-324).  out_identity[i] is the same bits as the score mc2_score_pairs gives
+ * the pair (set_a = set_d row out_d[i], set_b = set_q row out_q[i]), and the decision is made on that value.
+ * Ranges, capacity (*n_out is the total, which may exceed max_out), *n_scored (equal to mc2_all_pairs' for the same
+ * ranges and cutoff) and the unspecified survivor order are those of mc2_all_pairs; every shape it serves is served.
+ * MC2_ERR_ARG for a classifier model or a NaN min_identity, besides mc2_all_pairs' argument checks; MC2_ERR_FEATURE when
+ * an in-window pair hits the reference's throw (length 0 with length_difference, NaN after normalising). */
+int mc2_identity_pairs(mc2_ctx *ctx, const mc2_model *model, double min_identity, const mc2_hset *set_q, uint64_t q_begin,
+		       uint64_t q_end, const mc2_hset *set_d, uint64_t d_begin, uint64_t d_end, int32_t upper_only, double cutoff,
+		       uint64_t max_out, uint64_t *out_q, uint64_t *out_d, double *out_identity, uint64_t *n_out,
+		       uint64_t *n_scored);
+
 /* Measured issue rate (warp-instructions per second, whole GPU) of the tile sweep's inner instruction pair -- VIMNMX.U16x2 on
  * the ALU pipe feeding IDP.2A on the FMA pipe, register operands only, 32 resident warps per SM: the denominator of
  * bench.py's roofline for the CUDA-core EMD term (SURVEY.md section 8d: "achieved ... vs a measured ALU peak"). */

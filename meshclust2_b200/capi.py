@@ -38,7 +38,7 @@ SYMBOLS = [
     "mc2_seqs_total_bases", "mc2_count_kmers", "mc2_count_kmers_into", "mc2_count_kmers_auto", "mc2_hset_largest_count", "mc2_hset_alloc", "mc2_count_kmers_into_rows", "mc2_hset_refresh", "mc2_width_for_count", "mc2_kmer_table_increment", "mc2_hset_from_host", "mc2_hset_from_device", "mc2_hset_update_from_device", "mc2_hset_device_sideband", "mc2_hset_free",
     "mc2_hset_count", "mc2_hset_k", "mc2_hset_elem_bytes", "mc2_hset_device_bins", "mc2_hset_download", "mc2_hset_copy_to_device",
     "mc2_hset_set_sideband", "mc2_hset_set_row", "mc2_hset_assign_rows", "mc2_model_create", "mc2_model_free", "mc2_model_desc_from_file",
-    "mc2_score_pairs", "mc2_get_close", "mc2_get_close_as", "mc2_filter", "mc2_filter_as", "mc2_merge", "mc2_all_pairs", "mc2_debug_tile_reductions", "mc2_distance", "mc2_mean_closest", "mc2_closest",
+    "mc2_score_pairs", "mc2_get_close", "mc2_get_close_as", "mc2_filter", "mc2_filter_as", "mc2_merge", "mc2_all_pairs", "mc2_identity_pairs", "mc2_debug_tile_reductions", "mc2_distance", "mc2_mean_closest", "mc2_closest",
     "mc2_update_centers", "mc2_merge_centers",
     "mc2_bench_score_pairs", "mc2_bench_count_kmers", "mc2_bench_issue_rate", "mc2_encode_dna", "mc2_encode_dna_batch",
 ]
@@ -100,6 +100,9 @@ def lib():
         L.mc2_hset_device_bins.restype = C.c_void_p
         L.mc2_hset_device_sideband.restype = C.c_void_p
         L.mc2_ctx_flush_l2.argtypes = [C.c_void_p, C.c_size_t]
+        L.mc2_identity_pairs.argtypes = [C.c_void_p, C.c_void_p, C.c_double, C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p,
+                                         C.c_uint64, C.c_uint64, C.c_int32, C.c_double, C.c_uint64, C.c_void_p, C.c_void_p,
+                                         C.c_void_p, C.c_void_p, C.c_void_p]
         _lib = L
     return _lib
 
@@ -372,6 +375,25 @@ class Context:
                                    _p(od), _p(osc), C.byref(n_out), C.byref(n_scored)))
         got = min(n_out.value, max_out)
         return dict(q=oq[:got], d=od[:got], score=osc[:got], n_out=n_out.value, n_scored=n_scored.value)
+
+    def identity_pairs(self, model, set_q, set_d, min_identity, cutoff, q_range=None, d_range=None, upper_only=False,
+                       max_out=1 << 20, out=None):
+        """Identity search with a regression model: the in-window pairs of all_pairs whose predicted identity (the GLM sum
+        clamped to [0, 1]) is >= min_identity, with that identity.  out: optional (q, d, identity) buffers as in all_pairs."""
+        q0, q1 = q_range if q_range else (0, len(set_q))
+        d0, d1 = d_range if d_range else (0, len(set_d))
+        if out is not None:
+            oq, od, oid = out
+            assert len(oq) >= max_out and len(od) >= max_out and len(oid) >= max_out
+        else:
+            oq = np.empty(max_out, dtype=np.uint64)
+            od = np.empty(max_out, dtype=np.uint64)
+            oid = np.empty(max_out)
+        n_out, n_scored = C.c_uint64(), C.c_uint64()
+        _check(lib().mc2_identity_pairs(self.h, model.h, min_identity, set_q.h, q0, q1, set_d.h, d0, d1, int(upper_only), cutoff,
+                                        max_out, _p(oq), _p(od), _p(oid), C.byref(n_out), C.byref(n_scored)))
+        got = min(n_out.value, max_out)
+        return dict(q=oq[:got], d=od[:got], identity=oid[:got], n_out=n_out.value, n_scored=n_scored.value)
 
     def issue_rate(self, iters=100000):
         """measured warp-instructions / s of the VIMNMX.U16x2 + IDP.2A pair (roofline denominator of the tile sweep)"""

@@ -107,7 +107,9 @@ struct DevModel {
 	float scr_w[MC2_SCR_MAX_COMBOS + 1];
 	int scr_ka[MC2_SCR_MAX_COMBOS], scr_kb[MC2_SCR_MAX_COMBOS], scr_pa2[MC2_SCR_MAX_COMBOS], scr_pb2[MC2_SCR_MAX_COMBOS];
 	float scr_k1, scr_k0;
-	float scr_thr;                // a pair whose fp32 sum + bound stays below this is not close: logit(0.5 - bias) - margin
+	// a pair whose fp32 sum + bound stays below this is not close: logit(0.5 - bias) - margin for a classifier; for a
+	// regression model it is set per call on a copy (min_identity - margin, mc2_identity_pairs)
+	float scr_thr;
 };
 
 // Mailbox of the resident scan server: the accumulate stage of the mean-shift driver issues one Trainer::get_close per
@@ -275,21 +277,23 @@ int launch_argmax(mc2_ctx *ctx, const double *dist, const uint8_t *skipped, cons
 int launch_count(mc2_ctx *ctx, const mc2_seqs *s, int k, int eb, mc2_hset *h, u64 init_value);
 int launch_sideband(mc2_ctx *ctx, mc2_hset *h, bool set_mag);
 int launch_pack(mc2_ctx *ctx, const char *d_codes, const u64 *d_seq_off, mc2_seqs *s);
+// identity != 0 (mc2_identity_pairs, regression models): a pair survives on score >= min_identity instead of `close`
 int launch_all_pairs(mc2_ctx *ctx, const DevModel &dm, const mc2_hset *q, u64 q0, u64 q1, const mc2_hset *d, u64 d0, u64 d1,
 		     int upper_only, double cutoff, u64 max_out, u64 *d_out_q, u64 *d_out_d, double *d_out_score,
-		     u64 *d_counters);
+		     u64 *d_counters, int identity, double min_identity);
 int launch_distance(mc2_ctx *ctx, const PairArgs &a, u64 *d_out);
 int ensure_lane_off(mc2_ctx *ctx, const mc2_hset *h); // builds h->lane_off if the shape allows; no-op otherwise
 // tile_sweep.cu: the all-pairs sweep over 1 KiB uint8 rows as 64 x 128 pair tiles (TMA ring, tcgen05 Gram term, u16 cumulative EMD)
 int ensure_tile_operands(mc2_ctx *ctx, const mc2_hset *h, int base);
-bool tile_sweep_supported(const DevModel &dm, const mc2_hset *q, const mc2_hset *d);
+// identity: the model must be a regression model (identity search), else a classifier (mc2_all_pairs)
+bool tile_sweep_supported(const DevModel &dm, const mc2_hset *q, const mc2_hset *d, int identity);
 bool tile_sweep_shape_ok(const mc2_hset *q, const mc2_hset *d);
 int launch_issue_probe(mc2_ctx *ctx, int iters, u32 *d_out, u64 *warp_instr);
 // pair_score.cu: start the resident scan server for 1- or 2-byte bins on ctx->server_stream
 int launch_scan_server(mc2_ctx *ctx, const DevModel &dm, int eb, u64 first_seq);
 int launch_tile_sweep(mc2_ctx *ctx, const DevModel &dm, int need, const mc2_hset *q, u64 q0, u64 q1, const mc2_hset *d, u64 d0, u64 d1,
 		      int upper_only, double cutoff, u64 max_out, u64 *d_out_q, u64 *d_out_d, double *d_out_score, u64 *d_counters,
-		      u32 *raw_dot, u32 *raw_emd, u32 *raw_sad);
+		      u32 *raw_dot, u32 *raw_emd, u32 *raw_sad, int identity, double min_identity);
 int launch_mean_closest(mc2_ctx *ctx, const mc2_hset *h, const u64 *d_members, u64 n, u64 *d_sums, double *d_mean, double *d_dist,
 			void *d_out, bool have_mean);
 int launch_update_batch(mc2_ctx *ctx, const mc2_hset *h, const u64 *d_member_off, const u64 *d_members, const uint8_t *d_close,

@@ -1406,6 +1406,8 @@ struct SweepArgs {
 	u64 *out_q, *out_d;
 	double *out_score;
 	u64 *counters; // [0] survivors, [1] scored pairs
+	int identity;  // 0: survivors are the classifier's close pairs; 1 (regression models): pairs whose score >= min_identity
+	double min_identity;
 };
 
 #ifndef MC2_SWEEP_SPAN
@@ -1521,6 +1523,9 @@ __global__ void __launch_bounds__(ONE ? 128 : 256, ONE ? MC2_SWEEP_CTAS_PER_SM :
 			if (bad) {
 				atomicOr(a.err, bad & 1 ? 1 : 2);
 			}
+			if (g.identity) {
+				close = score >= g.min_identity;
+			}
 		}
 		unsigned cm = __ballot_sync(0xffffffffu, close);
 		u64 base = 0;
@@ -1631,6 +1636,9 @@ __global__ void __launch_bounds__(512, 1) sweep_wide_kernel(const __grid_constan
 				const int bad = eval_pair_fast(dm, a.N, mn, sd, sq, true, score, d0v, close);
 				if (bad) {
 					atomicOr(a.err, bad & 1 ? 1 : 2);
+				}
+				if (g.identity) {
+					close = score >= g.min_identity;
 				}
 				if (close) {
 					const u64 idx = atomicAdd(g.counters, 1ULL);
@@ -2082,14 +2090,14 @@ static void launch_sweep_wide(int need, int grid, size_t smem, cudaStream_t st, 
 
 int launch_all_pairs(mc2_ctx *ctx, const DevModel &dm, const mc2_hset *q, u64 q0, u64 q1, const mc2_hset *d, u64 d0, u64 d1,
 		     int upper_only, double cutoff, u64 max_out, u64 *d_out_q, u64 *d_out_d, double *d_out_score,
-		     u64 *d_counters)
+		     u64 *d_counters, int identity, double min_identity)
 {
-	// uint8 / uint16 rows of whole 1 KiB slabs with a classifier the fast epilogue covers: 64 x 256 pair tiles
+	// uint8 / uint16 rows of whole 1 KiB slabs with a model the fast epilogue covers: 64 x 256 pair tiles
 	// (tile_sweep.cu).  Its operand pass may still find the rows unfit (a uint16 bin above 255, a bin below the
 	// pseudo-count): nothing has been written then, and the row-streaming kernels below take the call.
-	if (tile_sweep_supported(dm, q, d)) {
+	if (tile_sweep_supported(dm, q, d, identity)) {
 		const int rc = launch_tile_sweep(ctx, dm, dm.need & 7, q, q0, q1, d, d0, d1, upper_only, cutoff, max_out, d_out_q, d_out_d,
-						 d_out_score, d_counters, nullptr, nullptr, nullptr);
+						 d_out_score, d_counters, nullptr, nullptr, nullptr, identity, min_identity);
 		if (rc != MC2_ERR_UNSUPPORTED) {
 			return rc;
 		}
@@ -2120,6 +2128,8 @@ int launch_all_pairs(mc2_ctx *ctx, const DevModel &dm, const mc2_hset *q, u64 q0
 	g.out_d = d_out_d;
 	g.out_score = d_out_score;
 	g.counters = d_counters;
+	g.identity = identity;
+	g.min_identity = min_identity;
 	const u64 groups = (q1 - q0) * ((d1 - d0 + 31) / 32);
 	u64 want = (groups + 7) / 8, cap = (u64)ctx->sm_count * 8;
 	int grid = (int)(want < cap ? want : cap);
@@ -2135,7 +2145,7 @@ int launch_all_pairs(mc2_ctx *ctx, const DevModel &dm, const mc2_hset *q, u64 q0
 	static const bool one_query = getenv("MC2_SWEEP_TWO_QUERY") == nullptr;
 	static const bool no_wide = getenv("MC2_SWEEP_NO_WIDE") != nullptr; // A/B switch: wide rows through sweep_kernel
 	if (fast) {
-		if (a.eb == 1 && row_bytes == 1024 && a.loffA && a.loffB && (dm.need & NEED_EMD) && !one_query) {
+		if (a.eb == 1 && row_bytes == 1024 && a.loffA && a.loffB && (dm.need & NEED_EMD) && !one_query && !identity) {
 			const u64 groups2 = ((q1 - q0 + 1) / 2) * ((d1 - d0 + 31) / 32);
 			u64 want2 = (groups2 + 3) / 4, cap2 = (u64)ctx->sm_count * 3;
 			int grid2 = (int)(want2 < cap2 ? want2 : cap2);

@@ -30,6 +30,9 @@
 // whatever the rounding); the rest is ballot-compacted into a per-warp list and goes, one pair per lane, through the exact fp64
 // epilogue shared with the other pair kernels (eval_pair_fast), so scores and decisions are the same bits as theirs.
 // The screen is for 1024-bin rows; wider rows send every in-window pair through the exact epilogue.
+// Identity search (Params::identity, mc2_identity_pairs): a regression model, clamp(sum) >= t <=> sum >= t for 0 < t <= 1,
+// so the same screen rejects on sum + bound < t - margin (DevModel::scr_thr, set per call) and the exact epilogue keeps
+// the pairs whose clamped sum is >= t.  The mode is a uniform runtime field read by the epilogue warps only.
 #include "mc2_internal.cuh"
 #include "pair_eval.cuh"
 #include <cuda.h>
@@ -95,6 +98,8 @@ struct Params {
 	double *out_score;
 	u64 *counters;          // [0] survivors, [1] scored pairs
 	int *err;
+	int identity;           // 0: survivors are the classifier's close pairs; 1: pairs whose score >= min_identity
+	double min_identity;
 	Sideband sbQ, sbD;
 	const u32 *csQ, *csD;   // per-row sum of the cumulative row (EMD identity)
 	u32 nqt, ndt;           // tiles along each side
@@ -897,6 +902,9 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 									if (bad) {
 										atomicOr(p.err, bad & 1 ? 1 : 2);
 									}
+									if (p.identity) {
+										close = score >= p.min_identity;
+									}
 								}
 								const unsigned cm = __ballot_sync(0xffffffffu, close);
 								u64 obase = 0;
@@ -1243,13 +1251,13 @@ bool tile_sweep_shape_ok(const mc2_hset *q, const mc2_hset *d)
 	return shape && sums && !known_bad;
 }
 
-bool tile_sweep_supported(const DevModel &dm, const mc2_hset *q, const mc2_hset *d)
+bool tile_sweep_supported(const DevModel &dm, const mc2_hset *q, const mc2_hset *d, int identity)
 {
 	const bool off = getenv("MC2_SWEEP_LEGACY") != nullptr; // read per call: bench.py times both forms in one process
 	if (off) {
 		return false;
 	}
-	const bool model = dm.fast_epi && !dm.regression && !(dm.need & NEED_LOG) && (dm.need & 7) != 0;
+	const bool model = dm.fast_epi && (dm.regression != 0) == (identity != 0) && !(dm.need & NEED_LOG) && (dm.need & 7) != 0;
 	return model && tile_sweep_shape_ok(q, d);
 }
 
@@ -1268,7 +1276,7 @@ template <int NEED, bool RAW> static int launch_need(int grid, cudaStream_t st, 
 
 int launch_tile_sweep(mc2_ctx *ctx, const DevModel &dm, int need, const mc2_hset *q, u64 q0, u64 q1, const mc2_hset *d, u64 d0, u64 d1,
 		      int upper_only, double cutoff, u64 max_out, u64 *d_out_q, u64 *d_out_d, double *d_out_score, u64 *d_counters,
-		      u32 *raw_dot, u32 *raw_emd, u32 *raw_sad)
+		      u32 *raw_dot, u32 *raw_emd, u32 *raw_sad, int identity, double min_identity)
 {
 	if (!ctx->d_sched) {
 		MC2_CUDA(cudaMalloc(&ctx->d_sched, (ts::MAX_SUPER + 1) * 4));
@@ -1296,6 +1304,8 @@ int launch_tile_sweep(mc2_ctx *ctx, const DevModel &dm, int need, const mc2_hset
 	p.out_q = d_out_q; p.out_d = d_out_d; p.out_score = d_out_score;
 	p.counters = d_counters;
 	p.err = ctx->d_err;
+	p.identity = identity;
+	p.min_identity = min_identity;
 	p.sbQ = Sideband{q->mag, q->sum, q->sumsq, q->len};
 	p.sbD = Sideband{d->mag, d->sum, d->sumsq, d->len};
 	p.csQ = q->cumsum; p.csD = d->cumsum;

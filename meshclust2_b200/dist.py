@@ -141,15 +141,18 @@ class Comm:
         return float(t.item())
 
 
-def all_pairs_step(engine, comm, torch, n_total, cutoff, upper_only=True, blocks_per_rank=1, max_out=1 << 20):
+def all_pairs_step(engine, comm, torch, n_total, cutoff, upper_only=True, blocks_per_rank=1, max_out=1 << 20, identity=None):
     """One pass of the hot path over a batch: local K1 -> all-gather -> row-block K2 sweep.
+
+    identity: None sweeps with the engine's classifier; (regression model, min_identity) makes it an identity search
+    (survivors = pairs whose predicted identity is >= min_identity, Survivors.scores() = those identities).
 
     engine.count()                  K1 over this rank's shard
     engine.export_local()           -> (bins [per, N] tensor, length [per] int64 tensor, mag [per] int64 tensor) padded
     engine.install_full(bins, length, mag, n_total)   make the gathered set the sweep's database
     engine.use_local_as_full()      single rank: the counted shard is the database (no copy, no collective)
-    engine.sweep(q0, q1, upper_only, cutoff, max_out) -> (n_survivors, n_scored, survivors: array [m,2], (q[m], d[m])
-                                    or (q[m], d[m], score[m]))
+    engine.sweep(q0, q1, upper_only, cutoff, max_out[, identity=(model, min_identity)])
+                                    -> (n_survivors, n_scored, survivors: array [m,2], (q[m], d[m]) or (q[m], d[m], score[m]))
     Returns dict(n_scored, n_close, survivors (this rank's), blocks)."""
     if comm.world > 1 and hasattr(engine, "count_and_gather_in_place"):
         # the product engine: K1 writes this rank's rows straight into the full set, the all-gathers run in place on it
@@ -176,7 +179,10 @@ def all_pairs_step(engine, comm, torch, n_total, cutoff, upper_only=True, blocks
     n_scored = n_close = 0
     surv = Survivors()
     for q0, q1 in blocks:
-        ns, sc, pairs = engine.sweep(q0, q1, upper_only, cutoff, max_out)
+        if identity is None:
+            ns, sc, pairs = engine.sweep(q0, q1, upper_only, cutoff, max_out)
+        else:
+            ns, sc, pairs = engine.sweep(q0, q1, upper_only, cutoff, max_out, identity=identity)
         n_close += ns
         n_scored += sc
         surv.add(pairs)
@@ -476,7 +482,8 @@ class GpuEngine:
         sc = self._stage_centers(rows, mag, length)
         return self.ctx.merge_centers(self.model, sc, len(rows), delta, cutoff)
 
-    def sweep(self, q0, q1, upper_only, cutoff, max_out):
+    def sweep(self, q0, q1, upper_only, cutoff, max_out, identity=None):
+        """identity: None = the engine's classifier (all_pairs), else (regression model, min_identity) (identity_pairs)"""
         # survivor buffers: one page-locked triple per block of a step, allocated once and reused by every step (fresh
         # pageable arrays cost page faults + a staged copy per call; a shared triple would force a host copy per block)
         slots = getattr(self, "_surv_slots", None)
@@ -500,6 +507,11 @@ class GpuEngine:
                     pass
             slots[slot] = bufs + (pinned,)
         nd = min(len(self.full), getattr(self, "n_total", None) or len(self.full))   # rows past n_total are shard padding
+        if identity is not None:
+            model, t = identity
+            r = self.ctx.identity_pairs(model, self.full, self.full, t, cutoff, q_range=(q0, q1), d_range=(0, nd),
+                                        upper_only=upper_only, max_out=max_out, out=slots[slot][:3])
+            return r["n_out"], r["n_scored"], (r["q"], r["d"], r["identity"])
         r = self.ctx.all_pairs(self.model, self.full, self.full, cutoff, q_range=(q0, q1), d_range=(0, nd),
                                upper_only=upper_only, max_out=max_out, out=slots[slot][:3])
         return r["n_out"], r["n_scored"], (r["q"], r["d"], r["score"])
