@@ -372,6 +372,11 @@ int mc2_bench_issue_rate(mc2_ctx *ctx, int iters, double *warp_instr_per_s);
 int mc2_debug_tile_reductions(mc2_ctx *ctx, const mc2_hset *set_q, uint64_t q_begin, uint64_t q_end, const mc2_hset *set_d,
 			      uint64_t d_begin, uint64_t d_end, int32_t need, uint32_t *out_dot, uint32_t *out_emd, uint32_t *out_sad);
 
+/* Diagnostic (tests, benchmarks): of the last mc2_all_pairs / mc2_identity_pairs call on this context, *n_exact = the pairs
+ * the tile sweep sent through the exact fp64 epilogue (those its fp32 screen could not reject; 0 for the row-streaming
+ * kernels) and *coarse = 1 if it took the coarse form (the screen on 64 sampled cumulative bins), else 0. */
+int mc2_debug_last_sweep(mc2_ctx *ctx, uint64_t *n_exact, int32_t *coarse);
+
 /* DivergencePoint<T>::distance (src/clutil/DivergencePoint.cpp:70-82) for pairs of rows */
 int mc2_distance(mc2_ctx *ctx, const mc2_pairs *pairs, uint64_t *out);
 

@@ -38,7 +38,7 @@ SYMBOLS = [
     "mc2_seqs_total_bases", "mc2_count_kmers", "mc2_count_kmers_into", "mc2_count_kmers_auto", "mc2_hset_largest_count", "mc2_hset_alloc", "mc2_count_kmers_into_rows", "mc2_hset_refresh", "mc2_width_for_count", "mc2_kmer_table_increment", "mc2_hset_from_host", "mc2_hset_from_device", "mc2_hset_update_from_device", "mc2_hset_device_sideband", "mc2_hset_free",
     "mc2_hset_count", "mc2_hset_k", "mc2_hset_elem_bytes", "mc2_hset_device_bins", "mc2_hset_download", "mc2_hset_copy_to_device",
     "mc2_hset_set_sideband", "mc2_hset_set_row", "mc2_hset_assign_rows", "mc2_model_create", "mc2_model_free", "mc2_model_desc_from_file",
-    "mc2_score_pairs", "mc2_get_close", "mc2_get_close_as", "mc2_filter", "mc2_filter_as", "mc2_merge", "mc2_all_pairs", "mc2_identity_pairs", "mc2_debug_tile_reductions", "mc2_distance", "mc2_mean_closest", "mc2_closest",
+    "mc2_score_pairs", "mc2_get_close", "mc2_get_close_as", "mc2_filter", "mc2_filter_as", "mc2_merge", "mc2_all_pairs", "mc2_identity_pairs", "mc2_debug_tile_reductions", "mc2_debug_last_sweep", "mc2_distance", "mc2_mean_closest", "mc2_closest",
     "mc2_update_centers", "mc2_merge_centers",
     "mc2_bench_score_pairs", "mc2_bench_count_kmers", "mc2_bench_issue_rate", "mc2_encode_dna", "mc2_encode_dna_batch",
 ]
@@ -411,6 +411,13 @@ class Context:
                                                C.c_uint64(d1), int(need), _p(out["dot"]) if "dot" in out else None,
                                                _p(out["emd"]) if "emd" in out else None, _p(out["sad"]) if "sad" in out else None))
         return out
+
+    def last_sweep(self):
+        """Diagnostic: {n_exact, coarse} of the last all_pairs / identity_pairs call -- the pairs the tile sweep sent
+        through the exact epilogue, and whether it took the coarse form"""
+        n, c = C.c_uint64(), C.c_int32()
+        _check(lib().mc2_debug_last_sweep(self.h, C.byref(n), C.byref(c)))
+        return dict(n_exact=n.value, coarse=bool(c.value))
 
     def distance(self, set_a, set_b, ia, ib):
         p = self._pairs(set_a, set_b, ia, ib, len(ia))

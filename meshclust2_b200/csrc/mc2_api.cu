@@ -100,6 +100,9 @@ struct CtxExtra {
 	std::vector<cudaEvent_t> pool;
 	double prof_ms[MC2_KERNEL_KINDS] = {0};
 	u64 prof_n[MC2_KERNEL_KINDS] = {0};
+	// the last all-pairs / identity sweep: pairs the tile sweep sent through the exact epilogue, 1 if it took the coarse form
+	u64 last_exact = 0;
+	int last_coarse = 0;
 };
 
 static cudaEvent_t prof_event(CtxExtra *x)
@@ -248,6 +251,13 @@ static int d2h(mc2_ctx *ctx, void *dst, const void *src, size_t bytes)
 //   a combo of total degree P <= 4 in factors bounded by u with that error: |delta| <= u^4 * eps * (1.01 P gamma + P);
 //   weights in fp32 and the fused accumulation add eps * (2 + n_combos + 1) per term.
 // Hence |fp32 sum - exact sum| <= eps * (K1 * u^4 + K0); both constants are doubled before rounding to float.
+// The coarse form of the sweep knows the EMD only as an interval [e1, e2] of exact integers and bounds the sum from
+// above: each combo with the EMD factor takes the larger of its values at x(e1), x(e2) (and 0 for a squared factor whose
+// interval spans 0).  Both ends are the same cancellation-free expressions as the exact EMD's, so the per-term bound holds
+// at each end with u = 1 + max |x| over both; the max of two fused sums fma(w, f_i, s) is the rounding of
+// max(w f_i) + s (rounding is monotone), so the accumulation's term is unchanged; the ends' fp32 values are each within
+// eps * gamma * u of the exact ones, so the spans-0 test on the interval widened by scr_dx * u = eps * gamma * u never
+// misses a sign change.  The bound, hence K1 and K0, is the same: |fp32 sum - exact upper bound| <= eps * (K1 u^4 + K0).
 // The threshold on the sum, rounded down past that margin: a pair whose fp32 sum + bound stays below it has exact sum < t.
 static float screen_threshold(double t)
 {
@@ -259,7 +269,7 @@ static float screen_threshold(double t)
 static void build_screen(DevModel &dm)
 {
 	dm.scr_ok = 0;
-	dm.scr_k1 = dm.scr_k0 = 0;
+	dm.scr_k1 = dm.scr_k0 = dm.scr_dx = 0;
 	dm.scr_thr = 0;
 	memset(dm.scr_a, 0, sizeof dm.scr_a);
 	memset(dm.scr_b, 0, sizeof dm.scr_b);
@@ -341,6 +351,7 @@ static void build_screen(DevModel &dm)
 	const double K0 = (dm.n_combos + 2) * fabs(dm.weight[0]);
 	dm.scr_k1 = nextafterf((float)(2 * eps * K1), INFINITY);
 	dm.scr_k0 = nextafterf((float)(2 * eps * K0), INFINITY);
+	dm.scr_dx = nextafterf((float)(2 * eps * gamma), INFINITY);
 	dm.scr_ok = 1;
 }
 
@@ -1153,6 +1164,7 @@ int mc2_count_kmers_into_rows(mc2_ctx *ctx, const mc2_seqs *seqs, mc2_hset *dst,
 	view.maxc = dst->maxc + first_row;
 	view.lane_off = nullptr;
 	view.cum16 = nullptr;
+	view.cum16s = nullptr;
 	view.plane8 = nullptr;
 	view.cumsum = nullptr;
 	return count_into(ctx, seqs, dst->k, dst->eb, 1, &view);
@@ -1380,6 +1392,7 @@ void mc2_hset_free(mc2_hset *h)
 	cudaFree(h->maxc);
 	cudaFree(h->lane_off);
 	cudaFree(h->cum16);
+	cudaFree(h->cum16s);
 	cudaFree(h->plane8);
 	cudaFree(h->cumsum);
 	delete h;
@@ -2143,8 +2156,10 @@ static int sweep_pairs(const char *who, mc2_ctx *ctx, const DevModel &dm, int id
 	MC2_CUDA(cudaSetDevice(ctx->device));
 	*n_out = 0;
 	if (n_scored) *n_scored = 0;
-	if (q_begin == q_end || d_begin == d_end) return MC2_OK;
 	CtxExtra *x = extra(ctx);
+	x->last_exact = 0;
+	x->last_coarse = 0;
+	if (q_begin == q_end || d_begin == d_end) return MC2_OK;
 	int rc;
 	u64 cap = max_out ? max_out : 1;
 	rc = ensure(x->d[B_OUTQ], cap * 8, false); if (rc) return rc;
@@ -2160,10 +2175,12 @@ static int sweep_pairs(const char *who, mc2_ctx *ctx, const DevModel &dm, int id
 	if (rc == MC2_OK) rc = fetch_err(ctx);
 	if (rc != MC2_OK) return rc;
 	cudaStream_t st = ctx->stream;
-	MC2_CUDA(cudaMemcpyAsync(ctx->h_slot, d_counters, 16, cudaMemcpyDeviceToHost, st));
+	MC2_CUDA(cudaMemcpyAsync(ctx->h_slot, d_counters, 32, cudaMemcpyDeviceToHost, st));
 	MC2_CUDA(cudaStreamSynchronize(st));
 	u64 total = ((u64 *)ctx->h_slot)[0];
 	if (n_scored) *n_scored = ((u64 *)ctx->h_slot)[1];
+	x->last_exact = ((u64 *)ctx->h_slot)[2];
+	x->last_coarse = ((u64 *)ctx->h_slot)[3] != 0;
 	*n_out = total;
 	u64 got = total < max_out ? total : max_out;
 	if (got) {
@@ -2201,6 +2218,15 @@ int mc2_identity_pairs(mc2_ctx *ctx, const mc2_model *model, double min_identity
 	}
 	return sweep_pairs("mc2_identity_pairs", ctx, dm, 1, min_identity, set_q, q_begin, q_end, set_d, d_begin, d_end, upper_only,
 			   cutoff, max_out, out_q, out_d, out_identity, n_out, n_scored);
+}
+
+int mc2_debug_last_sweep(mc2_ctx *ctx, uint64_t *n_exact, int32_t *coarse)
+{
+	MC2_REQUIRE(ctx && n_exact && coarse, "mc2_debug_last_sweep: NULL argument");
+	const CtxExtra *x = extra(ctx);
+	*n_exact = x->last_exact;
+	*coarse = x->last_coarse;
+	return MC2_OK;
 }
 
 int mc2_bench_issue_rate(mc2_ctx *ctx, int iters, double *warp_instr_per_s)

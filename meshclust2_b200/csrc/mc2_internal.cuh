@@ -107,6 +107,7 @@ struct DevModel {
 	float scr_w[MC2_SCR_MAX_COMBOS + 1];
 	int scr_ka[MC2_SCR_MAX_COMBOS], scr_kb[MC2_SCR_MAX_COMBOS], scr_pa2[MC2_SCR_MAX_COMBOS], scr_pb2[MC2_SCR_MAX_COMBOS];
 	float scr_k1, scr_k0;
+	float scr_dx;                 // |fl(x) - x| <= scr_dx * (1 + max |x|) for every single x (the coarse form's sign test)
 	// a pair whose fp32 sum + bound stays below this is not close: logit(0.5 - bias) - margin for a classifier; for a
 	// regression model it is set per call on a copy (min_identity - margin, mc2_identity_pairs)
 	float scr_thr;
@@ -223,7 +224,10 @@ struct mc2_hset {
 	// Operands of the tile sweep (tile_sweep.cu; uint8 / uint16 rows of whole 1 KiB slabs): inclusive cumulative rows of
 	// (bin - cum_base) as u16 (n x N), each row's sum of them (u32), and for uint16 bins the rows as bytes.  Built lazily,
 	// dropped whenever bins change.  cum16_valid: 0 not built, 1 built, -1 the set cannot be served with cum_base.
+	// Rows of one slab (N = 1024) also get cum16s: the cumulative values at bins 16 j + 15 (n x 64, u16), the operand of
+	// the tile sweep's coarse form; same lifetime as cum16.
 	unsigned short *cum16;
+	unsigned short *cum16s;
 	u32 *cumsum;
 	unsigned char *plane8;
 	int cum16_valid;

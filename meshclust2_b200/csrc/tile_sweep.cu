@@ -30,6 +30,13 @@
 // whatever the rounding); the rest is ballot-compacted into a per-warp list and goes, one pair per lane, through the exact fp64
 // epilogue shared with the other pair kernels (eval_pair_fast), so scores and decisions are the same bits as theirs.
 // The screen is for 1024-bin rows; wider rows send every in-window pair through the exact epilogue.
+// Coarse form (COARSE, one-slab rows with a screen, the bench shape): the screen needs an upper bound on the GLM sum, not
+// the exact EMD.  Cumulative rows are non-decreasing (every bin >= base), so m_i = min(cumP_i, cumQ_i) is too, and its
+// values at the 64 block ends s_j = 16 j + 15 (mc2_hset::cum16s, one ring stage) bound the whole sum:
+// 16 (M - T) <= sum_i m_i <= 16 M with M = sum_j m(s_j), T = m(s_63) = min(totP, totQ).  A tile streams the 8 u8 stages
+// and that single stage; the screen takes the EMD as the interval [cs - 32 M, cs - 32 (M - T)] and the candidates it
+// keeps get the exact sum min(cumP, cumQ) over the full rows from global memory (one warp per candidate) before the same
+// exact epilogue, so scores and decisions are the bits of the full form.
 // Identity search (Params::identity, mc2_identity_pairs): a regression model, clamp(sum) >= t <=> sum >= t for 0 < t <= 1,
 // so the same screen rejects on sum + bound < t - margin (DevModel::scr_thr, set per call) and the exact epilogue keeps
 // the pairs whose clamped sum is >= t.  The mode is a uniform runtime field read by the epilogue warps only.
@@ -96,12 +103,15 @@ struct Params {
 	u64 max_out;
 	u64 *out_q, *out_d;
 	double *out_score;
-	u64 *counters;          // [0] survivors, [1] scored pairs
+	u64 *counters;          // [0] survivors, [1] scored pairs, [2] pairs through the exact epilogue, [3] 1: coarse form
 	int *err;
 	int identity;           // 0: survivors are the classifier's close pairs; 1: pairs whose score >= min_identity
 	double min_identity;
 	Sideband sbQ, sbD;
 	const u32 *csQ, *csD;   // per-row sum of the cumulative row (EMD identity)
+	// coarse form: the full cumulative rows (exact refinement of the candidates) and the 64 samples per row (the last one
+	// is the row's total)
+	const unsigned short *cumQ, *cumD, *smpQ, *smpD;
 	u32 nqt, ndt;           // tiles along each side
 	u32 group;              // query tiles per super-row of the schedule
 	u32 n_super;
@@ -365,9 +375,11 @@ struct RowF {          // per-row values of the screen
 	float rss;     // 1 / sqrt(sumsq)
 	float rnn;     // 1 / sqrt(N*sumsq - 2*mag*sum + mag^2)  (pearson's centred norm, exact integer -> float)
 	u32 big;       // mag or len outside the screen's comfortable range -> exact path
+	u32 tot;       // coarse form: the row's last cumulative value
 };
 
-__device__ __forceinline__ RowF make_rowf(const Sideband &sb, const u32 *cs, u64 row, bool ok, u64 &len)
+// smp: the coarse form's samples (64 per row) or nullptr
+__device__ __forceinline__ RowF make_rowf(const Sideband &sb, const u32 *cs, const unsigned short *smp, u64 row, bool ok, u64 &len)
 {
 	RowF r;
 	memset(&r, 0, sizeof r);
@@ -387,6 +399,7 @@ __device__ __forceinline__ RowF make_rowf(const Sideband &sb, const u32 *cs, u64
 		const long long m = (long long)(mag & 0x3FFFFFFull);
 		r.rnn = rsqrtf((float)(1024ll * (long long)sumsq - 2ll * m * (long long)sum + m * m));
 		r.cs = cs ? cs[row] : 0u;
+		r.tot = smp ? smp[row * 64 + 63] : 0u;
 	}
 	return r;
 }
@@ -400,9 +413,13 @@ __device__ __forceinline__ float sqrt_approx(float x)
 
 // sx: this thread's column of the epilogue's scratch, element (slot, t) at sx[(slot * NP + t) * (NEW * 32)]; slot = single
 // slot (scr_slot), the last slot holds the constant 1 (written once per kernel)
-template <int NEED, int NP>
-__device__ __forceinline__ u32 screen_pairs(const DevModel &dm, float *sx, const u32 (&dot)[NP], const u32 (&emd)[NP], const u32 (&sad)[NP],
-					    const RowF &P, const RowF *Q)
+// COARSE: the EMD is only known to lie in [emd[t], emd_hi[t]] (exact integers).  x is evaluated at both ends, u covers
+// both, and a combo with the EMD factor adds the larger of its values at the two ends: the other factor is fixed, so the
+// combo is linear in x or in x^2, and x^2 over an interval that spans 0 also takes the value 0 (the fused sums are
+// monotone in the exact value, so max(fma(w, f1, s), fma(w, f2, s)) = fl(max(w f1, w f2) + s) keeps the error model).
+template <int NEED, int NP, bool COARSE>
+__device__ __forceinline__ u32 screen_pairs(const DevModel &dm, float *sx, const u32 (&dot)[NP], const u32 (&emd)[NP], const u32 (&emd_hi)[NP],
+					    const u32 (&sad)[NP], const RowF &P, const RowF *Q)
 {
 	constexpr int ET = NEW * 32;
 	float m[NP];
@@ -447,8 +464,22 @@ __device__ __forceinline__ u32 screen_pairs(const DevModel &dm, float *sx, const
 		MC2_SCR(SC_INTERSECTION, __fdividef(two_smin[t], P.magf + Q[t].magf))
 		MC2_SCR(SC_KULCZYNSKI2, __fdividef(P.magf + Q[t].magf, 2.0f * (P.magf * (1.0f / 1024.0f)) * (Q[t].magf * (1.0f / 1024.0f))) * (0.5f * two_smin[t]))
 	}
+	float xe_hi[NP]; // COARSE: the EMD single at the upper end of its interval (the lower end is in its slot)
 	if constexpr ((NEED & NEED_EMD) != 0) {
-		MC2_SCR(SC_EMD, (float)emd[t])
+		if constexpr (COARSE) {
+			if (dm.slot[SC_EMD] >= 0) {
+				const float a_ = dm.scr_a[SC_EMD], b_ = dm.scr_b[SC_EMD];
+#pragma unroll
+				for (int t = 0; t < NP; t++) {
+					const float x1 = __fmaf_rn(a_, (float)emd[t], b_);
+					sx[(scr_slot(NEED & 7, SC_EMD) * NP + t) * ET] = x1;
+					xe_hi[t] = __fmaf_rn(a_, (float)emd_hi[t], b_);
+					m[t] = fmaxf(m[t], fmaxf(fabsf(x1), fabsf(xe_hi[t])));
+				}
+			}
+		} else {
+			MC2_SCR(SC_EMD, (float)emd[t])
+		}
 	}
 	MC2_SCR(SC_LENGTHD, fabsf(P.lenf - Q[t].lenf))
 #undef MC2_SCR
@@ -457,16 +488,38 @@ __device__ __forceinline__ u32 screen_pairs(const DevModel &dm, float *sx, const
 	for (int t = 0; t < NP; t++) {
 		s[t] = dm.scr_w[0];
 	}
+	constexpr int KE = scr_slot(NEED & 7, SC_EMD);
 #pragma unroll 1
 	for (int c = 0; c < dm.n_combos; c++) {
-		const int ka = dm.scr_ka[c] * NP * ET, kb = dm.scr_kb[c] * NP * ET;
+		const int sa = dm.scr_ka[c], sb = dm.scr_kb[c];
+		const int ka = sa * NP * ET, kb = sb * NP * ET;
 		const bool pa2 = dm.scr_pa2[c] != 0, pb2 = dm.scr_pb2[c] != 0;
 		const float w = dm.scr_w[c + 1];
+		if (COARSE && (NEED & NEED_EMD) != 0 && (sa == KE || sb == KE)) {
+			// the EMD factor (a combo holds it once: EMD x EMD is one factor squared) against the other, fixed one
+			const bool ea = sa == KE, e2 = ea ? pa2 : pb2, o2 = ea ? pb2 : pa2;
+			const int ko = ea ? kb : ka;
 #pragma unroll
-		for (int t = 0; t < NP; t++) {
-			const float xa = sx[ka + t * ET], xb = sx[kb + t * ET];
-			const float fa = pa2 ? xa * xa : xa, fb = pb2 ? xb * xb : xb;
-			s[t] = __fmaf_rn(w, fa * fb, s[t]);
+			for (int t = 0; t < NP; t++) {
+				const float xo = sx[ko + t * ET], fo = o2 ? xo * xo : xo;
+				const float x1 = sx[KE * NP * ET + t * ET], x2 = xe_hi[t];
+				const float f1 = e2 ? x1 * x1 : x1, f2 = e2 ? x2 * x2 : x2;
+				float sn = fmaxf(__fmaf_rn(w, f1 * fo, s[t]), __fmaf_rn(w, f2 * fo, s[t]));
+				// x^2 reaches 0 inside the interval: tested on the interval widened by the bound on |fl(x) - x|, so a
+				// sign change the rounding hides is still taken
+				const float tol = dm.scr_dx * ((1.0f + m[t]) * 1.001f);
+				if (e2 && fminf(x1, x2) <= tol && fmaxf(x1, x2) >= -tol) {
+					sn = fmaxf(sn, s[t]);
+				}
+				s[t] = sn;
+			}
+		} else {
+#pragma unroll
+			for (int t = 0; t < NP; t++) {
+				const float xa = sx[ka + t * ET], xb = sx[kb + t * ET];
+				const float fa = pa2 ? xa * xa : xa, fb = pb2 ? xb * xb : xb;
+				s[t] = __fmaf_rn(w, fa * fb, s[t]);
+			}
 		}
 	}
 	u32 maybe = 0;
@@ -503,8 +556,9 @@ template <int NEED> struct Smem {
 	static_assert(TOTAL <= 232448, "shared memory per CTA");
 };
 
-// ONE: rows of one 1 KiB slab (k = 5), stage counts known at compile time; otherwise Params::n_slabs slabs per row
-template <int NEED, bool RAW, bool ONE>
+// ONE: rows of one 1 KiB slab (k = 5), stage counts known at compile time; otherwise Params::n_slabs slabs per row.
+// COARSE: the coarse form (header comment); the cumulative tensor maps are those of the samples (64 per row)
+template <int NEED, bool RAW, bool ONE, bool COARSE>
 __global__ void __launch_bounds__(THREADS, 1)
 tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ Params p, const __grid_constant__ CUtensorMap mapCumD,
 		  const __grid_constant__ CUtensorMap mapCumQ, const __grid_constant__ CUtensorMap mapU8D,
@@ -513,14 +567,16 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 	using L = Smem<NEED>;
 	constexpr int NP = L::NP, LIST_CAP = L::LIST_CAP;
 	constexpr bool DOT = (NEED & NEED_DOT) != 0, EMD = (NEED & NEED_EMD) != 0, MIN = (NEED & NEED_MIN) != 0;
+	static_assert(!COARSE || (ONE && EMD && !RAW), "the coarse form is for one-slab rows, a model with EMD, scoring");
 	constexpr bool U8_PHASE = DOT || MIN;
 	constexpr bool CUDA_RED = EMD || MIN;             // compute warps produce sums for the epilogue
 	const int n_slabs = ONE ? 1 : (int)p.n_slabs;
 	const int N_U8 = U8_PHASE ? n_slabs * (NBINS / KC_U8) : 0;   // ring stages per tile while the u8 rows stream
-	const int N_CUM = EMD ? n_slabs * (NBINS / KC_CUM) : 0;      // ... while the cumulative rows stream
+	const int N_CUM = EMD ? (COARSE ? 1 : n_slabs * (NBINS / KC_CUM)) : 0; // ... while the cumulative rows (samples) stream
 	// Gram + EMD models: every third stage carries u8 rows (for the MMA issuer only), so the compute warps never sit
-	// through a whole u8 phase; otherwise the u8 stages come first, then the cumulative ones
-	constexpr bool INTERLEAVE = DOT && EMD && !MIN;
+	// through a whole u8 phase; otherwise (and in the coarse form, 8 + 1 stages) the u8 stages come first, then the
+	// cumulative ones
+	constexpr bool INTERLEAVE = DOT && EMD && !MIN && !COARSE;
 	auto stage_is_u8 = [N_U8](int c) { return INTERLEAVE ? (c % 3 == 2) : (c < N_U8); };
 	auto stage_index = [N_U8](int c) { return INTERLEAVE ? (c % 3 == 2 ? c / 3 : c - c / 3) : (c < N_U8 ? c : c - N_U8); };
 	extern __shared__ unsigned char smem_raw[];
@@ -770,7 +826,10 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 		}
 		const int qc0 = (ew >> 2) * QE; // this warp's query columns: qc0 .. qc0 + QE - 1
 		u32 it = 0;
-		u64 scored_total = 0;
+		u64 scored_total = 0, exact_total = 0;
+		if (COARSE && blockIdx.x == 0 && etid == 0) {
+			p.counters[3] = 1;
+		}
 		for (u32 item = blockIdx.x; item < n_items; item += gridDim.x) {
 			const Tile t = decode_item(p, s_sched, item);
 			if (!t.valid) {
@@ -785,7 +844,7 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 					const u64 row = qrow0 + etid;
 					const bool ok = row < p.q1;
 					u64 len;
-					s_rowQ[par * TQ + etid] = make_rowf(p.sbQ, p.csQ, row, ok, len);
+					s_rowQ[par * TQ + etid] = make_rowf(p.sbQ, p.csQ, COARSE ? p.smpQ : nullptr, row, ok, len);
 					// FC_Runner.cpp:435-444: size_t truncation of len * id and len / id; an empty window marks an unused row
 					const u64 wlo = ok ? (u64)((double)len * p.cutoff) : 1, whi = ok ? (u64)((double)len / p.cutoff) : 0;
 					s_winQ[(par * TQ + etid) * 2] = wlo;
@@ -797,7 +856,7 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 				for (int r = 0; r < 2; r++) {
 					const u64 row = drow0 + r * 128 + lane_row;
 					const bool ok = row < p.d1;
-					PD[r] = make_rowf(p.sbD, p.csD, row, ok, lenD[r]);
+					PD[r] = make_rowf(p.sbD, p.csD, COARSE ? p.smpD : nullptr, row, ok, lenD[r]);
 					if (!ok) {
 						lenD[r] = ~0ull;
 					}
@@ -818,7 +877,7 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 			for (int r = 0; r < 2; r++) {
 #pragma unroll 1
 				for (int qc = qc0; qc < qc0 + QE; qc += NP) {
-					u32 vd[NP] = {}, ve[NP] = {}, vs[NP] = {};
+					u32 vd[NP] = {}, ve[NP] = {}, vs[NP] = {}, ve_hi[NP] = {};
 					if (DOT) tc_ldn(tmem_base + tlane + TM_DOT + buf * 128 + r * 64 + qc, vd);
 					if (EMD) tc_ldn(tmem_base + tlane + TM_EMD + eb * 128 + r * 64 + qc, ve);
 					if (MIN) tc_ldn(tmem_base + tlane + TM_SAD + r * 64 + qc, vs);
@@ -848,7 +907,16 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 							}
 							const bool g = inwin && (!p.upper_only || d > qrow0 + qc + k);
 							go |= g ? (1u << k) : 0u;
-							if (EMD) ve[k] = g ? Q[k].cs + PD[r].cs - 2u * ve[k] : 0u;
+							if constexpr (COARSE) {
+								// ve = M: sum_i m_i lies in [16 (M - T), 16 M], so the EMD in [cs - 32 M, cs - 32 (M - T)]
+								// (the exact EMD is >= 0, which also bounds it from below)
+								const u32 cs = Q[k].cs + PD[r].cs, M32 = 32u * ve[k];
+								const u32 T = min(Q[k].tot, PD[r].tot);
+								ve_hi[k] = g ? cs - M32 + 32u * T : 0u;
+								ve[k] = g && cs > M32 ? cs - M32 : 0u;
+							} else if (EMD) {
+								ve[k] = g ? Q[k].cs + PD[r].cs - 2u * ve[k] : 0u;
+							}
 						}
 						scored += __popc(go);
 						u32 cand = p.no_screen ? 0u : go;
@@ -859,7 +927,7 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 							anybig |= Q[k].big;
 						}
 						if (can_screen && __any_sync(0xffffffffu, cand != 0 && !anybig)) {
-							const u32 maybe = screen_pairs<NEED, NP>(dm, sx, vd, ve, vs, PD[r], Q);
+							const u32 maybe = screen_pairs<NEED, NP, COARSE>(dm, sx, vd, ve, ve_hi, vs, PD[r], Q);
 							if (!anybig) {
 								cand &= maybe;
 							}
@@ -883,8 +951,40 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 						}
 						if (n_list > LIST_CAP - 32 * NP || (r == 1 && qc == qc0 + QE - NP)) {
 							__syncwarp();
+							exact_total += n_list;
 							for (u32 base = 0; base < n_list; base += 32) {
 								const u32 e = base + (u32)lane;
+								// coarse form: the exact sum min(cumP, cumQ) of the batch's candidates, one warp per
+								// candidate (lane l: bins 32 l .. 32 l + 31 of both rows), kept by the candidate's lane
+								u32 smin = 0;
+								if constexpr (COARSE) {
+									const u32 nb = min(n_list - base, 32u);
+#pragma unroll 1
+									for (u32 j = 0; j < nb; j++) {
+										const u32 pr = s_list[base + j].pair;
+										const u64 jq = qrow0 + (pr & 63), jd = drow0 + ((pr >> 6) & 1) * 128 + quarter * 32 + ((pr >> 8) & 31);
+										const uint4 *a = reinterpret_cast<const uint4 *>(p.cumQ + jq * NBINS) + lane * 4;
+										const uint4 *b = reinterpret_cast<const uint4 *>(p.cumD + jd * NBINS) + lane * 4;
+										uint4 A[4], B[4];
+#pragma unroll
+										for (int i = 0; i < 4; i++) {
+											A[i] = __ldg(a + i);
+											B[i] = __ldg(b + i);
+										}
+										u32 acc = 0;
+#pragma unroll
+										for (int i = 0; i < 4; i++) {
+											acc = dp2a_sum(vmin2(A[i].x, B[i].x), acc);
+											acc = dp2a_sum(vmin2(A[i].y, B[i].y), acc);
+											acc = dp2a_sum(vmin2(A[i].z, B[i].z), acc);
+											acc = dp2a_sum(vmin2(A[i].w, B[i].w), acc);
+										}
+										acc = __reduce_add_sync(0xffffffffu, acc);
+										if ((u32)lane == j) {
+											smin = acc;
+										}
+									}
+								}
 								int close = 0;
 								double score = 0, d0v;
 								u64 cq = 0, cd = 0;
@@ -896,7 +996,7 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 									RedN rd;
 									rd.jeff = rd.js = 0;
 									rd.dot = c.dot;
-									rd.emd = c.emd;
+									rd.emd = COARSE ? p.csQ[cq] + p.csD[cd] - 2u * smin : c.emd; // u32, as the full form's
 									rd.smin = MIN ? (sd.sum + sq.sum - (u64)c.sad) >> 1 : 0;
 									const int bad = eval_pair_fast(dm, (u64)n_slabs * NBINS, rd, sd, sq, true, score, d0v, close);
 									if (bad) {
@@ -944,6 +1044,9 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 			if (lane == 0 && (lo | hi)) {
 				atomicAdd(p.counters + 1, ((u64)hi << 16) + lo);
 			}
+			if (lane == 0 && exact_total) { // warp-uniform
+				atomicAdd(p.counters + 2, exact_total);
+			}
 		}
 	}
 	tc_fence_before();
@@ -954,9 +1057,9 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 }
 
 // cumulative rows: warp per row, lane l owns bins [32 l, 32 l + 32); inclusive prefix, u16 (row sums < 65536), plus the
-// row's sum of prefixes for the EMD identity
+// row's sum of prefixes for the EMD identity and the samples at bins 16 j + 15 (j = 2 l, 2 l + 1) of the coarse form
 __global__ void __launch_bounds__(256) cum16_kernel(const unsigned char *__restrict__ bins, u64 n, unsigned short *__restrict__ cum,
-						    u32 *__restrict__ cumsum)
+						    u32 *__restrict__ cumsum, unsigned short *__restrict__ samples)
 {
 	const int lane = threadIdx.x & 31;
 	const u64 warps_total = (u64)gridDim.x * (blockDim.x >> 5);
@@ -995,6 +1098,7 @@ __global__ void __launch_bounds__(256) cum16_kernel(const unsigned char *__restr
 		dst[1] = make_uint4(out[4], out[5], out[6], out[7]);
 		dst[2] = make_uint4(out[8], out[9], out[10], out[11]);
 		dst[3] = make_uint4(out[12], out[13], out[14], out[15]);
+		reinterpret_cast<u32 *>(samples + r * 64)[lane] = (out[7] >> 16) | (out[15] & 0xFFFF0000u); // bins 32 l + 15, 32 l + 31
 		cs = __reduce_add_sync(0xffffffffu, cs);
 		if (lane == 0) {
 			cumsum[r] = cs;
@@ -1007,10 +1111,12 @@ __global__ void __launch_bounds__(256) cum16_kernel(const unsigned char *__restr
 // difference of cumulative values unchanged -- and brings rows whose sums reach 65536 only through the 4^k pseudo-counts
 // (k >= 6) back into 16 bits.  For uint16 bins the kernel also writes the row as bytes (the tensor-core and VABSDIFF4
 // operands).  flags: 1 a bin below base, 2 a uint16 bin above 255, 4 a cumulative value beyond 16 bits -- any of them
-// means the set cannot take the tile sweep with this base.
+// means the set cannot take the tile sweep with this base.  Rows of one slab also get the coarse form's samples (as
+// cum16_kernel).
 template <typename T>
 __global__ void __launch_bounds__(256) cum_wide_kernel(const T *__restrict__ bins, u64 n, u32 n_slabs, u32 base, unsigned short *__restrict__ cum,
-						       u32 *__restrict__ cumsum, unsigned char *__restrict__ plane, int *flags)
+						       u32 *__restrict__ cumsum, unsigned char *__restrict__ plane, unsigned short *__restrict__ samples,
+						       int *flags)
 {
 	const int lane = threadIdx.x & 31;
 	const u64 warps_total = (u64)gridDim.x * (blockDim.x >> 5);
@@ -1081,6 +1187,9 @@ __global__ void __launch_bounds__(256) cum_wide_kernel(const T *__restrict__ bin
 			dst[1] = make_uint4(out[4], out[5], out[6], out[7]);
 			dst[2] = make_uint4(out[8], out[9], out[10], out[11]);
 			dst[3] = make_uint4(out[12], out[13], out[14], out[15]);
+			if (samples && n_slabs == 1) { // bins 32 l + 15, 32 l + 31
+				reinterpret_cast<u32 *>(samples + r * 64)[lane] = (out[7] >> 16) | (out[15] & 0xFFFF0000u);
+			}
 			carry += __shfl_sync(0xffffffffu, x, 31);
 		}
 		cs = __reduce_add_sync(0xffffffffu, cs);
@@ -1148,12 +1257,15 @@ int ensure_tile_operands(mc2_ctx *ctx, const mc2_hset *hc, int base)
 	if (h->eb == 2 && !h->plane8) {
 		MC2_CUDA(cudaMalloc((void **)&h->plane8, h->n * N));
 	}
+	if (N == 1024 && !h->cum16s) {
+		MC2_CUDA(cudaMalloc((void **)&h->cum16s, h->n * 64 * 2));
+	}
 	h->cum_base = base;
 	u64 want = (h->n + 7) / 8, cap = (u64)ctx->sm_count * 8;
 	int grid = (int)(want < cap ? want : cap);
 	if (h->eb == 1 && N == 1024 && base == 0) {
 		prof_begin(ctx, 5);
-		ts::cum16_kernel<<<grid, 256, 0, ctx->stream>>>((const unsigned char *)h->bins, h->n, h->cum16, h->cumsum);
+		ts::cum16_kernel<<<grid, 256, 0, ctx->stream>>>((const unsigned char *)h->bins, h->n, h->cum16, h->cumsum, h->cum16s);
 		prof_end(ctx);
 		ctx->launches++;
 		MC2_CUDA(cudaGetLastError());
@@ -1166,10 +1278,10 @@ int ensure_tile_operands(mc2_ctx *ctx, const mc2_hset *hc, int base)
 	prof_begin(ctx, 5);
 	if (h->eb == 1) {
 		ts::cum_wide_kernel<unsigned char><<<grid, 256, 0, ctx->stream>>>((const unsigned char *)h->bins, h->n, (u32)(N / 1024), (u32)base,
-										      h->cum16, h->cumsum, nullptr, d_flags);
+										      h->cum16, h->cumsum, nullptr, h->cum16s, d_flags);
 	} else {
 		ts::cum_wide_kernel<unsigned short><<<grid, 256, 0, ctx->stream>>>((const unsigned short *)h->bins, h->n, (u32)(N / 1024), (u32)base,
-										       h->cum16, h->cumsum, h->plane8, d_flags);
+										       h->cum16, h->cumsum, h->plane8, h->cum16s, d_flags);
 	}
 	prof_end(ctx);
 	ctx->launches++;
@@ -1261,17 +1373,24 @@ bool tile_sweep_supported(const DevModel &dm, const mc2_hset *q, const mc2_hset 
 	return model && tile_sweep_shape_ok(q, d);
 }
 
-template <int NEED, bool RAW> static int launch_need(int grid, cudaStream_t st, const DevModel &dm, const ts::Params &p, const CUtensorMap *m)
+template <int NEED, bool RAW, bool ONE, bool COARSE>
+static int launch_form(int grid, cudaStream_t st, const DevModel &dm, const ts::Params &p, const CUtensorMap *m)
 {
 	const int smem = ts::Smem<NEED>::TOTAL;
-	if (p.n_slabs == 1) {
-		MC2_CUDA(cudaFuncSetAttribute(ts::tile_sweep_kernel<NEED, RAW, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-		ts::tile_sweep_kernel<NEED, RAW, true><<<grid, ts::THREADS, smem, st>>>(dm, p, m[0], m[1], m[2], m[3]);
-	} else {
-		MC2_CUDA(cudaFuncSetAttribute(ts::tile_sweep_kernel<NEED, RAW, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-		ts::tile_sweep_kernel<NEED, RAW, false><<<grid, ts::THREADS, smem, st>>>(dm, p, m[0], m[1], m[2], m[3]);
-	}
+	MC2_CUDA(cudaFuncSetAttribute(ts::tile_sweep_kernel<NEED, RAW, ONE, COARSE>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+	ts::tile_sweep_kernel<NEED, RAW, ONE, COARSE><<<grid, ts::THREADS, smem, st>>>(dm, p, m[0], m[1], m[2], m[3]);
 	return MC2_OK;
+}
+
+template <int NEED, bool RAW>
+static int launch_need(int grid, cudaStream_t st, const DevModel &dm, const ts::Params &p, const CUtensorMap *m, bool coarse)
+{
+	if constexpr ((NEED & NEED_EMD) != 0 && !RAW) {
+		if (coarse) {
+			return launch_form<NEED, false, true, true>(grid, st, dm, p, m);
+		}
+	}
+	return p.n_slabs == 1 ? launch_form<NEED, RAW, true, false>(grid, st, dm, p, m) : launch_form<NEED, RAW, false, false>(grid, st, dm, p, m);
 }
 
 int launch_tile_sweep(mc2_ctx *ctx, const DevModel &dm, int need, const mc2_hset *q, u64 q0, u64 q1, const mc2_hset *d, u64 d0, u64 d1,
@@ -1334,7 +1453,18 @@ int launch_tile_sweep(mc2_ctx *ctx, const DevModel &dm, int need, const mc2_hset
 	ctx->launches++;
 	CUtensorMap maps[4];
 	memset(maps, 0, sizeof maps);
-	if (need & NEED_EMD) {
+	// the coarse form wherever the screen runs on rows of one slab: its cumulative stage is the 64 samples per row, and
+	// the full rows are read for the screen's survivors only.  Raw mode, models without a screen (an identity search
+	// with t <= 0 among them) and wider rows take the full form.
+	const bool coarse = (need & NEED_EMD) && !raw && p.n_slabs == 1 && dm.scr_ok && q->cum16s && d->cum16s;
+	if (coarse) {
+		p.cumQ = q->cum16; p.cumD = d->cum16;
+		p.smpQ = q->cum16s; p.smpD = d->cum16s;
+		rc = make_map(&maps[0], d->cum16s, d->n, 64, 2, ts::TD);
+		if (rc != MC2_OK) return rc;
+		rc = make_map(&maps[1], q->cum16s, q->n, 64, 2, ts::TQ);
+		if (rc != MC2_OK) return rc;
+	} else if (need & NEED_EMD) {
 		rc = make_map(&maps[0], d->cum16, d->n, d->N, 2, ts::TD);
 		if (rc != MC2_OK) return rc;
 		rc = make_map(&maps[1], q->cum16, q->n, q->N, 2, ts::TQ);
@@ -1352,8 +1482,8 @@ int launch_tile_sweep(mc2_ctx *ctx, const DevModel &dm, int need, const mc2_hset
 	switch (need & 7) {
 #define MC2_TS_CASE(n)                                                                                  \
 	case n:                                                                                         \
-		rc = raw ? launch_need<n, true>(grid, ctx->stream, dm, p, maps)           \
-			 : launch_need<n, false>(grid, ctx->stream, dm, p, maps);         \
+		rc = raw ? launch_need<n, true>(grid, ctx->stream, dm, p, maps, false)    \
+			 : launch_need<n, false>(grid, ctx->stream, dm, p, maps, coarse); \
 		break;
 		MC2_TS_CASE(1)
 		MC2_TS_CASE(2)
