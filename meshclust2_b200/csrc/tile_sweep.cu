@@ -7,8 +7,9 @@
 //
 // One persistent CTA per SM (28 warps, warp specialised, registers re-dealt per warpgroup with setmaxnreg) walks
 // 64 (query) x 256 (database) pair tiles in the order of a precomputed schedule (database-tile major inside super-rows
-// of query tiles, so concurrently running CTAs share tiles in L2).  Per tile the bins stream through a 4-stage
-// shared-memory ring of 40 KB stages filled by TMA (cp.async.bulk.tensor.2d, SWIZZLE_128B, one elected producer thread):
+// of query tiles, so concurrently running CTAs share tiles in L2).  Per tile the bins stream through a 4-stage (coarse
+// form without SAD sums: 2-stage) shared-memory ring of 40 KB stages filled by TMA (cp.async.bulk.tensor.2d,
+// SWIZZLE_128B, one elected producer thread):
 // per 1024 bins 16 stages of 64 bins of the u16 cumulative rows and 8 stages of 128 bins of the u8 rows, interleaved 2 : 1.
 // Rows of several slabs (k >= 6) and uint16 bins: the cumulative rows are those of (bin - pseudo-count), which keeps them
 // in 16 bits without changing any difference cumP - cumQ, and uint16 bins below 256 travel as a byte plane (cum_wide_kernel).
@@ -24,7 +25,8 @@
 //                                The sums go to TMEM (tcgen05.st) for the epilogue warps, double buffered.
 //   S_sad = sum |p - q|          VABSDIFF4.U8.ACC on the u8 stages (4 bins / instruction) -> S_min = (sumP+sumQ-S_sad)/2
 // Epilogue (8 warps, thread = TMEM lane, two warps per lane quarter splitting the query columns; one warp per scheduler
-// is latency bound and stalls the compute warps at the tile hand-over): tcgen05.ld of 4 (or 2) query columns at a time; length window
+// is latency bound and stalls the compute warps at the tile hand-over; 16 epilogue and 8 compute warps in the coarse
+// form without SAD sums, see Layout): tcgen05.ld of 4 (or 2) query columns at a time; length window
 // (FC_Runner.cpp:435-444) in 32 bits with an exact 64-bit path for lengths >= 2^32; an fp32 evaluation of the GLM sum
 // with a rigorous host-derived error bound that can only REJECT (sum + bound < logit(0.5 - bias) - 1e-6 => not close
 // whatever the rounding); the rest is ballot-compacted into a per-warp list and goes, one pair per lane, through the exact fp64
@@ -35,8 +37,9 @@
 // values at the 64 block ends s_j = 16 j + 15 (mc2_hset::cum16s, one ring stage) bound the whole sum:
 // 16 (M - T) <= sum_i m_i <= 16 M with M = sum_j m(s_j), T = m(s_63) = min(totP, totQ).  A tile streams the 8 u8 stages
 // and that single stage; the screen takes the EMD as the interval [cs - 32 M, cs - 32 (M - T)] and the candidates it
-// keeps get the exact sum min(cumP, cumQ) over the full rows from global memory (one warp per candidate) before the same
-// exact epilogue, so scores and decisions are the bits of the full form.
+// keeps get the exact sum min(cumP, cumQ) over the full rows from global memory (one warp per candidate; the rows are
+// prefetched into L2 when the screen keeps the pair) before the same exact epilogue, so scores and decisions are the bits
+// of the full form.
 // Identity search (Params::identity, mc2_identity_pairs): a regression model, clamp(sum) >= t <=> sum >= t for 0 < t <= 1,
 // so the same screen rejects on sum + bound < t - margin (DevModel::scr_thr, set per call) and the exact epilogue keeps
 // the pairs whose clamped sum is >= t.  The mode is a uniform runtime field read by the epilogue warps only.
@@ -55,42 +58,46 @@ constexpr int TD = 256;         // database rows per tile: two regions of 128 (U
 constexpr int NBINS = 1024;      // bins per slab; rows are Params::n_slabs slabs long
 constexpr int KC_CUM = 64;      // bins per ring stage while the u16 cumulative rows stream (128-byte rows)
 constexpr int KC_U8 = 128;      // bins per ring stage while the u8 rows stream (128-byte rows)
-#ifndef MC2_TS_NCW
-#define MC2_TS_NCW 16
-#endif
-constexpr int NCW = MC2_TS_NCW; // compute warps (CTA warps 4 .. 4 + NCW - 1, whole warpgroups): 8 or 16
-constexpr int QN = TQ / (NCW / 4); // query rows per compute thread (x 2 database rows): 32 or 16 accumulator pairs
-// measured on 100 k x 1 kb (bench model), ms per 1.8e9 pairs: 4 epilogue warps x 4 pairs per thread 95.6, 8 x 2: 91.5,
-// 4 x 2: 105.7
-#ifndef MC2_TS_NEW
-#define MC2_TS_NEW 8
-#endif
-constexpr int NEW = MC2_TS_NEW; // epilogue warps (after the compute warps, whole warpgroups): NEW / 4 per TMEM lane quarter, each
-                                // taking TQ / (NEW / 4) query columns of both regions
-// pairs a thread of the epilogue screens at a time (query columns per tcgen05.ld): 4 where the screen's scratch
-// (slots x pairs x 256 threads x 4 bytes) leaves room for a candidate list that is flushed once per tile, else 2
-#ifdef MC2_TS_NP
-constexpr int np_of(int) { return MC2_TS_NP; }
-#else
-constexpr int np_of(int need) { return scr_slots(need) <= 7 ? 4 : 2; }
-#endif
-constexpr int list_cap_of(int need) { return NEW == 8 ? (np_of(need) == 4 ? 192 : 128) : 256; } // candidate records per epilogue warp
-constexpr int QE = TQ / (NEW / 4); // query columns per epilogue warp
-constexpr int THREADS = (4 + NCW + NEW) * 32; // warpgroup 0: TMA producer, MMA issuer, two idle warps
-// setmaxnreg per warpgroup.  The pool is what the launch allocated (threads x launch registers, at most 64 K): the
-// per-role sums below must not exceed it.
-//   8 compute + 4 epilogue warps: launch 128, control 40, compute 168, epilogue 128
-//  16 compute + 4 epilogue warps: launch  80, control 40, compute  80, epilogue 120
-//  16 compute + 8 epilogue warps: launch  72, control 24, compute  80, epilogue  80
-constexpr int REGS_LAUNCH = NEW == 8 ? 72 : (NCW == 8 ? 128 : 80);
-constexpr int REGS_CTRL = NEW == 8 ? 24 : 40, REGS_COMPUTE = NCW == 8 ? 168 : 80, REGS_EPI = NEW == 8 ? 80 : (NCW == 8 ? 128 : 120);
-static_assert(128 * REGS_CTRL + NCW * 32 * REGS_COMPUTE + NEW * 32 * REGS_EPI <= THREADS * REGS_LAUNCH, "register pool");
-static_assert(THREADS * REGS_LAUNCH <= 65536, "register file");
 constexpr int D_BYTES = TD * 128;        // 32 KB, SWIZZLE_128B
 constexpr int Q_BYTES = TQ * 128;        //  8 KB
 constexpr int STAGE_BYTES = D_BYTES + Q_BYTES; // 40 KB
-constexpr int STAGES = 4;
 constexpr int MAX_SUPER = 1024;          // entries of the tile schedule's prefix array
+
+// Warp layout of an instantiation, in whole warpgroups (setmaxnreg is per warpgroup, and a warp reaches only the TMEM lane
+// quarter warp % 4).  Warpgroup 0: TMA producer, MMA issuer, two idle warps; then NCW compute warps; then NEW epilogue
+// warps, NEW / 4 per TMEM lane quarter, each taking QE query columns of both regions.
+//  - full form, and the coarse form with SAD sums (its compute warps still stream the eight u8 stages): 16 compute +
+//    8 epilogue warps, a 4-stage ring.  Measured on 100 k x 1 kb (bench model, full form), ms per 1.8e9 pairs: 4 epilogue
+//    warps x 4 pairs per thread 95.6, 8 x 2: 91.5, 4 x 2: 105.7.
+//  - coarse form without SAD sums: the compute warps work on one ring stage of nine (the 64 samples) and the epilogue's
+//    per-pair work paces the tile, so the warps go the other way: 8 compute + 16 epilogue warps.  A compute thread then
+//    covers 32 query rows, in two passes of 16 stored to TMEM one after the other (80 registers).  The screen's scratch
+//    grows with the epilogue threads (NEED 6: 7 slots x 4 pairs x 512 threads x 4 B = 56 KiB), which leaves room for a
+//    2-stage ring: a tile streams 9 stages, and the MMAs and sample sums of the next tile overlap this tile's epilogue
+//    through the double-buffered TMEM.
+// Registers (setmaxnreg per warpgroup; the pool is threads x launch registers, at most 64 K) are the same for both:
+// launch 72, control 24, compute 80, epilogue 80 = 128 x 24 + 512 x 80 + 256 x 80 = 28 x 32 x 72.
+template <int NEED, bool COARSE> struct Layout {
+	static constexpr bool EPI_HEAVY = COARSE && (NEED & NEED_MIN) == 0;
+	static constexpr int NCW = EPI_HEAVY ? 8 : 16;
+	static constexpr int NEW = EPI_HEAVY ? 16 : 8;
+	static constexpr int THREADS = (4 + NCW + NEW) * 32;
+	static constexpr int QN = 16;                      // query rows per compute pass (x 2 database rows): 32 accumulators
+	static constexpr int QPASS = TQ / (NCW / 4) / QN;  // passes per stage over a compute warpgroup's TQ / (NCW / 4) rows
+	static constexpr int QE = TQ / (NEW / 4);          // query columns per epilogue warp
+	// pairs a thread of the epilogue screens at a time (query columns per tcgen05.ld): 4 where the screen's scratch
+	// (slots x pairs x NEW * 32 threads x 4 bytes) leaves room for a candidate list that is flushed once per tile, else 2
+	static constexpr int NP = scr_slots(NEED & 7) <= 7 ? 4 : 2;
+	static constexpr int LIST_CAP = NP == 4 ? 192 : 128; // candidate records per epilogue warp
+	static constexpr int STAGES = EPI_HEAVY ? 2 : 4;
+	static constexpr int REGS_LAUNCH = 72, REGS_CTRL = 24, REGS_COMPUTE = 80, REGS_EPI = 80;
+	static_assert(NCW % 4 == 0 && NEW % 4 == 0, "roles are whole warpgroups");
+	static_assert(QPASS >= 1 && QPASS * QN * (NCW / 4) == TQ && QE * (NEW / 4) == TQ && QE % NP == 0, "query rows and columns");
+	static_assert(QPASS == 1 || (COARSE && (NEED & NEED_MIN) == 0), "several passes only over the one sample stage");
+	static_assert(128 * REGS_CTRL + NCW * 32 * REGS_COMPUTE + NEW * 32 * REGS_EPI <= THREADS * REGS_LAUNCH, "register pool");
+	static_assert(THREADS * REGS_LAUNCH <= 65536 && 65536 / THREADS >= REGS_LAUNCH, "register file");
+	static_assert(LIST_CAP >= 32 * NP, "a batch of candidates fits the list");
+};
 // TMEM columns (512 allocated): Gram accumulators double buffered, EMD / SAD sums single buffered
 constexpr u32 TM_DOT = 0;                // + buf * 128 + region * 64
 constexpr u32 TM_EMD = 256;              // + ebuf * 128 + region * 64 (double buffered when no SAD sums are needed)
@@ -209,6 +216,11 @@ __device__ __forceinline__ void tc_st16(u32 taddr, const u32 (&v)[16])
 __device__ __forceinline__ void tc_st(u32 taddr, const u32 (&v)[32]) { tc_st32(taddr, v); }
 __device__ __forceinline__ void tc_st(u32 taddr, const u32 (&v)[16]) { tc_st16(taddr, v); }
 __device__ __forceinline__ void tc_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
+// bulk prefetch of global memory into L2 (no registers, no completion to wait for)
+__device__ __forceinline__ void l2_prefetch(const void *ptr, u32 bytes)
+{
+	asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(ptr), "r"(bytes) : "memory");
+}
 __device__ __forceinline__ void named_sync(int id, int threads) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(threads) : "memory"); }
 __device__ __forceinline__ uint4 lds128(u32 addr)
 {
@@ -309,15 +321,16 @@ __device__ __forceinline__ Tile decode_item(const Params &p, const u32 *s_sched,
 
 // ---------------------------------------------------------------------------------------------------------------
 // CUDA-core work of one compute warp on one ring stage.  The thread owns database rows L and 128 + L of the tile
-// (L = 32 * (warp % 4) + lane, its TMEM lane) against the QN query rows of its share: 2 * QN accumulators (QN = 16 with
-// 16 compute warps).  Per 16-byte step: 2 conflict-free row loads, QN warp-uniform (broadcast) query loads, 16 * QN (EMD:
-// VIMNMX.U16x2 + IDP.2A per word) or 8 * QN (SAD: VABSDIFF4 per word) arithmetic instructions.
+// (L = 32 * (warp % 4) + lane, its TMEM lane) against QN query rows of its share: 2 * QN accumulators (QN = 16).  Per
+// 16-byte step: 2 conflict-free row loads, QN warp-uniform (broadcast) query loads, 16 * QN (EMD: VIMNMX.U16x2 + IDP.2A
+// per word) or 8 * QN (SAD: VABSDIFF4 per word) arithmetic instructions.
 // 128-byte rows under SWIZZLE_128B: 16-byte chunk c of row r sits at r * 128 + ((c ^ (r & 7)) << 4).
 // ---------------------------------------------------------------------------------------------------------------
-template <bool IS_EMD>
+template <bool IS_EMD, int QN>
 __device__ __forceinline__ void stage_compute(const unsigned char *stage, u32 lane_row, int qsel, u32 (&acc)[2][QN])
 {
-	// plain loads (not asm): the compiler may order and pipeline them freely inside the stage
+	// plain loads (not asm): the compiler may order and pipeline them freely inside the stage.  Query rows QN * qsel ..
+	// QN * qsel + QN - 1
 	const uint4 *dptr = reinterpret_cast<const uint4 *>(stage) + lane_row * 8;
 	const uint4 *qptr = reinterpret_cast<const uint4 *>(stage + D_BYTES) + qsel * (QN * 8);
 	const u32 dsw = lane_row & 7;
@@ -411,17 +424,16 @@ __device__ __forceinline__ float sqrt_approx(float x)
 	return r;
 }
 
-// sx: this thread's column of the epilogue's scratch, element (slot, t) at sx[(slot * NP + t) * (NEW * 32)]; slot = single
-// slot (scr_slot), the last slot holds the constant 1 (written once per kernel)
+// sx: this thread's column of the epilogue's scratch, element (slot, t) at sx[(slot * NP + t) * ET] (ET: epilogue
+// threads); slot = single slot (scr_slot), the last slot holds the constant 1 (written once per kernel)
 // COARSE: the EMD is only known to lie in [emd[t], emd_hi[t]] (exact integers).  x is evaluated at both ends, u covers
 // both, and a combo with the EMD factor adds the larger of its values at the two ends: the other factor is fixed, so the
 // combo is linear in x or in x^2, and x^2 over an interval that spans 0 also takes the value 0 (the fused sums are
 // monotone in the exact value, so max(fma(w, f1, s), fma(w, f2, s)) = fl(max(w f1, w f2) + s) keeps the error model).
-template <int NEED, int NP, bool COARSE>
+template <int NEED, int NP, bool COARSE, int ET>
 __device__ __forceinline__ u32 screen_pairs(const DevModel &dm, float *sx, const u32 (&dot)[NP], const u32 (&emd)[NP], const u32 (&emd_hi)[NP],
 					    const u32 (&sad)[NP], const RowF &P, const RowF *Q)
 {
-	constexpr int ET = NEW * 32;
 	float m[NP];
 #pragma unroll
 	for (int t = 0; t < NP; t++) {
@@ -541,31 +553,34 @@ struct Cand {
 	u32 dot, emd, sad;
 };
 
-template <int NEED> struct Smem {
-	static constexpr int NP = np_of(NEED & 7), LIST_CAP = list_cap_of(NEED & 7);
+template <int NEED, bool COARSE> struct Smem {
+	using LY = Layout<NEED, COARSE>;
 	static constexpr int RING = 0;
-	static constexpr int LIST = STAGES * STAGE_BYTES;                         // Cand[NEW][LIST_CAP]
-	static constexpr int SCRX = LIST + NEW * LIST_CAP * (int)sizeof(Cand);    // float [slots][NP][NEW * 32]: the screen's scratch
-	static constexpr int ROWQ = SCRX + scr_slots(NEED & 7) * NP * NEW * 32 * 4; // RowF[2][TQ]
-	static constexpr int WINQ = ROWQ + 2 * TQ * (int)sizeof(RowF);            // u64 window [2][TQ][2]
-	static constexpr int WIN32 = WINQ + 2 * TQ * 16;                          // uint2 window [2][TQ], saturated to 32 bits
-	static constexpr int SCHED = WIN32 + 2 * TQ * 8;                          // u32 [MAX_SUPER + 1]
-	static constexpr int BARS = SCHED + (MAX_SUPER + 1) * 4 + 4;              // mbarriers
-	static constexpr int MISC = BARS + 32 * 8;                                // tmem base
-	static constexpr int TOTAL = MISC + 64 + 1024;                            // + alignment slack
+	static constexpr int LIST = LY::STAGES * STAGE_BYTES;                             // Cand[NEW][LIST_CAP]
+	static constexpr int SCRX = LIST + LY::NEW * LY::LIST_CAP * (int)sizeof(Cand);     // float [slots][NP][NEW * 32]: the screen's scratch
+	static constexpr int ROWQ = SCRX + scr_slots(NEED & 7) * LY::NP * LY::NEW * 32 * 4; // RowF[2][TQ]
+	static constexpr int WINQ = ROWQ + 2 * TQ * (int)sizeof(RowF);                    // u64 window [2][TQ][2]
+	static constexpr int WIN32 = WINQ + 2 * TQ * 16;                                  // uint2 window [2][TQ], saturated to 32 bits
+	static constexpr int SCHED = WIN32 + 2 * TQ * 8;                                  // u32 [MAX_SUPER + 1]
+	static constexpr int BARS = SCHED + (MAX_SUPER + 1) * 4 + 4;                      // mbarriers
+	static constexpr int MISC = BARS + 32 * 8;                                        // tmem base
+	static constexpr int TOTAL = MISC + 64 + 1024;                                    // + alignment slack
+	static_assert(2 * LY::STAGES + 8 <= 32, "mbarriers");
 	static_assert(TOTAL <= 232448, "shared memory per CTA");
 };
 
 // ONE: rows of one 1 KiB slab (k = 5), stage counts known at compile time; otherwise Params::n_slabs slabs per row.
 // COARSE: the coarse form (header comment); the cumulative tensor maps are those of the samples (64 per row)
 template <int NEED, bool RAW, bool ONE, bool COARSE>
-__global__ void __launch_bounds__(THREADS, 1)
+__global__ void __launch_bounds__(Layout<NEED, COARSE>::THREADS, 1)
 tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ Params p, const __grid_constant__ CUtensorMap mapCumD,
 		  const __grid_constant__ CUtensorMap mapCumQ, const __grid_constant__ CUtensorMap mapU8D,
 		  const __grid_constant__ CUtensorMap mapU8Q)
 {
-	using L = Smem<NEED>;
-	constexpr int NP = L::NP, LIST_CAP = L::LIST_CAP;
+	using L = Smem<NEED, COARSE>;
+	using LY = Layout<NEED, COARSE>;
+	constexpr int NCW = LY::NCW, NEW = LY::NEW, STAGES = LY::STAGES, QN = LY::QN, QE = LY::QE, NP = LY::NP, LIST_CAP = LY::LIST_CAP;
+	constexpr int REGS_LAUNCH = LY::REGS_LAUNCH, REGS_CTRL = LY::REGS_CTRL, REGS_COMPUTE = LY::REGS_COMPUTE, REGS_EPI = LY::REGS_EPI;
 	constexpr bool DOT = (NEED & NEED_DOT) != 0, EMD = (NEED & NEED_EMD) != 0, MIN = (NEED & NEED_MIN) != 0;
 	static_assert(!COARSE || (ONE && EMD && !RAW), "the coarse form is for one-slab rows, a model with EMD, scoring");
 	constexpr bool U8_PHASE = DOT || MIN;
@@ -701,7 +716,7 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 		}
 		const int cw = warp - 4;
 		const u32 quarter = (u32)warp & 3;          // the TMEM lanes this warp may touch: 32 * quarter ..
-		const int qsel = cw >> 2;                   // query rows QN * qsel .. of the tile
+		const int qsel = cw >> 2;                   // query rows QN * QPASS * qsel .. of the tile
 		const u32 lane_row = quarter * 32 + (u32)lane;
 		const u32 tlane = (quarter * 32) << 16;
 		u32 s = 0, ph = 0, it = 0;
@@ -769,7 +784,35 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 					tc_st(tmem_base + tlane + TM_SAD + 64 + qsel * QN, acc[1]);
 				}
 			}
-			if (!INTERLEAVE && EMD) {
+			if (!INTERLEAVE && EMD && LY::QPASS > 1) {
+				// the one sample stage, the warpgroup's query rows in passes of QN: each pass goes to TMEM before the next
+				// one reuses the accumulators
+				mbar_wait(bar_full + s * 8, ph, p.err, p.sleep_comp);
+#pragma unroll 1
+				for (int h = 0; h < LY::QPASS; h++) {
+					u32 acc[2][QN];
+#pragma unroll
+					for (int q = 0; q < QN; q++) {
+						acc[0][q] = acc[1][q] = 0;
+					}
+					stage_compute<true>(smem + s * STAGE_BYTES, lane_row, qsel * LY::QPASS + h, acc);
+					if (h == 0) {
+						mbar_wait(bar_eempty + eb * 8, (eit & 1) ^ 1, p.err, p.sleep_comp);
+						tc_fence_after();
+					}
+					tc_st(tmem_base + tlane + TM_EMD + eb * 128 + (qsel * LY::QPASS + h) * QN, acc[0]);
+					tc_st(tmem_base + tlane + TM_EMD + eb * 128 + 64 + (qsel * LY::QPASS + h) * QN, acc[1]);
+				}
+				__syncwarp();
+				if (lane == 0) {
+					mbar_arrive(bar_empty + s * 8);
+				}
+				if (++s == (u32)STAGES) {
+					s = 0;
+					ph ^= 1;
+				}
+			}
+			if (!INTERLEAVE && EMD && LY::QPASS == 1) {
 				u32 acc[2][QN];
 #pragma unroll
 				for (int q = 0; q < QN; q++) {
@@ -927,7 +970,7 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 							anybig |= Q[k].big;
 						}
 						if (can_screen && __any_sync(0xffffffffu, cand != 0 && !anybig)) {
-							const u32 maybe = screen_pairs<NEED, NP, COARSE>(dm, sx, vd, ve, ve_hi, vs, PD[r], Q);
+							const u32 maybe = screen_pairs<NEED, NP, COARSE, NEW * 32>(dm, sx, vd, ve, ve_hi, vs, PD[r], Q);
 							if (!anybig) {
 								cand &= maybe;
 							}
@@ -945,6 +988,13 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 								rec.emd = ve[k];
 								rec.sad = vs[k];
 								s_list[n_list + __popc(m & ((1u << lane) - 1))] = rec;
+								if constexpr (COARSE) {
+									// the flush refines one candidate at a time, and each reads both full cumulative
+									// rows (cum16 is larger than L2): start bringing them into L2 now, so that the
+									// flush's loads wait for L2 and not for a DRAM round trip each
+									l2_prefetch(p.cumQ + (qrow0 + qc + k) * NBINS, NBINS * 2);
+									l2_prefetch(p.cumD + d * NBINS, NBINS * 2);
+								}
 							}
 							n_list += __popc(m);
 						}
@@ -1376,9 +1426,9 @@ bool tile_sweep_supported(const DevModel &dm, const mc2_hset *q, const mc2_hset 
 template <int NEED, bool RAW, bool ONE, bool COARSE>
 static int launch_form(int grid, cudaStream_t st, const DevModel &dm, const ts::Params &p, const CUtensorMap *m)
 {
-	const int smem = ts::Smem<NEED>::TOTAL;
+	const int smem = ts::Smem<NEED, COARSE>::TOTAL;
 	MC2_CUDA(cudaFuncSetAttribute(ts::tile_sweep_kernel<NEED, RAW, ONE, COARSE>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-	ts::tile_sweep_kernel<NEED, RAW, ONE, COARSE><<<grid, ts::THREADS, smem, st>>>(dm, p, m[0], m[1], m[2], m[3]);
+	ts::tile_sweep_kernel<NEED, RAW, ONE, COARSE><<<grid, ts::Layout<NEED, COARSE>::THREADS, smem, st>>>(dm, p, m[0], m[1], m[2], m[3]);
 	return MC2_OK;
 }
 
