@@ -241,6 +241,16 @@ int mc2_hset_set_row(mc2_ctx *ctx, mc2_hset *dst, uint64_t dst_row, const mc2_hs
 int mc2_hset_assign_rows(mc2_ctx *ctx, mc2_hset *dst, uint64_t n, const uint64_t *dst_rows, const mc2_hset *src,
 			 const uint64_t *src_rows, const uint64_t *mag, const uint64_t *len);
 
+/* The other strand: row i of *out is the histogram of the reverse complement of the sequence row i of src counted.  The
+ * bin index is the big-endian base-4 k-mer (A=0, C=1, G=2, T=3), so out[i][rc(j)] = src[i][j] with
+ * rc(j) = reverse_base4_digits(j) XOR (4^k - 1); this is exact, saturated bins included (rc is a bijection on k-mers, a bin
+ * is min(max(T), 1 + count) whatever the order of the bases, and mirroring a segment maps its k-mers to their reverse
+ * complements).  Every k (1..12) and width.  Side-band: mag (stale or not), len, the true sums, stddev and the per-row
+ * largest count are copied; the k = 1 table swaps A<->T and C<->G; mc2_hset_largest_count answers as for src.  The
+ * per-row count of overflowing segments depends on segment order, which reversal changes: *out reports 0, as a set made by
+ * mc2_hset_from_host does.  Derived operands that depend on bin order are built for *out when first needed. */
+int mc2_hset_reverse_complement(mc2_ctx *ctx, const mc2_hset *src, mc2_hset **out);
+
 /* ---- model -------------------------------------------------------------------------------------- */
 int mc2_model_create(mc2_ctx *ctx, const mc2_model_desc *desc, mc2_model **out);
 void mc2_model_free(mc2_model *m);
@@ -358,6 +368,29 @@ int mc2_identity_pairs(mc2_ctx *ctx, const mc2_model *model, double min_identity
 		       uint64_t max_out, uint64_t *out_q, uint64_t *out_d, double *out_identity, uint64_t *n_out,
 		       uint64_t *n_scored);
 
+/* Both-strand identity search: mc2_identity_pairs over each in-window (query, database) pair on both strands of the query.
+ * id+ = similarity(database d, query q) as mc2_identity_pairs scores it; id- = similarity(database d, reverse complement of q)
+ * (mc2_hset_reverse_complement: only the query is flipped, the database stays forward).  A pair survives iff
+ * max(id+, id-) >= min_identity; out_identity[i] is that max and out_strand[i] the strand it came from, 0 forward or 1
+ * reverse, a tie (equal values) going to forward.  out_identity[i] is the same bits as the score mc2_score_pairs gives the pair
+ * on the reported strand (set_a = set_d row out_d[i], set_b = set_q or its reverse-complement set, row out_q[i]).
+ * The reverse complement has the query's length, so both strands have the same length window and *n_scored is the number
+ * mc2_identity_pairs reports.  Ranges, window, upper_only (c > r on row indices, which the reverse-complement rows keep),
+ * capacity (*n_out is the total, which may exceed max_out; out_strand may be NULL), the unspecified survivor order and the
+ * error codes are those of mc2_identity_pairs.
+ * How: the forward sweep gives A = {id+ >= t}, at most max_out of it kept; the reverse sweep over the reverse-complement
+ * rows gives B = {id- >= t}, query-row block by block into a fixed scratch of max(d_end - d_begin, 2^20) pairs (a block
+ * whose survivors overflow it is split and swept again); id+ is recomputed for B's pairs and those with id+ < t join A;
+ * id- is scored for the returned members of A.  Extra device memory does not grow with the number of survivors.  For
+ * min_identity <= 0 every in-window pair is in A and only the returned entries' id- is scored.  The reverse-complement set
+ * of set_q is built on first use and kept with set_q until its bins, magnitudes or lengths change.
+ * mc2_debug_last_sweep afterwards: n_exact summed over every sweep of both strands, coarse = 1 iff every sweep took the
+ * coarse form. */
+int mc2_identity_pairs_both_strands(mc2_ctx *ctx, const mc2_model *model, double min_identity, const mc2_hset *set_q,
+				    uint64_t q_begin, uint64_t q_end, const mc2_hset *set_d, uint64_t d_begin, uint64_t d_end,
+				    int32_t upper_only, double cutoff, uint64_t max_out, uint64_t *out_q, uint64_t *out_d,
+				    double *out_identity, int8_t *out_strand, uint64_t *n_out, uint64_t *n_scored);
+
 /* Measured issue rate (warp-instructions per second, whole GPU) of the tile sweep's inner instruction pair -- VIMNMX.U16x2 on
  * the ALU pipe feeding IDP.2A on the FMA pipe, register operands only, 32 resident warps per SM: the denominator of
  * bench.py's roofline for the CUDA-core EMD term (SURVEY.md section 8d: "achieved ... vs a measured ALU peak"). */
@@ -372,8 +405,8 @@ int mc2_bench_issue_rate(mc2_ctx *ctx, int iters, double *warp_instr_per_s);
 int mc2_debug_tile_reductions(mc2_ctx *ctx, const mc2_hset *set_q, uint64_t q_begin, uint64_t q_end, const mc2_hset *set_d,
 			      uint64_t d_begin, uint64_t d_end, int32_t need, uint32_t *out_dot, uint32_t *out_emd, uint32_t *out_sad);
 
-/* Diagnostic (tests, benchmarks): of the last mc2_all_pairs / mc2_identity_pairs call on this context, *n_exact = the pairs
- * the tile sweep sent through the exact fp64 epilogue (those its fp32 screen could not reject; 0 for the row-streaming
+/* Diagnostic (tests, benchmarks): of the last mc2_all_pairs / mc2_identity_pairs call on this context (for
+ * mc2_identity_pairs_both_strands see there), *n_exact = the pairs the tile sweep sent through the exact fp64 epilogue (those its fp32 screen could not reject; 0 for the row-streaming
  * kernels) and *coarse = 1 if it took the coarse form (the screen on 64 sampled cumulative bins), else 0. */
 int mc2_debug_last_sweep(mc2_ctx *ctx, uint64_t *n_exact, int32_t *coarse);
 

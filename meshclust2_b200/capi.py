@@ -37,8 +37,8 @@ SYMBOLS = [
     "mc2_ctx_launch_count", "mc2_ctx_profile", "mc2_ctx_kernel_time", "mc2_ctx_flush_l2", "mc2_seqs_upload", "mc2_seqs_upload_into", "mc2_seqs_from_text", "mc2_seqs_from_text_into", "mc2_seqs_download_segments", "mc2_seqs_total_segments", "mc2_host_register", "mc2_host_unregister", "mc2_seqs_free", "mc2_seqs_count",
     "mc2_seqs_total_bases", "mc2_count_kmers", "mc2_count_kmers_into", "mc2_count_kmers_auto", "mc2_hset_largest_count", "mc2_hset_alloc", "mc2_count_kmers_into_rows", "mc2_hset_refresh", "mc2_width_for_count", "mc2_kmer_table_increment", "mc2_hset_from_host", "mc2_hset_from_device", "mc2_hset_update_from_device", "mc2_hset_device_sideband", "mc2_hset_free",
     "mc2_hset_count", "mc2_hset_k", "mc2_hset_elem_bytes", "mc2_hset_device_bins", "mc2_hset_download", "mc2_hset_copy_to_device",
-    "mc2_hset_set_sideband", "mc2_hset_set_row", "mc2_hset_assign_rows", "mc2_model_create", "mc2_model_free", "mc2_model_desc_from_file",
-    "mc2_score_pairs", "mc2_get_close", "mc2_get_close_as", "mc2_filter", "mc2_filter_as", "mc2_merge", "mc2_all_pairs", "mc2_identity_pairs", "mc2_debug_tile_reductions", "mc2_debug_last_sweep", "mc2_distance", "mc2_mean_closest", "mc2_closest",
+    "mc2_hset_set_sideband", "mc2_hset_set_row", "mc2_hset_assign_rows", "mc2_hset_reverse_complement", "mc2_model_create", "mc2_model_free", "mc2_model_desc_from_file",
+    "mc2_score_pairs", "mc2_get_close", "mc2_get_close_as", "mc2_filter", "mc2_filter_as", "mc2_merge", "mc2_all_pairs", "mc2_identity_pairs", "mc2_identity_pairs_both_strands", "mc2_debug_tile_reductions", "mc2_debug_last_sweep", "mc2_distance", "mc2_mean_closest", "mc2_closest",
     "mc2_update_centers", "mc2_merge_centers",
     "mc2_bench_score_pairs", "mc2_bench_count_kmers", "mc2_bench_issue_rate", "mc2_encode_dna", "mc2_encode_dna_batch",
 ]
@@ -103,6 +103,8 @@ def lib():
         L.mc2_identity_pairs.argtypes = [C.c_void_p, C.c_void_p, C.c_double, C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p,
                                          C.c_uint64, C.c_uint64, C.c_int32, C.c_double, C.c_uint64, C.c_void_p, C.c_void_p,
                                          C.c_void_p, C.c_void_p, C.c_void_p]
+        L.mc2_identity_pairs_both_strands.argtypes = (L.mc2_identity_pairs.argtypes[:15] + [C.c_void_p]
+                                                      + L.mc2_identity_pairs.argtypes[15:])
         _lib = L
     return _lib
 
@@ -395,6 +397,29 @@ class Context:
         got = min(n_out.value, max_out)
         return dict(q=oq[:got], d=od[:got], identity=oid[:got], n_out=n_out.value, n_scored=n_scored.value)
 
+    def identity_pairs_both_strands(self, model, set_q, set_d, min_identity, cutoff, q_range=None, d_range=None,
+                                    upper_only=False, max_out=1 << 20, out=None):
+        """identity_pairs on both strands of each query: a pair survives when the larger of its forward identity and its
+        identity against the query's reverse complement is >= min_identity.  Returns identity_pairs' dict plus `strand`
+        (int8: 0 forward, 1 reverse; ties go to forward).  out: optional (q, d, identity, strand) buffers."""
+        q0, q1 = q_range if q_range else (0, len(set_q))
+        d0, d1 = d_range if d_range else (0, len(set_d))
+        if out is not None:
+            oq, od, oid, ostr = out
+            assert min(len(oq), len(od), len(oid), len(ostr)) >= max_out
+        else:
+            oq = np.empty(max_out, dtype=np.uint64)
+            od = np.empty(max_out, dtype=np.uint64)
+            oid = np.empty(max_out)
+            ostr = np.empty(max_out, dtype=np.int8)
+        n_out, n_scored = C.c_uint64(), C.c_uint64()
+        _check(lib().mc2_identity_pairs_both_strands(self.h, model.h, min_identity, set_q.h, q0, q1, set_d.h, d0, d1,
+                                                     int(upper_only), cutoff, max_out, _p(oq), _p(od), _p(oid), _p(ostr),
+                                                     C.byref(n_out), C.byref(n_scored)))
+        got = min(n_out.value, max_out)
+        return dict(q=oq[:got], d=od[:got], identity=oid[:got], strand=ostr[:got], n_out=n_out.value,
+                    n_scored=n_scored.value)
+
     def issue_rate(self, iters=100000):
         """measured warp-instructions / s of the VIMNMX.U16x2 + IDP.2A pair (roofline denominator of the tile sweep)"""
         out = C.c_double()
@@ -591,6 +616,12 @@ class HistSet:
         dst_rows, src_rows = _u64(dst_rows), _u64(src_rows)
         _check(lib().mc2_hset_assign_rows(self.ctx.h, self.h, C.c_uint64(len(dst_rows)), _p(dst_rows), src.h, _p(src_rows),
                                           _p(_u64(mag)), _p(_u64(length))))
+
+    def reverse_complement(self):
+        """a new set whose row i is the histogram of the other strand of the sequence row i counted"""
+        h = C.c_void_p()
+        _check(lib().mc2_hset_reverse_complement(self.ctx.h, self.h, C.byref(h)))
+        return HistSet(self.ctx, h)
 
     def free(self):
         if self.h:

@@ -75,7 +75,8 @@ static void release(Buf &b)
 	b.cap = 0;
 }
 
-enum { B_IA = 0, B_IB, B_SCORE, B_DIST, B_CLOSE, B_SKIP, B_CACHE, B_RAW, B_MISC, B_OUTQ, B_OUTD, B_OUTS, B_STAGE_CODES, B_STAGE_BOFF, B_ROWMAX, B_ROWMAX_H, B_SEGCOUNT, B_OVERRIDE, B_COUNT };
+enum { B_IA = 0, B_IB, B_SCORE, B_DIST, B_CLOSE, B_SKIP, B_CACHE, B_RAW, B_MISC, B_OUTQ, B_OUTD, B_OUTS, B_STAGE_CODES, B_STAGE_BOFF, B_ROWMAX, B_ROWMAX_H, B_SEGCOUNT, B_OVERRIDE,
+       B_STR_Q, B_STR_D, B_STR_S, B_STR_F, B_STR_OQ, B_STR_OD, B_STR_OS, B_STR_OSTR, B_STR_CNT, B_COUNT };
 
 struct ProfRec {
 	int kind;
@@ -519,6 +520,15 @@ static int alloc_hset(mc2_ctx *ctx, u64 n, int k, int eb, mc2_hset **out)
 #undef A
 	*out = h;
 	return MC2_OK;
+}
+
+// the derived reverse-complement set carries bins, magnitudes and lengths: every write to one of them drops it
+static void drop_rc(mc2_hset *h)
+{
+	if (h->rc) {
+		mc2_hset_free(h->rc);
+		h->rc = nullptr;
+	}
 }
 
 // max over rows of the bin sums and of the raw k-mer multiplicities: out[0], out[1] (zeroed by the caller)
@@ -1147,6 +1157,7 @@ int mc2_count_kmers_into_rows(mc2_ctx *ctx, const mc2_seqs *seqs, mc2_hset *dst,
 	dst->lane_off_valid = 0;
 	dst->cum16_valid = 0;
 	dst->counted = 0;
+	drop_rc(dst);
 	if (seqs->n == 0) {
 		return MC2_OK;
 	}
@@ -1177,6 +1188,7 @@ int mc2_hset_refresh(mc2_ctx *ctx, mc2_hset *h, int32_t set_mag)
 	h->lane_off_valid = 0;
 	h->cum16_valid = 0;
 	h->counted = 0;
+	drop_rc(h);
 	if (h->n == 0) {
 		return MC2_OK;
 	}
@@ -1241,6 +1253,7 @@ int mc2_count_kmers_into(mc2_ctx *ctx, const mc2_seqs *seqs, mc2_hset *dst)
 	MC2_CUDA(cudaSetDevice(ctx->device));
 	dst->lane_off_valid = 0;
 	dst->cum16_valid = 0;
+	drop_rc(dst);
 	int rc = count_into(ctx, seqs, dst->k, dst->eb, 1, dst);
 	if (rc == MC2_OK) rc = refresh_max_sum(ctx, dst);
 	dst->counted = rc == MC2_OK;
@@ -1354,6 +1367,7 @@ int mc2_hset_update_from_device(mc2_ctx *ctx, mc2_hset *h, const void *d_bins, c
 	h->lane_off_valid = 0;
 	h->cum16_valid = 0;
 	h->counted = 0;
+	drop_rc(h);
 	MC2_CUDA(cudaMemcpyAsync(h->bins, d_bins, n * h->N * (u64)h->eb, cudaMemcpyDeviceToDevice, ctx->stream));
 	MC2_CUDA(cudaMemcpyAsync(h->len, d_len, n * 8, cudaMemcpyDeviceToDevice, ctx->stream));
 	if (d_mag) MC2_CUDA(cudaMemcpyAsync(h->mag, d_mag, n * 8, cudaMemcpyDeviceToDevice, ctx->stream));
@@ -1395,6 +1409,7 @@ void mc2_hset_free(mc2_hset *h)
 	cudaFree(h->cum16s);
 	cudaFree(h->plane8);
 	cudaFree(h->cumsum);
+	mc2_hset_free(h->rc);
 	delete h;
 }
 
@@ -1460,6 +1475,7 @@ int mc2_hset_set_sideband(mc2_ctx *ctx, mc2_hset *h, uint64_t count, const uint6
 			  const uint64_t *len)
 {
 	MC2_REQUIRE(ctx && h && (count == 0 || rows), "mc2_hset_set_sideband: NULL argument");
+	drop_rc(h);
 	for (u64 i = 0; i < count; i++) {
 		MC2_REQUIRE(rows[i] < h->n, "mc2_hset_set_sideband: row out of range");
 		if (mag) MC2_CUDA(cudaMemcpyAsync(h->mag + rows[i], mag + i, 8, cudaMemcpyHostToDevice, ctx->stream));
@@ -1477,6 +1493,7 @@ int mc2_hset_set_row(mc2_ctx *ctx, mc2_hset *dst, uint64_t dst_row, const mc2_hs
 	dst->lane_off_valid = 0;
 	dst->cum16_valid = 0;
 	dst->counted = 0;
+	drop_rc(dst);
 	cudaStream_t st = ctx->stream;
 	const u64 rb = dst->N * (u64)dst->eb;
 	// DivergencePoint::set (src/clutil/DivergencePoint.cpp:182-190): points + length (+header/id), NOT mag
@@ -1506,6 +1523,7 @@ int mc2_hset_assign_rows(mc2_ctx *ctx, mc2_hset *dst, uint64_t n, const uint64_t
 	dst->lane_off_valid = keep_loff ? 1 : 0;
 	dst->cum16_valid = 0;
 	dst->counted = 0;
+	drop_rc(dst);
 	const int parts = 2 + (mag ? 1 : 0) + (len ? 1 : 0);
 	std::vector<u64> idx((size_t)parts * n);
 	for (u64 i = 0; i < n; i++) {
@@ -2139,6 +2157,48 @@ int mc2_merge(mc2_ctx *ctx, const mc2_model *model, const mc2_hset *centers, con
 	return MC2_OK;
 }
 
+// the model of an identity search for min_identity: clamp(sum, 0, 1) >= t <=> sum >= t for 0 < t <= 1 (and t > 1 keeps
+// nothing, which the same threshold also rejects): the screen's threshold on the sum is t itself.  t <= 0 keeps every
+// in-window pair: nothing to screen.
+static DevModel identity_model(const mc2_model *model, double min_identity)
+{
+	DevModel dm = model->dm;
+	if (min_identity > 0) {
+		dm.scr_thr = screen_threshold(min_identity);
+	} else {
+		dm.scr_ok = 0;
+	}
+	return dm;
+}
+
+// One launch of the all-pairs sweep into device buffers of capacity max_out (arguments checked by the caller): *total = all
+// survivors (may exceed max_out), the sweep's diagnostics in last_exact / last_coarse.  The device error word is fetched
+// into ctx->h_err, not checked.
+static int run_sweep(mc2_ctx *ctx, const DevModel &dm, int identity, double min_identity, const mc2_hset *set_q, u64 q_begin,
+		     u64 q_end, const mc2_hset *set_d, u64 d_begin, u64 d_end, int32_t upper_only, double cutoff, u64 max_out,
+		     u64 *d_out_q, u64 *d_out_d, double *d_out_score, u64 *total, uint64_t *n_scored)
+{
+	CtxExtra *x = extra(ctx);
+	int rc = ensure(x->d[B_MISC], 64, false);
+	if (rc) return rc;
+	u64 *d_counters = (u64 *)x->d[B_MISC].p;
+	MC2_CUDA(cudaMemsetAsync(d_counters, 0, 64, ctx->stream));
+	rc = reset_err(ctx);
+	if (rc == MC2_OK)
+		rc = launch_all_pairs(ctx, dm, set_q, q_begin, q_end, set_d, d_begin, d_end, upper_only, cutoff, max_out, d_out_q, d_out_d,
+				      d_out_score, d_counters, identity, min_identity);
+	if (rc == MC2_OK) rc = fetch_err(ctx);
+	if (rc != MC2_OK) return rc;
+	cudaStream_t st = ctx->stream;
+	MC2_CUDA(cudaMemcpyAsync(ctx->h_slot, d_counters, 32, cudaMemcpyDeviceToHost, st));
+	MC2_CUDA(cudaStreamSynchronize(st));
+	*total = ((u64 *)ctx->h_slot)[0];
+	if (n_scored) *n_scored = ((u64 *)ctx->h_slot)[1];
+	x->last_exact = ((u64 *)ctx->h_slot)[2];
+	x->last_coarse = ((u64 *)ctx->h_slot)[3] != 0;
+	return MC2_OK;
+}
+
 // the sweep behind mc2_all_pairs and mc2_identity_pairs (`who` names the entry point in error messages); identity != 0:
 // survivors are the pairs whose regression score is >= min_identity, dm carries the screen threshold of that search
 static int sweep_pairs(const char *who, mc2_ctx *ctx, const DevModel &dm, int identity, double min_identity, const mc2_hset *set_q,
@@ -2165,22 +2225,11 @@ static int sweep_pairs(const char *who, mc2_ctx *ctx, const DevModel &dm, int id
 	rc = ensure(x->d[B_OUTQ], cap * 8, false); if (rc) return rc;
 	rc = ensure(x->d[B_OUTD], cap * 8, false); if (rc) return rc;
 	rc = ensure(x->d[B_OUTS], cap * 8, false); if (rc) return rc;
-	rc = ensure(x->d[B_MISC], 64, false); if (rc) return rc;
-	u64 *d_counters = (u64 *)x->d[B_MISC].p;
-	MC2_CUDA(cudaMemsetAsync(d_counters, 0, 64, ctx->stream));
-	rc = reset_err(ctx);
-	if (rc == MC2_OK)
-		rc = launch_all_pairs(ctx, dm, set_q, q_begin, q_end, set_d, d_begin, d_end, upper_only, cutoff, max_out,
-				      (u64 *)x->d[B_OUTQ].p, (u64 *)x->d[B_OUTD].p, (double *)x->d[B_OUTS].p, d_counters, identity, min_identity);
-	if (rc == MC2_OK) rc = fetch_err(ctx);
+	u64 total = 0;
+	rc = run_sweep(ctx, dm, identity, min_identity, set_q, q_begin, q_end, set_d, d_begin, d_end, upper_only, cutoff, max_out,
+		       (u64 *)x->d[B_OUTQ].p, (u64 *)x->d[B_OUTD].p, (double *)x->d[B_OUTS].p, &total, n_scored);
 	if (rc != MC2_OK) return rc;
 	cudaStream_t st = ctx->stream;
-	MC2_CUDA(cudaMemcpyAsync(ctx->h_slot, d_counters, 32, cudaMemcpyDeviceToHost, st));
-	MC2_CUDA(cudaStreamSynchronize(st));
-	u64 total = ((u64 *)ctx->h_slot)[0];
-	if (n_scored) *n_scored = ((u64 *)ctx->h_slot)[1];
-	x->last_exact = ((u64 *)ctx->h_slot)[2];
-	x->last_coarse = ((u64 *)ctx->h_slot)[3] != 0;
 	*n_out = total;
 	u64 got = total < max_out ? total : max_out;
 	if (got) {
@@ -2208,16 +2257,204 @@ int mc2_identity_pairs(mc2_ctx *ctx, const mc2_model *model, double min_identity
 {
 	MC2_REQUIRE(ctx && model && set_q && set_d && n_out, "mc2_identity_pairs: NULL argument");
 	MC2_REQUIRE(!std::isnan(min_identity), "mc2_identity_pairs: min_identity is NaN");
-	// clamp(sum, 0, 1) >= t <=> sum >= t for 0 < t <= 1 (and t > 1 keeps nothing, which the same threshold also rejects):
-	// the screen's threshold on the sum is t itself.  t <= 0 keeps every in-window pair: nothing to screen.
-	DevModel dm = model->dm;
-	if (min_identity > 0) {
-		dm.scr_thr = screen_threshold(min_identity);
-	} else {
-		dm.scr_ok = 0;
-	}
+	const DevModel dm = identity_model(model, min_identity);
 	return sweep_pairs("mc2_identity_pairs", ctx, dm, 1, min_identity, set_q, q_begin, q_end, set_d, d_begin, d_end, upper_only,
 			   cutoff, max_out, out_q, out_d, out_identity, n_out, n_scored);
+}
+
+/* ---- the other strand ------------------------------------------------------------------------- */
+static int reverse_complement_set(mc2_ctx *ctx, const mc2_hset *src, mc2_hset **out)
+{
+	mc2_hset *h = nullptr;
+	int rc = alloc_hset(ctx, src->n, src->k, src->eb, &h);
+	if (rc != MC2_OK) return rc;
+	const u64 n = src->n;
+	cudaStream_t st = ctx->stream;
+	cudaError_t e = cudaSuccess;
+	if (n) {
+		// everything but the bins and the k = 1 table depends on the multiset of counts only, which the permutation keeps
+		e = cudaMemcpyAsync(h->mag, src->mag, n * 8, cudaMemcpyDeviceToDevice, st);
+		if (e == cudaSuccess) e = cudaMemcpyAsync(h->len, src->len, n * 8, cudaMemcpyDeviceToDevice, st);
+		if (e == cudaSuccess) e = cudaMemcpyAsync(h->sum, src->sum, n * 8, cudaMemcpyDeviceToDevice, st);
+		if (e == cudaSuccess) e = cudaMemcpyAsync(h->sumsq, src->sumsq, n * 8, cudaMemcpyDeviceToDevice, st);
+		if (e == cudaSuccess) e = cudaMemcpyAsync(h->stddev, src->stddev, n * 8, cudaMemcpyDeviceToDevice, st);
+		if (e == cudaSuccess) e = cudaMemcpyAsync(h->maxc, src->maxc, n * 4, cudaMemcpyDeviceToDevice, st);
+		// the overflowing-segment count depends on the order of the segments: reported as for a set built from histograms
+		if (e == cudaSuccess) e = cudaMemsetAsync(h->novf, 0, n * 4, st);
+	}
+	if (e != cudaSuccess) {
+		mc2_hset_free(h);
+		return cuda_fail(e, "reverse complement side-band copies", __FILE__, __LINE__);
+	}
+	rc = launch_revcomp(ctx, src, h);
+	if (rc == MC2_OK) {
+		e = cudaStreamSynchronize(st);
+		if (e != cudaSuccess) rc = cuda_fail(e, "reverse complement", __FILE__, __LINE__);
+	}
+	if (rc != MC2_OK) {
+		mc2_hset_free(h);
+		return rc;
+	}
+	h->max_sum = src->max_sum;
+	h->max_count = src->max_count;
+	h->counted = src->counted;
+	*out = h;
+	return MC2_OK;
+}
+
+int mc2_hset_reverse_complement(mc2_ctx *ctx, const mc2_hset *src, mc2_hset **out)
+{
+	MC2_REQUIRE(ctx && src && out, "mc2_hset_reverse_complement: NULL argument");
+	*out = nullptr;
+	MC2_CUDA(cudaSetDevice(ctx->device));
+	return reverse_complement_set(ctx, src, out);
+}
+
+// pair-scoring launch over device-resident index lists (set_a row ia[j], set_b row ib[j]), scores into d_score: the launch and
+// arguments mc2_score_pairs uses for host lists, so the scores are the same bits
+static int score_device_lists(mc2_ctx *ctx, const DevModel &dm, const mc2_hset *A, const mc2_hset *B, const u64 *d_ia,
+			      const u64 *d_ib, u64 n, double *d_score)
+{
+	PairArgs a;
+	memset(&a, 0, sizeof a);
+	a.binsA = A->bins;
+	a.binsB = B->bins;
+	a.sbA = Sideband{A->mag, A->sum, A->sumsq, A->len};
+	a.sbB = Sideband{B->mag, B->sum, B->sumsq, B->len};
+	a.N = A->N;
+	a.eb = A->eb;
+	a.n_pairs = n;
+	a.ia = d_ia;
+	a.ib = d_ib;
+	a.err = ctx->d_err;
+	a.max_sum = A->max_sum > B->max_sum ? A->max_sum : B->max_sum;
+	if (ensure_lane_off(ctx, A) == MC2_OK && ensure_lane_off(ctx, B) == MC2_OK && A->lane_off_valid && B->lane_off_valid) {
+		a.loffA = A->lane_off;
+		a.loffB = B->lane_off;
+	}
+	a.score = d_score;
+	return launch_pair_score(ctx, dm, a);
+}
+
+// survivors of one reverse-strand block that the scratch holds; a query row has at most d_end - d_begin of them
+static const u64 kStrandScratch = 1ull << 20;
+
+int mc2_identity_pairs_both_strands(mc2_ctx *ctx, const mc2_model *model, double min_identity, const mc2_hset *set_q,
+				    uint64_t q_begin, uint64_t q_end, const mc2_hset *set_d, uint64_t d_begin, uint64_t d_end,
+				    int32_t upper_only, double cutoff, uint64_t max_out, uint64_t *out_q, uint64_t *out_d,
+				    double *out_identity, int8_t *out_strand, uint64_t *n_out, uint64_t *n_scored)
+{
+	const std::string w("mc2_identity_pairs_both_strands");
+	MC2_REQUIRE(ctx && model && set_q && set_d && n_out, w + ": NULL argument");
+	MC2_REQUIRE(!std::isnan(min_identity), w + ": min_identity is NaN");
+	MC2_REQUIRE(q_begin <= q_end && q_end <= set_q->n && d_begin <= d_end && d_end <= set_d->n, w + ": row range out of bounds");
+	MC2_REQUIRE(set_q->k == set_d->k && set_q->eb == set_d->eb, w + ": the two sets differ in k or histogram width");
+	MC2_REQUIRE(cutoff > 0, w + ": cutoff must be > 0");
+	MC2_REQUIRE((q_end - q_begin) * ((d_end - d_begin + 31) / 32) < (1ULL << 32),
+		    w + ": more than 2^32 (query row, 32-column block) groups in one call; split the query range");
+	MC2_REQUIRE(model->dm.regression != 0, w + ": needs a regression model");
+	MC2_CUDA(cudaSetDevice(ctx->device));
+	*n_out = 0;
+	if (n_scored) *n_scored = 0;
+	CtxExtra *x = extra(ctx);
+	x->last_exact = 0;
+	x->last_coarse = 0;
+	if (q_begin == q_end || d_begin == d_end) return MC2_OK;
+	const double t = min_identity;
+	const DevModel dm = identity_model(model, t);
+	const u64 cap = max_out ? max_out : 1, scratch = std::max<u64>(d_end - d_begin, kStrandScratch);
+	int rc;
+	const int bufs[] = {B_STR_Q, B_STR_D, B_STR_S, B_STR_F, B_STR_OQ, B_STR_OD, B_STR_OS, B_STR_OSTR, B_STR_CNT};
+	const u64 sizes[] = {scratch * 8, scratch * 8, scratch * 8, scratch * 8, cap * 8, cap * 8, cap * 8, cap, 8};
+	for (int i = 0; i < 9; i++) {
+		if ((rc = ensure(x->d[bufs[i]], sizes[i], false)) != MC2_OK) return rc;
+	}
+	u64 *sq = (u64 *)x->d[B_STR_Q].p, *sd = (u64 *)x->d[B_STR_D].p, *oq = (u64 *)x->d[B_STR_OQ].p, *od = (u64 *)x->d[B_STR_OD].p;
+	double *ss = (double *)x->d[B_STR_S].p, *sf = (double *)x->d[B_STR_F].p, *os = (double *)x->d[B_STR_OS].p;
+	int8_t *ostr = (int8_t *)x->d[B_STR_OSTR].p;
+	u64 *cnt = (u64 *)x->d[B_STR_CNT].p;
+	cudaStream_t st = ctx->stream;
+
+	// forward strand: A = {id+ >= t}, the first max_out of them straight into the output
+	u64 n_fwd = 0;
+	rc = run_sweep(ctx, dm, 1, t, set_q, q_begin, q_end, set_d, d_begin, d_end, upper_only, cutoff, max_out, oq, od, os, &n_fwd, n_scored);
+	if (rc == MC2_OK) rc = check_err(ctx);
+	if (rc != MC2_OK) return rc;
+	u64 exact = x->last_exact;
+	int coarse = x->last_coarse;
+
+	// the reverse-complement rows keep the query indices, so upper_only and the length window mean the same on both strands
+	if (!set_q->rc) {
+		mc2_hset *r = nullptr;
+		if ((rc = reverse_complement_set(ctx, set_q, &r)) != MC2_OK) return rc;
+		const_cast<mc2_hset *>(set_q)->rc = r;
+	}
+	const mc2_hset *rcq = set_q->rc;
+
+	// id- of the returned forward survivors: the strand and identity they report
+	const u64 got_fwd = std::min<u64>(n_fwd, max_out);
+	for (u64 i = 0; i < got_fwd; i += scratch) {
+		const u64 m = std::min<u64>(scratch, got_fwd - i);
+		rc = score_device_lists(ctx, dm, set_d, rcq, od + i, oq + i, m, sf);
+		if (rc == MC2_OK) rc = launch_strand_pick(ctx, os + i, sf, ostr + i, m);
+		if (rc != MC2_OK) return rc;
+	}
+	MC2_CUDA(cudaMemcpyAsync(cnt, &n_fwd, 8, cudaMemcpyHostToDevice, st));
+	rc = fetch_err(ctx);
+	if (rc != MC2_OK) return rc;
+	MC2_CUDA(cudaStreamSynchronize(st));
+	if ((rc = check_err(ctx)) != MC2_OK) return rc;
+
+	// Reverse strand: B = {id- >= t}, query-row block by block into the scratch; B \ A = the pairs of B with id+ < t.  For
+	// t <= 0 every in-window pair is in A and B adds nothing.
+	if (t > 0) {
+		// first block: sized from the forward survivor count (the other strand of random reads has about as many), with
+		// half the scratch to spare for rows denser than average (the early rows of an upper triangle)
+		const u64 all_rows = q_end - q_begin;
+		u64 qb = q_begin;
+		u64 rows = std::max<u64>(1, std::min<u64>(all_rows, (u64)((double)all_rows * (double)(scratch / 2) / (double)std::max<u64>(n_fwd, 1))));
+		while (qb < q_end) {
+			const u64 qe = qb + std::min<u64>(rows, q_end - qb);
+			u64 nb = 0;
+			rc = run_sweep(ctx, dm, 1, t, rcq, qb, qe, set_d, d_begin, d_end, upper_only, cutoff, scratch, sq, sd, ss, &nb, nullptr);
+			if (rc == MC2_OK) rc = check_err(ctx);
+			if (rc != MC2_OK) return rc;
+			exact += x->last_exact;
+			coarse &= x->last_coarse;
+			if (nb > scratch) { // more than the scratch holds: sweep a smaller block again (one row always fits)
+				const u64 span = qe - qb;
+				rows = std::max<u64>(1, std::min<u64>(span / 2, (u64)((double)span * (double)(scratch / 2) / (double)nb)));
+				continue;
+			}
+			if (nb) {
+				rc = score_device_lists(ctx, dm, set_d, set_q, sd, sq, nb, sf);
+				if (rc == MC2_OK) rc = launch_strand_append(ctx, sq, sd, ss, sf, nb, t, cnt, max_out, oq, od, os, ostr);
+				if (rc == MC2_OK) rc = fetch_err(ctx);
+				if (rc != MC2_OK) return rc;
+				MC2_CUDA(cudaStreamSynchronize(st));
+				if ((rc = check_err(ctx)) != MC2_OK) return rc;
+			}
+			qb = qe;
+			if (nb < scratch / 4) {
+				rows = std::min<u64>(rows * 2, all_rows);
+			}
+		}
+	}
+	MC2_CUDA(cudaMemcpyAsync(ctx->h_slot, cnt, 8, cudaMemcpyDeviceToHost, st));
+	MC2_CUDA(cudaStreamSynchronize(st));
+	const u64 total = ((u64 *)ctx->h_slot)[0];
+	*n_out = total;
+	x->last_exact = exact;
+	x->last_coarse = coarse;
+	const u64 got = std::min<u64>(total, max_out);
+	if (got) {
+		if (out_q) MC2_CUDA(cudaMemcpyAsync(out_q, oq, got * 8, cudaMemcpyDeviceToHost, st));
+		if (out_d) MC2_CUDA(cudaMemcpyAsync(out_d, od, got * 8, cudaMemcpyDeviceToHost, st));
+		if (out_identity) MC2_CUDA(cudaMemcpyAsync(out_identity, os, got * 8, cudaMemcpyDeviceToHost, st));
+		if (out_strand) MC2_CUDA(cudaMemcpyAsync(out_strand, ostr, got, cudaMemcpyDeviceToHost, st));
+		MC2_CUDA(cudaStreamSynchronize(st));
+	}
+	return MC2_OK;
 }
 
 int mc2_debug_last_sweep(mc2_ctx *ctx, uint64_t *n_exact, int32_t *coarse)

@@ -232,6 +232,9 @@ struct mc2_hset {
 	unsigned char *plane8;
 	int cum16_valid;
 	int cum_base;
+	// the reverse-complement set (strand.cu) that mc2_identity_pairs_both_strands sweeps for the other strand of these rows;
+	// built lazily, freed whenever bins, magnitudes or lengths change.
+	mc2_hset *rc;
 };
 
 struct mc2_model {
@@ -302,6 +305,11 @@ int launch_mean_closest(mc2_ctx *ctx, const mc2_hset *h, const u64 *d_members, u
 			void *d_out, bool have_mean);
 int launch_update_batch(mc2_ctx *ctx, const mc2_hset *h, const u64 *d_member_off, const u64 *d_members, const uint8_t *d_close,
 			const uint8_t *d_skipped, u64 c_begin, u64 count, double *d_mean, long long *d_next, u64 *d_n_good);
+// strand.cu: dst (same shape as src) receives the reverse-complement bins and the swapped k = 1 table of every row
+int launch_revcomp(mc2_ctx *ctx, const mc2_hset *src, mc2_hset *dst);
+int launch_strand_pick(mc2_ctx *ctx, double *score, const double *rev, int8_t *strand, u64 n);
+int launch_strand_append(mc2_ctx *ctx, const u64 *bq, const u64 *bd, const double *bs, const double *fwd, u64 n, double t,
+			 u64 *counter, u64 max_out, u64 *oq, u64 *od, double *os, int8_t *ostr);
 int launch_merge_batch(mc2_ctx *ctx, const double *d_dist, const uint8_t *d_skipped, const uint8_t *d_close, const u64 *d_off,
 		       u64 n_centers, long long *d_out);
 

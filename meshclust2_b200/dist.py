@@ -74,7 +74,8 @@ def rect_row_blocks(n, world, rank):
 class Survivors:
     """This rank's survivor pairs of one step, block by block, WITHOUT copying them together: an engine may hand back views
     of its own (page-locked, per-block) buffers, valid until its next step.  tolist() / array() build the [m, 2] form;
-    scores() the pairs' scores in the same order, where the engine reported them."""
+    scores() the pairs' scores in the same order, where the engine reported them; strands() the strand of each pair's
+    identity (0 forward, 1 reverse) after a both-strand identity search."""
 
     def __init__(self):
         self.parts = []
@@ -98,6 +99,11 @@ class Survivors:
         if not self.parts:
             return np.zeros(0)
         return np.concatenate([p[2] for p in self.parts])
+
+    def strands(self):
+        if not self.parts:
+            return np.zeros(0, dtype=np.int8)
+        return np.concatenate([p[3] for p in self.parts])
 
     def tolist(self):
         return self.array().tolist()
@@ -145,14 +151,18 @@ def all_pairs_step(engine, comm, torch, n_total, cutoff, upper_only=True, blocks
     """One pass of the hot path over a batch: local K1 -> all-gather -> row-block K2 sweep.
 
     identity: None sweeps with the engine's classifier; (regression model, min_identity) makes it an identity search
-    (survivors = pairs whose predicted identity is >= min_identity, Survivors.scores() = those identities).
+    (survivors = pairs whose predicted identity is >= min_identity, Survivors.scores() = those identities);
+    (regression model, min_identity, True) searches both strands of each query (identity = the better strand's,
+    Survivors.strands() = which strand).  Each rank reverse-complements the gathered set itself: no extra collective, and no
+    floating-point value is reduced across ranks.
 
     engine.count()                  K1 over this rank's shard
     engine.export_local()           -> (bins [per, N] tensor, length [per] int64 tensor, mag [per] int64 tensor) padded
     engine.install_full(bins, length, mag, n_total)   make the gathered set the sweep's database
     engine.use_local_as_full()      single rank: the counted shard is the database (no copy, no collective)
-    engine.sweep(q0, q1, upper_only, cutoff, max_out[, identity=(model, min_identity)])
-                                    -> (n_survivors, n_scored, survivors: array [m,2], (q[m], d[m]) or (q[m], d[m], score[m]))
+    engine.sweep(q0, q1, upper_only, cutoff, max_out[, identity=(model, min_identity[, both_strands])])
+                                    -> (n_survivors, n_scored, survivors: array [m,2], (q[m], d[m]), (q[m], d[m], score[m])
+                                        or, both strands, (q[m], d[m], identity[m], strand[m]))
     Returns dict(n_scored, n_close, survivors (this rank's), blocks)."""
     if comm.world > 1 and hasattr(engine, "count_and_gather_in_place"):
         # the product engine: K1 writes this rank's rows straight into the full set, the all-gathers run in place on it
@@ -483,7 +493,8 @@ class GpuEngine:
         return self.ctx.merge_centers(self.model, sc, len(rows), delta, cutoff)
 
     def sweep(self, q0, q1, upper_only, cutoff, max_out, identity=None):
-        """identity: None = the engine's classifier (all_pairs), else (regression model, min_identity) (identity_pairs)"""
+        """identity: None = the engine's classifier (all_pairs), else (regression model, min_identity) (identity_pairs) or
+        (regression model, min_identity, both_strands) (identity_pairs_both_strands when both_strands is true)"""
         # survivor buffers: one page-locked triple per block of a step, allocated once and reused by every step (fresh
         # pageable arrays cost page faults + a staged copy per call; a shared triple would force a host copy per block)
         slots = getattr(self, "_surv_slots", None)
@@ -507,8 +518,18 @@ class GpuEngine:
                     pass
             slots[slot] = bufs + (pinned,)
         nd = min(len(self.full), getattr(self, "n_total", None) or len(self.full))   # rows past n_total are shard padding
+        if identity is not None and len(identity) > 2 and identity[2]:
+            model, t = identity[:2]
+            strand = getattr(self, "_strand_slots", {})
+            self._strand_slots = strand
+            if slot not in strand or len(strand[slot]) < max_out:
+                strand[slot] = np.zeros(max_out, dtype=np.int8)
+            r = self.ctx.identity_pairs_both_strands(model, self.full, self.full, t, cutoff, q_range=(q0, q1), d_range=(0, nd),
+                                                     upper_only=upper_only, max_out=max_out,
+                                                     out=slots[slot][:3] + (strand[slot],))
+            return r["n_out"], r["n_scored"], (r["q"], r["d"], r["identity"], r["strand"])
         if identity is not None:
-            model, t = identity
+            model, t = identity[:2]
             r = self.ctx.identity_pairs(model, self.full, self.full, t, cutoff, q_range=(q0, q1), d_range=(0, nd),
                                         upper_only=upper_only, max_out=max_out, out=slots[slot][:3])
             return r["n_out"], r["n_scored"], (r["q"], r["d"], r["identity"])
