@@ -391,6 +391,34 @@ int mc2_identity_pairs_both_strands(mc2_ctx *ctx, const mc2_model *model, double
 				    int32_t upper_only, double cutoff, uint64_t max_out, uint64_t *out_q, uint64_t *out_d,
 				    double *out_identity, int8_t *out_strand, uint64_t *n_out, uint64_t *n_scored);
 
+/* Top-K identity search: for each query row r in [q_begin, q_end), its k_best best database hits.
+ * Hits: exactly the pairs (r, c) that mc2_identity_pairs keeps for the same arguments (same length window, upper_only rule
+ * c > r, feature order compute(database c, query r), same decision on the same bits).  exclude_self != 0 also drops c == r
+ * (an all-vs-all neighbour table without the self hit); it needs set_q == set_d.
+ * Order: identity descending, then database row ascending; the comparison is numeric (-0.0 equals +0.0).  Row r - q_begin of
+ * the output holds the first min(k_best, hits) entries of that order: out_d and out_identity are (q_end - q_begin) x k_best,
+ * row-major; out_identity[i] is the same bits as the score mc2_score_pairs gives the pair (set_a = set_d row out_d[i],
+ * set_b = set_q row r); unused slots hold d = UINT64_MAX and identity -1.0.  out_count[r - q_begin] = the filled slots,
+ * out_n_hits[r - q_begin] (may be NULL) = the query's total hit count, which may exceed k_best.  The order is total, so the
+ * result does not depend on survivor order, block sizes or how the query rows are split over calls or GPUs.
+ * *n_scored (may be NULL) equals mc2_identity_pairs'.  min_identity <= 0: every in-window pair is a hit; min_identity > 1:
+ * no query has one; empty ranges give zero counts.
+ * MC2_ERR_ARG: a classifier model, a NaN min_identity, k_best == 0 or > 1024, a (q_end - q_begin) x k_best table whose
+ * size in bytes overflows, a database range of 2^32 rows or more, exclude_self with two different sets, and every argument
+ * check of mc2_identity_pairs.  MC2_ERR_FEATURE as mc2_identity_pairs returns it.
+ * How: the unchanged identity sweep runs over blocks of query rows into a fixed scratch of max(d_end - d_begin, 2^22)
+ * pairs, starting with the whole range; a block whose survivors overflow it is swept again in smaller blocks, and blocks
+ * grow again while survivors stay sparse.  Each block's survivors are bucketed by query on the device and each bucket is
+ * reduced to its top k_best there (topk.cu), straight into the output table; one copy to the host at the end.  Extra device
+ * memory is the output table plus the fixed scratch: it does not grow with the number of hits.
+ * mc2_debug_last_sweep afterwards: n_exact summed over every block sweep run, coarse = 1 iff every one took the coarse form.
+ * Known limit: one strand only.  A both-strand ranking needs each pair's max over its two strands before it can be ranked,
+ * which this composition of one-strand sweeps does not compute. */
+int mc2_identity_topk(mc2_ctx *ctx, const mc2_model *model, double min_identity, uint32_t k_best, const mc2_hset *set_q,
+		      uint64_t q_begin, uint64_t q_end, const mc2_hset *set_d, uint64_t d_begin, uint64_t d_end, int32_t upper_only,
+		      int32_t exclude_self, double cutoff, uint64_t *out_d, double *out_identity, uint32_t *out_count,
+		      uint64_t *out_n_hits, uint64_t *n_scored);
+
 /* Measured issue rate (warp-instructions per second, whole GPU) of the tile sweep's inner instruction pair -- VIMNMX.U16x2 on
  * the ALU pipe feeding IDP.2A on the FMA pipe, register operands only, 32 resident warps per SM: the denominator of
  * bench.py's roofline for the CUDA-core EMD term (SURVEY.md section 8d: "achieved ... vs a measured ALU peak"). */

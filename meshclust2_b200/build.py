@@ -10,7 +10,8 @@ import sys
 from concurrent.futures import ThreadPoolExecutor
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-NAMES = ("mc2_api.cu", "kmer_count.cu", "pair_score.cu", "tile_sweep.cu", "mean_shift.cu", "text_ingest.cu", "strand.cu", "host_encode.cpp")
+NAMES = ("mc2_api.cu", "kmer_count.cu", "pair_score.cu", "tile_sweep.cu", "mean_shift.cu", "text_ingest.cu", "strand.cu", "topk.cu",
+         "host_encode.cpp")
 SRC = [os.path.join(HERE, "csrc", f) for f in NAMES]
 HDR = [os.path.join(HERE, "csrc", "mc2_internal.cuh"), os.path.join(HERE, "csrc", "pair_eval.cuh"),
        os.path.join(HERE, "..", "include", "meshclust2_b200.h")]

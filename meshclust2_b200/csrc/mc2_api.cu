@@ -76,7 +76,9 @@ static void release(Buf &b)
 }
 
 enum { B_IA = 0, B_IB, B_SCORE, B_DIST, B_CLOSE, B_SKIP, B_CACHE, B_RAW, B_MISC, B_OUTQ, B_OUTD, B_OUTS, B_STAGE_CODES, B_STAGE_BOFF, B_ROWMAX, B_ROWMAX_H, B_SEGCOUNT, B_OVERRIDE,
-       B_STR_Q, B_STR_D, B_STR_S, B_STR_F, B_STR_OQ, B_STR_OD, B_STR_OS, B_STR_OSTR, B_STR_CNT, B_COUNT };
+       B_STR_Q, B_STR_D, B_STR_S, B_STR_F, B_STR_OQ, B_STR_OD, B_STR_OS, B_STR_OSTR, B_STR_CNT,
+       B_TOPK_Q, B_TOPK_D, B_TOPK_S, B_TOPK_BID, B_TOPK_BD, B_TOPK_CNT, B_TOPK_OFF, B_TOPK_OD, B_TOPK_OID, B_TOPK_OCNT, B_TOPK_OHITS,
+       B_COUNT };
 
 struct ProfRec {
 	int kind;
@@ -2336,6 +2338,47 @@ static int score_device_lists(mc2_ctx *ctx, const DevModel &dm, const mc2_hset *
 	return launch_pair_score(ctx, dm, a);
 }
 
+// Sweeps query rows [q_begin, q_end) block by block into a scratch of `scratch` pairs (sq, sd, ss), starting with blocks of
+// `rows` rows.  A block whose survivors overflow the scratch is swept again in smaller blocks (one row always fits: scratch
+// >= d_end - d_begin); blocks double while their survivors fill less than a quarter of it.  on_block(qb, qe, nb) runs, in
+// row order, for each block [qb, qe) whose nb survivors all sit in the scratch: every row lies in exactly one such block.
+// *exact and *coarse gather the diagnostics of every sweep run (sum, and); *n_scored (may be NULL) sums the in-window pairs
+// of the blocks handed to on_block.
+extern "C++" { // a template: C++ linkage inside this file's extern "C" region
+template <typename F>
+static int sweep_row_blocks(mc2_ctx *ctx, const DevModel &dm, double t, const mc2_hset *set_q, u64 q_begin, u64 q_end,
+			    const mc2_hset *set_d, u64 d_begin, u64 d_end, int32_t upper_only, double cutoff, u64 scratch, u64 rows,
+			    u64 *sq, u64 *sd, double *ss, u64 *exact, int *coarse, uint64_t *n_scored, F &&on_block)
+{
+	CtxExtra *x = extra(ctx);
+	const u64 all_rows = q_end - q_begin;
+	u64 qb = q_begin;
+	while (qb < q_end) {
+		const u64 qe = qb + std::min<u64>(rows, q_end - qb);
+		u64 nb = 0;
+		uint64_t ns = 0;
+		int rc = run_sweep(ctx, dm, 1, t, set_q, qb, qe, set_d, d_begin, d_end, upper_only, cutoff, scratch, sq, sd, ss, &nb,
+				   n_scored ? &ns : nullptr);
+		if (rc == MC2_OK) rc = check_err(ctx);
+		if (rc != MC2_OK) return rc;
+		*exact += x->last_exact;
+		*coarse &= x->last_coarse;
+		if (nb > scratch) { // more than the scratch holds: sweep a smaller block again
+			const u64 span = qe - qb;
+			rows = std::max<u64>(1, std::min<u64>(span / 2, (u64)((double)span * (double)(scratch / 2) / (double)nb)));
+			continue;
+		}
+		if (n_scored) *n_scored += ns;
+		if ((rc = on_block(qb, qe, nb)) != MC2_OK) return rc;
+		qb = qe;
+		if (nb < scratch / 4) {
+			rows = std::min<u64>(rows * 2, all_rows);
+		}
+	}
+	return MC2_OK;
+}
+}
+
 // survivors of one reverse-strand block that the scratch holds; a query row has at most d_end - d_begin of them
 static const u64 kStrandScratch = 1ull << 20;
 
@@ -2411,34 +2454,18 @@ int mc2_identity_pairs_both_strands(mc2_ctx *ctx, const mc2_model *model, double
 		// first block: sized from the forward survivor count (the other strand of random reads has about as many), with
 		// half the scratch to spare for rows denser than average (the early rows of an upper triangle)
 		const u64 all_rows = q_end - q_begin;
-		u64 qb = q_begin;
-		u64 rows = std::max<u64>(1, std::min<u64>(all_rows, (u64)((double)all_rows * (double)(scratch / 2) / (double)std::max<u64>(n_fwd, 1))));
-		while (qb < q_end) {
-			const u64 qe = qb + std::min<u64>(rows, q_end - qb);
-			u64 nb = 0;
-			rc = run_sweep(ctx, dm, 1, t, rcq, qb, qe, set_d, d_begin, d_end, upper_only, cutoff, scratch, sq, sd, ss, &nb, nullptr);
-			if (rc == MC2_OK) rc = check_err(ctx);
-			if (rc != MC2_OK) return rc;
-			exact += x->last_exact;
-			coarse &= x->last_coarse;
-			if (nb > scratch) { // more than the scratch holds: sweep a smaller block again (one row always fits)
-				const u64 span = qe - qb;
-				rows = std::max<u64>(1, std::min<u64>(span / 2, (u64)((double)span * (double)(scratch / 2) / (double)nb)));
-				continue;
-			}
-			if (nb) {
-				rc = score_device_lists(ctx, dm, set_d, set_q, sd, sq, nb, sf);
-				if (rc == MC2_OK) rc = launch_strand_append(ctx, sq, sd, ss, sf, nb, t, cnt, max_out, oq, od, os, ostr);
-				if (rc == MC2_OK) rc = fetch_err(ctx);
-				if (rc != MC2_OK) return rc;
-				MC2_CUDA(cudaStreamSynchronize(st));
-				if ((rc = check_err(ctx)) != MC2_OK) return rc;
-			}
-			qb = qe;
-			if (nb < scratch / 4) {
-				rows = std::min<u64>(rows * 2, all_rows);
-			}
-		}
+		const u64 rows = std::max<u64>(1, std::min<u64>(all_rows, (u64)((double)all_rows * (double)(scratch / 2) / (double)std::max<u64>(n_fwd, 1))));
+		rc = sweep_row_blocks(ctx, dm, t, rcq, q_begin, q_end, set_d, d_begin, d_end, upper_only, cutoff, scratch, rows, sq, sd, ss,
+				      &exact, &coarse, nullptr, [&](u64, u64, u64 nb) -> int {
+			if (nb == 0) return MC2_OK;
+			int r = score_device_lists(ctx, dm, set_d, set_q, sd, sq, nb, sf);
+			if (r == MC2_OK) r = launch_strand_append(ctx, sq, sd, ss, sf, nb, t, cnt, max_out, oq, od, os, ostr);
+			if (r == MC2_OK) r = fetch_err(ctx);
+			if (r != MC2_OK) return r;
+			MC2_CUDA(cudaStreamSynchronize(st));
+			return check_err(ctx);
+		});
+		if (rc != MC2_OK) return rc;
 	}
 	MC2_CUDA(cudaMemcpyAsync(ctx->h_slot, cnt, 8, cudaMemcpyDeviceToHost, st));
 	MC2_CUDA(cudaStreamSynchronize(st));
@@ -2454,6 +2481,88 @@ int mc2_identity_pairs_both_strands(mc2_ctx *ctx, const mc2_model *model, double
 		if (out_strand) MC2_CUDA(cudaMemcpyAsync(out_strand, ostr, got, cudaMemcpyDeviceToHost, st));
 		MC2_CUDA(cudaStreamSynchronize(st));
 	}
+	return MC2_OK;
+}
+
+/* ---- top-K identity search ---------------------------------------------------------------------- */
+// survivors of one block of query rows that the scratch holds; a query row has at most d_end - d_begin of them
+static const u64 kTopkScratch = 1ull << 22;
+static const uint32_t kTopkMaxK = 1024;
+
+int mc2_identity_topk(mc2_ctx *ctx, const mc2_model *model, double min_identity, uint32_t k_best, const mc2_hset *set_q,
+		      uint64_t q_begin, uint64_t q_end, const mc2_hset *set_d, uint64_t d_begin, uint64_t d_end, int32_t upper_only,
+		      int32_t exclude_self, double cutoff, uint64_t *out_d, double *out_identity, uint32_t *out_count,
+		      uint64_t *out_n_hits, uint64_t *n_scored)
+{
+	const std::string w("mc2_identity_topk");
+	MC2_REQUIRE(ctx && model && set_q && set_d && out_d && out_identity && out_count, w + ": NULL argument");
+	MC2_REQUIRE(!std::isnan(min_identity), w + ": min_identity is NaN");
+	MC2_REQUIRE(k_best >= 1 && k_best <= kTopkMaxK, w + ": k_best must be in 1..1024");
+	MC2_REQUIRE(q_begin <= q_end && q_end <= set_q->n && d_begin <= d_end && d_end <= set_d->n, w + ": row range out of bounds");
+	MC2_REQUIRE(set_q->k == set_d->k && set_q->eb == set_d->eb, w + ": the two sets differ in k or histogram width");
+	MC2_REQUIRE(cutoff > 0, w + ": cutoff must be > 0");
+	MC2_REQUIRE((q_end - q_begin) * ((d_end - d_begin + 31) / 32) < (1ULL << 32),
+		    w + ": more than 2^32 (query row, 32-column block) groups in one call; split the query range");
+	MC2_REQUIRE(model->dm.regression != 0, w + ": needs a regression model");
+	MC2_REQUIRE(!exclude_self || set_q == set_d, w + ": exclude_self needs set_q == set_d");
+	const u64 nq = q_end - q_begin, K = k_best;
+	MC2_REQUIRE(nq <= UINT64_MAX / 16 / K, w + ": (q_end - q_begin) x k_best overflows");
+	MC2_REQUIRE(d_end - d_begin < (1ULL << 32), w + ": the database range must hold fewer than 2^32 rows");
+	MC2_CUDA(cudaSetDevice(ctx->device));
+	if (n_scored) *n_scored = 0;
+	CtxExtra *x = extra(ctx);
+	x->last_exact = 0;
+	x->last_coarse = 0;
+	if (nq == 0) return MC2_OK;
+	if (d_begin == d_end) {
+		std::fill(out_d, out_d + nq * K, UINT64_MAX);
+		std::fill(out_identity, out_identity + nq * K, -1.0);
+		std::fill(out_count, out_count + nq, 0u);
+		if (out_n_hits) std::fill(out_n_hits, out_n_hits + nq, (uint64_t)0);
+		return MC2_OK;
+	}
+	const DevModel dm = identity_model(model, min_identity);
+	const u64 scratch = std::max<u64>(d_end - d_begin, kTopkScratch);
+	int rc;
+	const int bufs[] = {B_TOPK_Q, B_TOPK_D, B_TOPK_S, B_TOPK_BID, B_TOPK_BD, B_TOPK_CNT, B_TOPK_OFF, B_TOPK_OD, B_TOPK_OID, B_TOPK_OCNT, B_TOPK_OHITS};
+	const u64 sizes[] = {scratch * 8, scratch * 8, scratch * 8, scratch * 8, scratch * 8, nq * 4, (nq + 1) * 8, nq * K * 8, nq * K * 8, nq * 4, nq * 8};
+	for (int i = 0; i < 11; i++) {
+		if ((rc = ensure(x->d[bufs[i]], sizes[i], false)) != MC2_OK) return rc;
+	}
+	u64 *sq = (u64 *)x->d[B_TOPK_Q].p, *sd = (u64 *)x->d[B_TOPK_D].p, *bd = (u64 *)x->d[B_TOPK_BD].p, *off = (u64 *)x->d[B_TOPK_OFF].p;
+	double *ss = (double *)x->d[B_TOPK_S].p, *bid = (double *)x->d[B_TOPK_BID].p;
+	u32 *cnt = (u32 *)x->d[B_TOPK_CNT].p;
+	u64 *od = (u64 *)x->d[B_TOPK_OD].p, *ohits = (u64 *)x->d[B_TOPK_OHITS].p;
+	double *oid = (double *)x->d[B_TOPK_OID].p;
+	u32 *ocnt = (u32 *)x->d[B_TOPK_OCNT].p;
+	cudaStream_t st = ctx->stream;
+
+	// Every query's hits land in exactly one block, so its top K is selected once from all of them.  The first block is the
+	// whole range: when the survivors fit, the call is one sweep.
+	u64 exact = 0;
+	uint64_t ns = 0;
+	int coarse = 1;
+	rc = sweep_row_blocks(ctx, dm, min_identity, set_q, q_begin, q_end, set_d, d_begin, d_end, upper_only, cutoff, scratch, nq,
+			      sq, sd, ss, &exact, &coarse, &ns, [&](u64 qb, u64 qe, u64 nb) -> int {
+		const u64 rows = qe - qb, r0 = qb - q_begin;
+		MC2_CUDA(cudaMemsetAsync(cnt, 0, rows * 4, st));
+		int r = launch_topk_count(ctx, sq, sd, nb, qb, exclude_self, cnt);
+		if (r == MC2_OK) r = launch_seg_scan(ctx, cnt, rows, off);
+		if (r != MC2_OK) return r;
+		MC2_CUDA(cudaMemsetAsync(cnt, 0, rows * 4, st)); // now the scatter's cursors
+		r = launch_topk_scatter(ctx, sq, sd, ss, nb, qb, exclude_self, off, cnt, bid, bd);
+		if (r == MC2_OK) r = launch_topk_select(ctx, off, bid, bd, rows, k_best, d_begin, od + r0 * K, oid + r0 * K, ocnt + r0, ohits + r0);
+		return r;
+	});
+	if (rc != MC2_OK) return rc;
+	x->last_exact = exact;
+	x->last_coarse = coarse;
+	if (n_scored) *n_scored = ns;
+	MC2_CUDA(cudaMemcpyAsync(out_d, od, nq * K * 8, cudaMemcpyDeviceToHost, st));
+	MC2_CUDA(cudaMemcpyAsync(out_identity, oid, nq * K * 8, cudaMemcpyDeviceToHost, st));
+	MC2_CUDA(cudaMemcpyAsync(out_count, ocnt, nq * 4, cudaMemcpyDeviceToHost, st));
+	if (out_n_hits) MC2_CUDA(cudaMemcpyAsync(out_n_hits, ohits, nq * 8, cudaMemcpyDeviceToHost, st));
+	MC2_CUDA(cudaStreamSynchronize(st));
 	return MC2_OK;
 }
 

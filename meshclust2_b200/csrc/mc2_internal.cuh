@@ -310,6 +310,13 @@ int launch_revcomp(mc2_ctx *ctx, const mc2_hset *src, mc2_hset *dst);
 int launch_strand_pick(mc2_ctx *ctx, double *score, const double *rev, int8_t *strand, u64 n);
 int launch_strand_append(mc2_ctx *ctx, const u64 *bq, const u64 *bd, const double *bs, const double *fwd, u64 n, double t,
 			 u64 *counter, u64 max_out, u64 *oq, u64 *od, double *os, int8_t *ostr);
+// topk.cu: survivors (sq, sd, ss)[0..n) of query rows [qb, ...) -> per-query counts, buckets at the counts' exclusive scan
+// off, and each query's first k_best (1..1024) entries by (identity desc, d asc) into its output row
+int launch_topk_count(mc2_ctx *ctx, const u64 *sq, const u64 *sd, u64 n, u64 qb, int exclude_self, u32 *cnt);
+int launch_topk_scatter(mc2_ctx *ctx, const u64 *sq, const u64 *sd, const double *ss, u64 n, u64 qb, int exclude_self,
+			const u64 *off, u32 *cur, double *bid, u64 *bd);
+int launch_topk_select(mc2_ctx *ctx, const u64 *off, const double *bid, const u64 *bd, u64 rows, u32 k_best, u64 d_begin,
+		       u64 *out_d, double *out_id, u32 *out_cnt, u64 *out_hits);
 int launch_merge_batch(mc2_ctx *ctx, const double *d_dist, const uint8_t *d_skipped, const uint8_t *d_close, const u64 *d_off,
 		       u64 n_centers, long long *d_out);
 

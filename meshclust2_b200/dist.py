@@ -147,7 +147,8 @@ class Comm:
         return float(t.item())
 
 
-def all_pairs_step(engine, comm, torch, n_total, cutoff, upper_only=True, blocks_per_rank=1, max_out=1 << 20, identity=None):
+def all_pairs_step(engine, comm, torch, n_total, cutoff, upper_only=True, blocks_per_rank=1, max_out=1 << 20, identity=None,
+                   top_k=None):
     """One pass of the hot path over a batch: local K1 -> all-gather -> row-block K2 sweep.
 
     identity: None sweeps with the engine's classifier; (regression model, min_identity) makes it an identity search
@@ -155,6 +156,10 @@ def all_pairs_step(engine, comm, torch, n_total, cutoff, upper_only=True, blocks
     (regression model, min_identity, True) searches both strands of each query (identity = the better strand's,
     Survivors.strands() = which strand).  Each rank reverse-complements the gathered set itself: no extra collective, and no
     floating-point value is reduced across ranks.
+    top_k: with a one-strand identity search, keep each query's top_k best hits instead of the survivor list: `topk` is
+    this rank's [(q0, q1, table)] with table = dict(d [q1-q0, top_k], identity [q1-q0, top_k], count, n_hits) as
+    engine.topk returns it.  A query lives in exactly one block of one rank, so the tables are complete per query and
+    nothing but the counters is reduced; n_close is the total hit count.
 
     engine.count()                  K1 over this rank's shard
     engine.export_local()           -> (bins [per, N] tensor, length [per] int64 tensor, mag [per] int64 tensor) padded
@@ -163,7 +168,10 @@ def all_pairs_step(engine, comm, torch, n_total, cutoff, upper_only=True, blocks
     engine.sweep(q0, q1, upper_only, cutoff, max_out[, identity=(model, min_identity[, both_strands])])
                                     -> (n_survivors, n_scored, survivors: array [m,2], (q[m], d[m]), (q[m], d[m], score[m])
                                         or, both strands, (q[m], d[m], identity[m], strand[m]))
-    Returns dict(n_scored, n_close, survivors (this rank's), blocks)."""
+    engine.topk(q0, q1, upper_only, cutoff, (model, min_identity), top_k) -> (n_hits, n_scored, table)
+    Returns dict(n_scored, n_close, survivors (this rank's), topk (this rank's, [] without top_k), blocks)."""
+    if top_k is not None and (identity is None or (len(identity) > 2 and identity[2])):
+        raise ValueError("top_k needs a one-strand identity search: identity=(regression model, min_identity)")
     if comm.world > 1 and hasattr(engine, "count_and_gather_in_place"):
         # the product engine: K1 writes this rank's rows straight into the full set, the all-gathers run in place on it
         engine.count_and_gather_in_place(comm, n_total)
@@ -188,7 +196,14 @@ def all_pairs_step(engine, comm, torch, n_total, cutoff, upper_only=True, blocks
               else rect_row_blocks(n_total, comm.world, comm.rank))
     n_scored = n_close = 0
     surv = Survivors()
+    tables = []
     for q0, q1 in blocks:
+        if top_k is not None:
+            ns, sc, table = engine.topk(q0, q1, upper_only, cutoff, identity, top_k)
+            tables.append((q0, q1, table))
+            n_close += ns
+            n_scored += sc
+            continue
         if identity is None:
             ns, sc, pairs = engine.sweep(q0, q1, upper_only, cutoff, max_out)
         else:
@@ -197,7 +212,8 @@ def all_pairs_step(engine, comm, torch, n_total, cutoff, upper_only=True, blocks
         n_scored += sc
         surv.add(pairs)
     tot_scored, tot_close = comm.all_reduce_sum([n_scored, n_close], torch, engine.device)
-    return dict(n_scored=tot_scored, n_close=tot_close, local_scored=n_scored, local_close=n_close, survivors=surv, blocks=blocks)
+    return dict(n_scored=tot_scored, n_close=tot_close, local_scored=n_scored, local_close=n_close, survivors=surv, topk=tables,
+                blocks=blocks)
 
 
 def candidate_scan(engine, comm, torch, q_global, n_total, cutoff):
@@ -491,6 +507,14 @@ class GpuEngine:
     def merge_centers(self, rows, mag, length, delta, cutoff):
         sc = self._stage_centers(rows, mag, length)
         return self.ctx.merge_centers(self.model, sc, len(rows), delta, cutoff)
+
+    def topk(self, q0, q1, upper_only, cutoff, identity, top_k):
+        """each query's top_k best identity hits (Context.identity_topk) -> (total hits, n_scored, table)"""
+        model, t = identity[:2]
+        nd = min(len(self.full), getattr(self, "n_total", None) or len(self.full))   # rows past n_total are shard padding
+        r = self.ctx.identity_topk(model, self.full, self.full, t, top_k, cutoff, q_range=(q0, q1), d_range=(0, nd),
+                                   upper_only=upper_only)
+        return int(r["n_hits"].sum()), r["n_scored"], r
 
     def sweep(self, q0, q1, upper_only, cutoff, max_out, identity=None):
         """identity: None = the engine's classifier (all_pairs), else (regression model, min_identity) (identity_pairs) or
