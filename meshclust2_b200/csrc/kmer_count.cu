@@ -468,9 +468,7 @@ __device__ __forceinline__ u32 shr64_lo(u32 hi, u32 lo, int r)
 	return (u32)((((u64)hi << 32) | lo) >> r);
 }
 
-#ifndef MC2_K1_MIN_CTAS
 #define MC2_K1_MIN_CTAS 4 // CTAs of 8 warps per SM the register budget must allow (4 -> 64 registers; 5 and 6 measured no faster)
-#endif
 template <typename T>
 __global__ void __launch_bounds__(256, MC2_K1_MIN_CTAS) count_warp_kernel(const __grid_constant__ CountArgs a)
 {
@@ -797,9 +795,7 @@ static int launch_count_t(mc2_ctx *ctx, const mc2_seqs *s, CountArgs &a)
 				MC2_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, count_warp_kernel<T>, warps * 32, smem));
 				per_sm = per_sm < 1 ? 1 : per_sm;
 				// one resident wave; every warp walks its sequences with the next one's loads in flight
-				const char *waves_env = getenv("MC2_K1_WAVES"); // tuning knob: CTAs launched per resident CTA
-				const int waves = waves_env ? (atoi(waves_env) > 0 ? atoi(waves_env) : 1) : 1;
-				const u64 want = (s->n + warps - 1) / warps, cap = (u64)ctx->sm_count * per_sm * waves;
+				const u64 want = (s->n + warps - 1) / warps, cap = (u64)ctx->sm_count * per_sm;
 				const int grid = (int)(want < cap ? want : cap);
 				prof_begin(ctx, 1);
 				count_warp_kernel<T><<<grid, warps * 32, smem, ctx->stream>>>(a);

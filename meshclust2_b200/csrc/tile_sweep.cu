@@ -124,9 +124,6 @@ struct Params {
 	u32 n_super;
 	u32 n_slabs;            // bins per row / 1024 (1 for k = 5, 64 for k = 8)
 	const u32 *sched;       // [n_super + 1] exclusive prefix of items per super-row (device)
-	int no_screen;          // experiments: skip the screen and the exact path (main-loop cost only)
-	int no_compute;         // experiments: the compute warps skip their arithmetic (epilogue cost only; results are wrong)
-	u32 sleep_ctrl, sleep_comp, sleep_epi; // experiments: back-off of the three roles' barrier waits (ns)
 	// raw mode (tests): dense (q1-q0) x (d1-d0) matrices of the reductions instead of scoring
 	u32 *raw_dot, *raw_emd, *raw_sad;
 };
@@ -152,16 +149,11 @@ __device__ __forceinline__ bool mbar_try(u32 bar, u32 parity)
 		     : "memory");
 	return ok != 0;
 }
-// bounded wait: a pipeline bug must end in an error, never in a hung GPU.  sleep_ns > 0: a warp that finds the barrier
-// not ready leaves the scheduler for that long instead of polling (its poll loop would take issue slots from the
-// compute warps of the same SM sub-partition)
-__device__ __forceinline__ void mbar_wait(u32 bar, u32 parity, int *err, u32 sleep_ns = 0)
+// bounded wait: a pipeline bug must end in an error, never in a hung GPU
+__device__ __forceinline__ void mbar_wait(u32 bar, u32 parity, int *err)
 {
 	u32 spins = 0;
 	while (!mbar_try(bar, parity)) {
-		if (sleep_ns) {
-			__nanosleep(sleep_ns);
-		}
 		if (++spins > (1u << 20)) {
 			atomicOr(err, 16);
 			__trap();
@@ -645,7 +637,7 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 				}
 				const int qrow = (int)(p.q0 + (u64)t.qt * TQ), drow = (int)(p.d0 + (u64)t.dt * TD);
 				for (int c = 0; c < N_U8 + N_CUM; c++) {
-					mbar_wait(bar_empty + s * 8, ph ^ 1, p.err, p.sleep_ctrl);
+					mbar_wait(bar_empty + s * 8, ph ^ 1, p.err);
 					const u32 st = sbase + s * STAGE_BYTES, fb = bar_full + s * 8;
 					mbar_expect_tx(fb, STAGE_BYTES);
 					if (stage_is_u8(c)) {
@@ -674,11 +666,11 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 				}
 				const u32 buf = it & 1;
 				if (DOT) {
-					mbar_wait(bar_tempty + buf * 8, ((it >> 1) & 1) ^ 1, p.err, p.sleep_ctrl);
+					mbar_wait(bar_tempty + buf * 8, ((it >> 1) & 1) ^ 1, p.err);
 					tc_fence_after();
 				}
 				for (int c = 0; c < N_U8 + N_CUM; c++) {
-					mbar_wait(bar_full + s * 8, ph, p.err, p.sleep_ctrl);
+					mbar_wait(bar_full + s * 8, ph, p.err);
 					if (DOT && stage_is_u8(c)) {
 						const int ku = stage_index(c);
 						tc_fence_after();
@@ -735,8 +727,8 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 				}
 #pragma unroll 1
 				for (int c = 0; c < N_U8 + N_CUM; c++) {
-					mbar_wait(bar_full + s * 8, ph, p.err, p.sleep_comp);
-					if (c % 3 != 2 && !p.no_compute) {
+					mbar_wait(bar_full + s * 8, ph, p.err);
+					if (c % 3 != 2) {
 						stage_compute<true>(smem + s * STAGE_BYTES, lane_row, qsel, acc);
 					}
 					__syncwarp();
@@ -748,7 +740,7 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 						ph ^= 1;
 					}
 				}
-				mbar_wait(bar_eempty + eb * 8, (eit & 1) ^ 1, p.err, p.sleep_comp); // the epilogue is done with this buffer's previous sums
+				mbar_wait(bar_eempty + eb * 8, (eit & 1) ^ 1, p.err); // the epilogue is done with this buffer's previous sums
 				tc_fence_after();
 				tc_st(tmem_base + tlane + TM_EMD + eb * 128 + qsel * QN, acc[0]);
 				tc_st(tmem_base + tlane + TM_EMD + eb * 128 + 64 + qsel * QN, acc[1]);
@@ -763,7 +755,7 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 				}
 #pragma unroll 1
 				for (int c = 0; c < N_U8; c++) {
-					mbar_wait(bar_full + s * 8, ph, p.err, p.sleep_comp);
+					mbar_wait(bar_full + s * 8, ph, p.err);
 					if (MIN) {
 						stage_compute<false>(smem + s * STAGE_BYTES, lane_row, qsel, acc);
 					}
@@ -777,7 +769,7 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 					}
 				}
 				if (MIN) {
-					mbar_wait(bar_eempty + eb * 8, (eit & 1) ^ 1, p.err, p.sleep_comp); // the epilogue is done with this buffer's previous sums
+					mbar_wait(bar_eempty + eb * 8, (eit & 1) ^ 1, p.err); // the epilogue is done with this buffer's previous sums
 					tc_fence_after();
 					tmem_free = true;
 					tc_st(tmem_base + tlane + TM_SAD + qsel * QN, acc[0]);
@@ -787,7 +779,7 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 			if (!INTERLEAVE && EMD && LY::QPASS > 1) {
 				// the one sample stage, the warpgroup's query rows in passes of QN: each pass goes to TMEM before the next
 				// one reuses the accumulators
-				mbar_wait(bar_full + s * 8, ph, p.err, p.sleep_comp);
+				mbar_wait(bar_full + s * 8, ph, p.err);
 #pragma unroll 1
 				for (int h = 0; h < LY::QPASS; h++) {
 					u32 acc[2][QN];
@@ -797,7 +789,7 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 					}
 					stage_compute<true>(smem + s * STAGE_BYTES, lane_row, qsel * LY::QPASS + h, acc);
 					if (h == 0) {
-						mbar_wait(bar_eempty + eb * 8, (eit & 1) ^ 1, p.err, p.sleep_comp);
+						mbar_wait(bar_eempty + eb * 8, (eit & 1) ^ 1, p.err);
 						tc_fence_after();
 					}
 					tc_st(tmem_base + tlane + TM_EMD + eb * 128 + (qsel * LY::QPASS + h) * QN, acc[0]);
@@ -820,7 +812,7 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 				}
 #pragma unroll 1
 				for (int c = 0; c < N_CUM; c++) {
-					mbar_wait(bar_full + s * 8, ph, p.err, p.sleep_comp);
+					mbar_wait(bar_full + s * 8, ph, p.err);
 					stage_compute<true>(smem + s * STAGE_BYTES, lane_row, qsel, acc);
 					__syncwarp();
 					if (lane == 0) {
@@ -832,7 +824,7 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 					}
 				}
 				if (!tmem_free) {
-					mbar_wait(bar_eempty + eb * 8, (eit & 1) ^ 1, p.err, p.sleep_comp);
+					mbar_wait(bar_eempty + eb * 8, (eit & 1) ^ 1, p.err);
 					tc_fence_after();
 				}
 				tc_st(tmem_base + tlane + TM_EMD + eb * 128 + qsel * QN, acc[0]);
@@ -909,10 +901,10 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 			const u32 buf = it & 1;
 			const u32 eb = EBUFS == 2 ? (it & 1) : 0, eit = EBUFS == 2 ? (it >> 1) : it;
 			if (CUDA_RED) {
-				mbar_wait(bar_efull + eb * 8, eit & 1, p.err, p.sleep_epi);
+				mbar_wait(bar_efull + eb * 8, eit & 1, p.err);
 			}
 			if (DOT) {
-				mbar_wait(bar_tfull + buf * 8, (it >> 1) & 1, p.err, p.sleep_epi);
+				mbar_wait(bar_tfull + buf * 8, (it >> 1) & 1, p.err);
 			}
 			tc_fence_after();
 			u32 n_list = 0, scored = 0;
@@ -962,7 +954,7 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 							}
 						}
 						scored += __popc(go);
-						u32 cand = p.no_screen ? 0u : go;
+						u32 cand = go;
 						const bool can_screen = dm.scr_ok != 0 && n_slabs == 1; // the screen's constants and bound are for 1024 bins
 						u32 anybig = PD[r].big;
 #pragma unroll
@@ -1488,11 +1480,6 @@ int launch_tile_sweep(mc2_ctx *ctx, const DevModel &dm, int need, const mc2_hset
 	p.n_super = (p.nqt + group - 1) / group;
 	p.n_slabs = (u32)(q->N / 1024);
 	p.sched = d_sched;
-	p.no_screen = getenv("MC2_TS_NOSCREEN") != nullptr;
-	p.no_compute = getenv("MC2_TS_NOCOMPUTE") != nullptr;
-	p.sleep_ctrl = getenv("MC2_TS_SLEEP_CTRL") ? (u32)atoi(getenv("MC2_TS_SLEEP_CTRL")) : 0;
-	p.sleep_comp = getenv("MC2_TS_SLEEP_COMP") ? (u32)atoi(getenv("MC2_TS_SLEEP_COMP")) : 0;
-	p.sleep_epi = getenv("MC2_TS_SLEEP_EPI") ? (u32)atoi(getenv("MC2_TS_SLEEP_EPI")) : 0;
 	p.raw_dot = raw_dot; p.raw_emd = raw_emd; p.raw_sad = raw_sad;
 	// the kernel reads the item count from the last prefix entry; it must fit 32 bits
 	if ((u64)p.n_super * group * p.ndt >= (1ull << 32)) {

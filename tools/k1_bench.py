@@ -14,7 +14,7 @@ def run(name, seqs, k, eb, iters=10):
     print("%-28s n=%d L=%.0f k=%d eb=%d: %.3f ms  %.3e hist/s  %.3e kmers/s  %.0f GB/s (%.1f%% of 6540)" % (
         name, len(seqs), L, k, eb, ms, len(seqs) / ms * 1e3, len(seqs) * L / ms * 1e3, byts / ms / 1e6, byts / ms / 1e6 / 65.4))
 seqs, _, k, eb = synth.make_config_range("cfg3", 0, int(os.environ.get("K1_N", 100000)))
-for legacy in ((False,) if os.environ.get("K1_NO_LEGACY") else (False, True)):
+for legacy in (False, True):
     if legacy:
         os.environ["MC2_K1_LEGACY"] = "1"   # count_kernel (the generic form) instead of count_warp_kernel
     else:
