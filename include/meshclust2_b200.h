@@ -412,12 +412,39 @@ int mc2_identity_pairs_both_strands(mc2_ctx *ctx, const mc2_model *model, double
  * reduced to its top k_best there (topk.cu), straight into the output table; one copy to the host at the end.  Extra device
  * memory is the output table plus the fixed scratch: it does not grow with the number of hits.
  * mc2_debug_last_sweep afterwards: n_exact summed over every block sweep run, coarse = 1 iff every one took the coarse form.
- * Known limit: one strand only.  A both-strand ranking needs each pair's max over its two strands before it can be ranked,
- * which this composition of one-strand sweeps does not compute. */
+ * One strand: mc2_identity_topk_both_strands ranks each pair's better strand. */
 int mc2_identity_topk(mc2_ctx *ctx, const mc2_model *model, double min_identity, uint32_t k_best, const mc2_hset *set_q,
 		      uint64_t q_begin, uint64_t q_end, const mc2_hset *set_d, uint64_t d_begin, uint64_t d_end, int32_t upper_only,
 		      int32_t exclude_self, double cutoff, uint64_t *out_d, double *out_identity, uint32_t *out_count,
 		      uint64_t *out_n_hits, uint64_t *n_scored);
+
+/* Both-strand top-K identity search: for each query row r in [q_begin, q_end), its k_best best database hits over both
+ * strands, with the strand of each.
+ * Hits: exactly the pairs (r, c) that mc2_identity_pairs_both_strands returns for the same arguments (and a large enough
+ * max_out): the identity is max(id+, id-), the same bits that call reports, and the strand is the one it reports (0 forward,
+ * 1 reverse, equal identities forward).  exclude_self != 0 drops (r, r) on both strands; it needs set_q == set_d.
+ * Order: that of mc2_identity_topk (identity descending, then database row ascending, -0.0 equal to +0.0).  A (r, c) pair
+ * appears once after the strand merge, so the order stays total; the strand is payload and never takes part in it.  The
+ * result therefore does not depend on survivor order, block sizes or how the query rows are split over calls or GPUs.
+ * Outputs: out_d, out_identity and out_strand (may be NULL) are (q_end - q_begin) x k_best, row-major; row r - q_begin holds
+ * the first min(k_best, hits) entries; unused slots hold d = UINT64_MAX, identity -1.0 and strand -1.  out_count and
+ * out_n_hits (may be NULL; the hit count over both strands) as in mc2_identity_topk.  *n_scored (may be NULL) is the forward
+ * in-window pair count, as mc2_identity_pairs_both_strands reports it.
+ * MC2_ERR_ARG, MC2_ERR_FEATURE: as mc2_identity_topk.
+ * How: one loop over blocks of query rows (the first block is the whole range) sweeps each block's rows forward and, for
+ * min_identity > 0, on the reverse-complement set, each into its own scratch of max(d_end - d_begin, 2^22) pairs; a block
+ * whose survivors overflow either scratch is swept again in smaller blocks.  The forward survivors keep max(id+, id-) with
+ * its strand; the reverse survivors whose id+ fails the threshold (the forward sweep's own decision) join them on strand 1;
+ * both lists are bucketed by query and each bucket is reduced to its top k_best on the device (topk.cu).  Extra device memory
+ * is the output table plus scratches of fixed size: it does not grow with the number of hits.  The reverse-complement set
+ * of set_q is built on first use and kept, as in mc2_identity_pairs_both_strands.
+ * mc2_debug_last_sweep afterwards: n_exact summed over every sweep of both strands, coarse = 1 iff every one took the coarse
+ * form. */
+int mc2_identity_topk_both_strands(mc2_ctx *ctx, const mc2_model *model, double min_identity, uint32_t k_best,
+				   const mc2_hset *set_q, uint64_t q_begin, uint64_t q_end, const mc2_hset *set_d, uint64_t d_begin,
+				   uint64_t d_end, int32_t upper_only, int32_t exclude_self, double cutoff, uint64_t *out_d,
+				   double *out_identity, int8_t *out_strand, uint32_t *out_count, uint64_t *out_n_hits,
+				   uint64_t *n_scored);
 
 /* Measured issue rate (warp-instructions per second, whole GPU) of the tile sweep's inner instruction pair -- VIMNMX.U16x2 on
  * the ALU pipe feeding IDP.2A on the FMA pipe, register operands only, 32 resident warps per SM: the denominator of
@@ -434,7 +461,7 @@ int mc2_debug_tile_reductions(mc2_ctx *ctx, const mc2_hset *set_q, uint64_t q_be
 			      uint64_t d_begin, uint64_t d_end, int32_t need, uint32_t *out_dot, uint32_t *out_emd, uint32_t *out_sad);
 
 /* Diagnostic (tests, benchmarks): of the last mc2_all_pairs / mc2_identity_pairs call on this context (for
- * mc2_identity_pairs_both_strands see there), *n_exact = the pairs the tile sweep sent through the exact fp64 epilogue (those its fp32 screen could not reject; 0 for the row-streaming
+ * mc2_identity_pairs_both_strands and the top-K searches see there), *n_exact = the pairs the tile sweep sent through the exact fp64 epilogue (those its fp32 screen could not reject; 0 for the row-streaming
  * kernels) and *coarse = 1 if it took the coarse form (the screen on 64 sampled cumulative bins), else 0. */
 int mc2_debug_last_sweep(mc2_ctx *ctx, uint64_t *n_exact, int32_t *coarse);
 

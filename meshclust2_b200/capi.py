@@ -38,7 +38,7 @@ SYMBOLS = [
     "mc2_seqs_total_bases", "mc2_count_kmers", "mc2_count_kmers_into", "mc2_count_kmers_auto", "mc2_hset_largest_count", "mc2_hset_alloc", "mc2_count_kmers_into_rows", "mc2_hset_refresh", "mc2_width_for_count", "mc2_kmer_table_increment", "mc2_hset_from_host", "mc2_hset_from_device", "mc2_hset_update_from_device", "mc2_hset_device_sideband", "mc2_hset_free",
     "mc2_hset_count", "mc2_hset_k", "mc2_hset_elem_bytes", "mc2_hset_device_bins", "mc2_hset_download", "mc2_hset_copy_to_device",
     "mc2_hset_set_sideband", "mc2_hset_set_row", "mc2_hset_assign_rows", "mc2_hset_reverse_complement", "mc2_model_create", "mc2_model_free", "mc2_model_desc_from_file",
-    "mc2_score_pairs", "mc2_get_close", "mc2_get_close_as", "mc2_filter", "mc2_filter_as", "mc2_merge", "mc2_all_pairs", "mc2_identity_pairs", "mc2_identity_pairs_both_strands", "mc2_identity_topk", "mc2_debug_tile_reductions", "mc2_debug_last_sweep", "mc2_distance", "mc2_mean_closest", "mc2_closest",
+    "mc2_score_pairs", "mc2_get_close", "mc2_get_close_as", "mc2_filter", "mc2_filter_as", "mc2_merge", "mc2_all_pairs", "mc2_identity_pairs", "mc2_identity_pairs_both_strands", "mc2_identity_topk", "mc2_identity_topk_both_strands", "mc2_debug_tile_reductions", "mc2_debug_last_sweep", "mc2_distance", "mc2_mean_closest", "mc2_closest",
     "mc2_update_centers", "mc2_merge_centers",
     "mc2_bench_score_pairs", "mc2_bench_count_kmers", "mc2_bench_issue_rate", "mc2_encode_dna", "mc2_encode_dna_batch",
 ]
@@ -108,6 +108,8 @@ def lib():
         L.mc2_identity_topk.argtypes = [C.c_void_p, C.c_void_p, C.c_double, C.c_uint32, C.c_void_p, C.c_uint64, C.c_uint64,
                                         C.c_void_p, C.c_uint64, C.c_uint64, C.c_int32, C.c_int32, C.c_double, C.c_void_p,
                                         C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.mc2_identity_topk_both_strands.argtypes = (L.mc2_identity_topk.argtypes[:15] + [C.c_void_p]
+                                                     + L.mc2_identity_topk.argtypes[15:])
         _lib = L
     return _lib
 
@@ -445,6 +447,31 @@ class Context:
         _check(lib().mc2_identity_topk(self.h, model.h, min_identity, k_best, set_q.h, q0, q1, set_d.h, d0, d1, int(upper_only),
                                        int(exclude_self), cutoff, _p(od), _p(oid), _p(cnt), _p(hits), C.byref(n_scored)))
         return dict(d=od, identity=oid, count=cnt, n_hits=hits, n_scored=n_scored.value)
+
+    def identity_topk_both_strands(self, model, set_q, set_d, min_identity, k_best, cutoff, q_range=None, d_range=None,
+                                   upper_only=False, exclude_self=False, out=None):
+        """Each query's k_best best identity_pairs_both_strands hits (identity = the better strand's), in identity_topk's
+        order.  Returns identity_topk's dict plus strand=int8[nq, K] (0 forward, 1 reverse, -1 in unused slots); n_scored
+        counts the forward in-window pairs.  out: optional (d, identity, strand, count, n_hits) arrays to fill."""
+        q0, q1 = q_range if q_range else (0, len(set_q))
+        d0, d1 = d_range if d_range else (0, len(set_d))
+        nq = max(q1 - q0, 0)
+        if out is not None:
+            od, oid, ostr, cnt, hits = out
+            assert od.shape == oid.shape == ostr.shape == (nq, k_best) and cnt.shape == hits.shape == (nq,)
+            assert od.dtype == np.uint64 and oid.dtype == np.float64 and ostr.dtype == np.int8
+            assert cnt.dtype == np.uint32 and hits.dtype == np.uint64
+        else:
+            od = np.empty((nq, k_best), dtype=np.uint64)
+            oid = np.empty((nq, k_best))
+            ostr = np.empty((nq, k_best), dtype=np.int8)
+            cnt = np.empty(nq, dtype=np.uint32)
+            hits = np.empty(nq, dtype=np.uint64)
+        n_scored = C.c_uint64()
+        _check(lib().mc2_identity_topk_both_strands(self.h, model.h, min_identity, k_best, set_q.h, q0, q1, set_d.h, d0, d1,
+                                                    int(upper_only), int(exclude_self), cutoff, _p(od), _p(oid), _p(ostr),
+                                                    _p(cnt), _p(hits), C.byref(n_scored)))
+        return dict(d=od, identity=oid, strand=ostr, count=cnt, n_hits=hits, n_scored=n_scored.value)
 
     def issue_rate(self, iters=100000):
         """measured warp-instructions / s of the VIMNMX.U16x2 + IDP.2A pair (roofline denominator of the tile sweep)"""

@@ -317,6 +317,15 @@ int launch_topk_scatter(mc2_ctx *ctx, const u64 *sq, const u64 *sd, const double
 			const u64 *off, u32 *cur, double *bid, u64 *bd);
 int launch_topk_select(mc2_ctx *ctx, const u64 *off, const double *bid, const u64 *bd, u64 rows, u32 k_best, u64 d_begin,
 		       u64 *out_d, double *out_id, u32 *out_cnt, u64 *out_hits);
+// the same with a strand per entry: a list with fwd != NULL keeps only its entries with !(fwd[i] >= t); sstr NULL = strand 1
+int launch_topk_count_strand(mc2_ctx *ctx, const u64 *sq, const u64 *sd, const double *fwd, double t, u64 n, u64 qb,
+			     int exclude_self, u32 *cnt);
+int launch_topk_scatter_strand(mc2_ctx *ctx, const u64 *sq, const u64 *sd, const double *ss, const int8_t *sstr,
+			       const double *fwd, double t, u64 n, u64 qb, int exclude_self, const u64 *off, u32 *cur,
+			       double *bid, u64 *bd, int8_t *bstr);
+int launch_topk_select_strand(mc2_ctx *ctx, const u64 *off, const double *bid, const u64 *bd, const int8_t *bstr, u64 rows,
+			      u32 k_best, u64 d_begin, u64 *out_d, double *out_id, int8_t *out_str, u32 *out_cnt,
+			      u64 *out_hits);
 int launch_merge_batch(mc2_ctx *ctx, const double *d_dist, const uint8_t *d_skipped, const uint8_t *d_close, const u64 *d_off,
 		       u64 n_centers, long long *d_out);
 

@@ -1,4 +1,5 @@
-// topk.cu — per-query selection of the top-K identity search (mc2_identity_topk, orchestrated in mc2_api.cu).
+// topk.cu — per-query selection of the top-K identity searches (mc2_identity_topk and mc2_identity_topk_both_strands,
+// orchestrated in mc2_api.cu).
 //
 // The unchanged identity sweep writes one block of query rows' survivors (q, d, identity), in no order, into a scratch.
 // Here they are bucketed by query (a count, an exclusive scan, a scatter) and each bucket is reduced to its first K entries
@@ -13,6 +14,11 @@
 // the K-th entry falls; it stops as soon as every entry with the chosen prefix is needed.  The winners, exactly K, are
 // gathered into shared memory and sorted there.  Passes stream the bucket from global memory (L2), so a bucket of any
 // size costs shared memory for K entries only.
+//
+// The both-strand search (STRAND = true) buckets two lists per block: the forward survivors with their picked strand and
+// identity, and the reverse survivors that the forward sweep rejected (fwd = id+, kept when !(id+ >= t), strand 1).  The
+// strand travels with each entry as payload, in its own shared array; it never takes part in the order.  The one-strand
+// instantiation (STRAND = false) does the work it did before the strand existed.
 #include "mc2_internal.cuh"
 
 namespace mc2 {
@@ -20,32 +26,45 @@ namespace mc2 {
 static constexpr int kTopkThreads = 256;
 static constexpr u32 kTopkMaxK = 1024;
 
-// survivors per block query (self pairs dropped when asked)
+// survivors per block query (self pairs dropped when asked); STRAND with fwd != NULL: only those with !(fwd[i] >= t)
+template <bool STRAND>
 __global__ void __launch_bounds__(256) topk_count_kernel(const u64 *__restrict__ sq, const u64 *__restrict__ sd, u64 n, u64 qb,
-							  int exclude_self, u32 *__restrict__ cnt)
+							  int exclude_self, const double *__restrict__ fwd, double t, u32 *__restrict__ cnt)
 {
 	for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (u64)gridDim.x * blockDim.x) {
 		const u64 q = sq[i];
+		if (STRAND && fwd && fwd[i] >= t) {
+			continue;
+		}
 		if (!(exclude_self && sd[i] == q)) {
 			atomicAdd(cnt + (q - qb), 1u);
 		}
 	}
 }
 
-// (identity, d) of each kept survivor into its query's bucket [off[q - qb], off[q - qb + 1]); cur (zeroed) is the fill cursor
+// (identity, d) of each kept survivor into its query's bucket [off[q - qb], off[q - qb + 1]); cur (zeroed) is the fill cursor.
+// STRAND: also its strand into bstr, sstr[i] (sstr NULL: 1), with the filter of topk_count_kernel
+template <bool STRAND>
 __global__ void __launch_bounds__(256) topk_scatter_kernel(const u64 *__restrict__ sq, const u64 *__restrict__ sd,
-							    const double *__restrict__ ss, u64 n, u64 qb, int exclude_self,
+							    const double *__restrict__ ss, const int8_t *__restrict__ sstr,
+							    const double *__restrict__ fwd, double t, u64 n, u64 qb, int exclude_self,
 							    const u64 *__restrict__ off, u32 *__restrict__ cur, double *__restrict__ bid,
-							    u64 *__restrict__ bd)
+							    u64 *__restrict__ bd, int8_t *__restrict__ bstr)
 {
 	for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (u64)gridDim.x * blockDim.x) {
 		const u64 q = sq[i], d = sd[i];
+		if (STRAND && fwd && fwd[i] >= t) {
+			continue;
+		}
 		if (exclude_self && d == q) {
 			continue;
 		}
 		const u64 pos = off[q - qb] + atomicAdd(cur + (q - qb), 1u);
 		bid[pos] = ss[i];
 		bd[pos] = d;
+		if (STRAND) {
+			bstr[pos] = sstr ? sstr[i] : (int8_t)1;
+		}
 	}
 }
 
@@ -78,14 +97,18 @@ __device__ __forceinline__ u32 mask_lo(int p)
 }
 
 // One CTA per block query (grid-stride): out row r = the first min(K, n) entries of bucket r in (identity desc, d asc)
-// order, then padding (d = UINT64_MAX, identity -1.0); out_cnt[r] = min(K, n), out_hits[r] = n.
+// order, then padding (d = UINT64_MAX, identity -1.0); out_cnt[r] = min(K, n), out_hits[r] = n.  STRAND: each entry's
+// strand (bstr) moves with it into out_str, padding -1.
+template <bool STRAND>
 __global__ void __launch_bounds__(kTopkThreads) topk_select_kernel(const u64 *__restrict__ off, const double *__restrict__ bid,
-								   const u64 *__restrict__ bd, u64 rows, u32 K, u64 d_begin,
-								   u64 *__restrict__ out_d, double *__restrict__ out_id,
-								   u32 *__restrict__ out_cnt, u64 *__restrict__ out_hits)
+								   const u64 *__restrict__ bd, const int8_t *__restrict__ bstr, u64 rows,
+								   u32 K, u64 d_begin, u64 *__restrict__ out_d, double *__restrict__ out_id,
+								   int8_t *__restrict__ out_str, u32 *__restrict__ out_cnt,
+								   u64 *__restrict__ out_hits)
 {
 	__shared__ double s_id[kTopkMaxK];
 	__shared__ u64 s_d[kTopkMaxK];
+	__shared__ int8_t s_str[STRAND ? kTopkMaxK : 1];
 	__shared__ u32 hist[256];
 	__shared__ u32 warp_tot[kTopkThreads / 32];
 	__shared__ u32 s_digit, s_above, s_count, s_nwin;
@@ -94,11 +117,15 @@ __global__ void __launch_bounds__(kTopkThreads) topk_select_kernel(const u64 *__
 		const u64 b = off[row], n = off[row + 1] - b;
 		const double *id = bid + b;
 		const u64 *dd = bd + b;
+		const int8_t *ds = STRAND ? bstr + b : nullptr;
 		const u32 take = n < K ? (u32)n : K;
 		if (n <= K) {
 			for (u32 i = tid; i < take; i += kTopkThreads) {
 				s_id[i] = id[i];
 				s_d[i] = dd[i];
+				if (STRAND) {
+					s_str[i] = ds[i];
+				}
 			}
 		} else {
 			u64 phi = 0;
@@ -168,6 +195,9 @@ __global__ void __launch_bounds__(kTopkThreads) topk_select_kernel(const u64 *__
 					const u32 slot = atomicAdd(&s_nwin, 1u);
 					s_id[slot] = v;
 					s_d[slot] = d;
+					if (STRAND) {
+						s_str[slot] = ds[i];
+					}
 				}
 			}
 		}
@@ -194,6 +224,11 @@ __global__ void __launch_bounds__(kTopkThreads) topk_select_kernel(const u64 *__
 						s_id[y] = vx;
 						s_d[x] = dy;
 						s_d[y] = dx;
+						if (STRAND) {
+							const int8_t sx = s_str[x];
+							s_str[x] = s_str[y];
+							s_str[y] = sx;
+						}
 					}
 				}
 				__syncthreads();
@@ -205,6 +240,9 @@ __global__ void __launch_bounds__(kTopkThreads) topk_select_kernel(const u64 *__
 			const bool have = j < take;
 			od[j] = have ? s_d[j] : ~0ull;
 			oi[j] = have ? s_id[j] : -1.0;
+			if (STRAND) {
+				out_str[row * K + j] = have ? s_str[j] : (int8_t)-1;
+			}
 		}
 		if (tid == 0) {
 			out_cnt[row] = take;
@@ -225,7 +263,7 @@ int launch_topk_count(mc2_ctx *ctx, const u64 *sq, const u64 *sd, u64 n, u64 qb,
 	if (n == 0) {
 		return MC2_OK;
 	}
-	topk_count_kernel<<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, n, qb, exclude_self, cnt);
+	topk_count_kernel<false><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, n, qb, exclude_self, nullptr, 0.0, cnt);
 	ctx->launches++;
 	MC2_CUDA(cudaGetLastError());
 	return MC2_OK;
@@ -237,7 +275,8 @@ int launch_topk_scatter(mc2_ctx *ctx, const u64 *sq, const u64 *sd, const double
 	if (n == 0) {
 		return MC2_OK;
 	}
-	topk_scatter_kernel<<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, ss, n, qb, exclude_self, off, cur, bid, bd);
+	topk_scatter_kernel<false><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, ss, nullptr, nullptr, 0.0, n, qb,
+											 exclude_self, off, cur, bid, bd, nullptr);
 	ctx->launches++;
 	MC2_CUDA(cudaGetLastError());
 	return MC2_OK;
@@ -249,8 +288,50 @@ int launch_topk_select(mc2_ctx *ctx, const u64 *off, const double *bid, const u6
 	if (rows == 0) {
 		return MC2_OK;
 	}
-	topk_select_kernel<<<grid_for(ctx, rows, 1, 8), kTopkThreads, 0, ctx->stream>>>(off, bid, bd, rows, k_best, d_begin, out_d,
-											 out_id, out_cnt, out_hits);
+	topk_select_kernel<false><<<grid_for(ctx, rows, 1, 8), kTopkThreads, 0, ctx->stream>>>(off, bid, bd, nullptr, rows, k_best,
+												   d_begin, out_d, out_id, nullptr,
+												   out_cnt, out_hits);
+	ctx->launches++;
+	MC2_CUDA(cudaGetLastError());
+	return MC2_OK;
+}
+
+int launch_topk_count_strand(mc2_ctx *ctx, const u64 *sq, const u64 *sd, const double *fwd, double t, u64 n, u64 qb,
+			     int exclude_self, u32 *cnt)
+{
+	if (n == 0) {
+		return MC2_OK;
+	}
+	topk_count_kernel<true><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, n, qb, exclude_self, fwd, t, cnt);
+	ctx->launches++;
+	MC2_CUDA(cudaGetLastError());
+	return MC2_OK;
+}
+
+int launch_topk_scatter_strand(mc2_ctx *ctx, const u64 *sq, const u64 *sd, const double *ss, const int8_t *sstr,
+			       const double *fwd, double t, u64 n, u64 qb, int exclude_self, const u64 *off, u32 *cur,
+			       double *bid, u64 *bd, int8_t *bstr)
+{
+	if (n == 0) {
+		return MC2_OK;
+	}
+	topk_scatter_kernel<true><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, ss, sstr, fwd, t, n, qb, exclude_self,
+											off, cur, bid, bd, bstr);
+	ctx->launches++;
+	MC2_CUDA(cudaGetLastError());
+	return MC2_OK;
+}
+
+int launch_topk_select_strand(mc2_ctx *ctx, const u64 *off, const double *bid, const u64 *bd, const int8_t *bstr, u64 rows,
+			      u32 k_best, u64 d_begin, u64 *out_d, double *out_id, int8_t *out_str, u32 *out_cnt,
+			      u64 *out_hits)
+{
+	if (rows == 0) {
+		return MC2_OK;
+	}
+	topk_select_kernel<true><<<grid_for(ctx, rows, 1, 8), kTopkThreads, 0, ctx->stream>>>(off, bid, bd, bstr, rows, k_best,
+												  d_begin, out_d, out_id, out_str,
+												  out_cnt, out_hits);
 	ctx->launches++;
 	MC2_CUDA(cudaGetLastError());
 	return MC2_OK;

@@ -156,9 +156,10 @@ def all_pairs_step(engine, comm, torch, n_total, cutoff, upper_only=True, blocks
     (regression model, min_identity, True) searches both strands of each query (identity = the better strand's,
     Survivors.strands() = which strand).  Each rank reverse-complements the gathered set itself: no extra collective, and no
     floating-point value is reduced across ranks.
-    top_k: with a one-strand identity search, keep each query's top_k best hits instead of the survivor list: `topk` is
-    this rank's [(q0, q1, table)] with table = dict(d [q1-q0, top_k], identity [q1-q0, top_k], count, n_hits) as
-    engine.topk returns it.  A query lives in exactly one block of one rank, so the tables are complete per query and
+    top_k: with an identity search, keep each query's top_k best hits instead of the survivor list: `topk` is this rank's
+    [(q0, q1, table)] with table = dict(d [q1-q0, top_k], identity [q1-q0, top_k], count, n_hits) as engine.topk returns
+    it; a both-strand search ranks each pair's better strand (engine.topk_both_strands) and its tables add
+    strand [q1-q0, top_k].  A query lives in exactly one block of one rank, so the tables are complete per query and
     nothing but the counters is reduced; n_close is the total hit count.
 
     engine.count()                  K1 over this rank's shard
@@ -169,9 +170,13 @@ def all_pairs_step(engine, comm, torch, n_total, cutoff, upper_only=True, blocks
                                     -> (n_survivors, n_scored, survivors: array [m,2], (q[m], d[m]), (q[m], d[m], score[m])
                                         or, both strands, (q[m], d[m], identity[m], strand[m]))
     engine.topk(q0, q1, upper_only, cutoff, (model, min_identity), top_k) -> (n_hits, n_scored, table)
+    engine.topk_both_strands(q0, q1, upper_only, cutoff, (model, min_identity), top_k) -> (n_hits, n_scored, table)
+                                    (optional: an engine without it takes no both-strand top_k)
     Returns dict(n_scored, n_close, survivors (this rank's), topk (this rank's, [] without top_k), blocks)."""
-    if top_k is not None and (identity is None or (len(identity) > 2 and identity[2])):
-        raise ValueError("top_k needs a one-strand identity search: identity=(regression model, min_identity)")
+    both_strands = identity is not None and len(identity) > 2 and bool(identity[2])
+    if top_k is not None and (identity is None or (both_strands and not hasattr(engine, "topk_both_strands"))):
+        raise ValueError("top_k needs a one-strand identity search: identity=(regression model, min_identity), or an "
+                         "engine with topk_both_strands for identity=(regression model, min_identity, True)")
     if comm.world > 1 and hasattr(engine, "count_and_gather_in_place"):
         # the product engine: K1 writes this rank's rows straight into the full set, the all-gathers run in place on it
         engine.count_and_gather_in_place(comm, n_total)
@@ -199,7 +204,10 @@ def all_pairs_step(engine, comm, torch, n_total, cutoff, upper_only=True, blocks
     tables = []
     for q0, q1 in blocks:
         if top_k is not None:
-            ns, sc, table = engine.topk(q0, q1, upper_only, cutoff, identity, top_k)
+            if both_strands:
+                ns, sc, table = engine.topk_both_strands(q0, q1, upper_only, cutoff, identity[:2], top_k)
+            else:
+                ns, sc, table = engine.topk(q0, q1, upper_only, cutoff, identity, top_k)
             tables.append((q0, q1, table))
             n_close += ns
             n_scored += sc
@@ -514,6 +522,15 @@ class GpuEngine:
         nd = min(len(self.full), getattr(self, "n_total", None) or len(self.full))   # rows past n_total are shard padding
         r = self.ctx.identity_topk(model, self.full, self.full, t, top_k, cutoff, q_range=(q0, q1), d_range=(0, nd),
                                    upper_only=upper_only)
+        return int(r["n_hits"].sum()), r["n_scored"], r
+
+    def topk_both_strands(self, q0, q1, upper_only, cutoff, identity, top_k):
+        """each query's top_k best identity hits over both strands (Context.identity_topk_both_strands) -> (total hits,
+        n_scored, table with strand)"""
+        model, t = identity[:2]
+        nd = min(len(self.full), getattr(self, "n_total", None) or len(self.full))   # rows past n_total are shard padding
+        r = self.ctx.identity_topk_both_strands(model, self.full, self.full, t, top_k, cutoff, q_range=(q0, q1),
+                                                d_range=(0, nd), upper_only=upper_only)
         return int(r["n_hits"].sum()), r["n_scored"], r
 
     def sweep(self, q0, q1, upper_only, cutoff, max_out, identity=None):
