@@ -462,8 +462,10 @@ int mc2_debug_tile_reductions(mc2_ctx *ctx, const mc2_hset *set_q, uint64_t q_be
 
 /* Diagnostic (tests, benchmarks): of the last mc2_all_pairs / mc2_identity_pairs call on this context (for
  * mc2_identity_pairs_both_strands and the top-K searches see there), *n_exact = the pairs the tile sweep sent through the exact fp64 epilogue (those its fp32 screen could not reject; 0 for the row-streaming
- * kernels) and *coarse = 1 if it took the coarse form (the screen on 64 sampled cumulative bins), else 0. */
-int mc2_debug_last_sweep(mc2_ctx *ctx, uint64_t *n_exact, int32_t *coarse);
+ * kernels) and *coarse = 1 if it took the coarse form (the screen on 64 sampled cumulative bins), else 0.  *n_inline (may
+ * be NULL) = how many of the n_exact pairs the coarse form refined inside the sweep because its candidate buffer (2^23
+ * records) was full; the others were refined by the kernel that follows the sweep. */
+int mc2_debug_last_sweep(mc2_ctx *ctx, uint64_t *n_exact, int32_t *coarse, uint64_t *n_inline);
 
 /* DivergencePoint<T>::distance (src/clutil/DivergencePoint.cpp:70-82) for pairs of rows */
 int mc2_distance(mc2_ctx *ctx, const mc2_pairs *pairs, uint64_t *out);

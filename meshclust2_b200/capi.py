@@ -491,11 +491,12 @@ class Context:
         return out
 
     def last_sweep(self):
-        """Diagnostic: {n_exact, coarse} of the last all_pairs / identity_pairs call -- the pairs the tile sweep sent
-        through the exact epilogue, and whether it took the coarse form"""
-        n, c = C.c_uint64(), C.c_int32()
-        _check(lib().mc2_debug_last_sweep(self.h, C.byref(n), C.byref(c)))
-        return dict(n_exact=n.value, coarse=bool(c.value))
+        """Diagnostic: {n_exact, coarse, n_inline} of the last all_pairs / identity_pairs call -- the pairs the tile sweep
+        sent through the exact epilogue, whether it took the coarse form, and how many of those pairs the coarse form
+        refined inside the sweep because its candidate buffer was full"""
+        n, c, i = C.c_uint64(), C.c_int32(), C.c_uint64()
+        _check(lib().mc2_debug_last_sweep(self.h, C.byref(n), C.byref(c), C.byref(i)))
+        return dict(n_exact=n.value, coarse=bool(c.value), n_inline=i.value)
 
     def distance(self, set_a, set_b, ia, ib):
         p = self._pairs(set_a, set_b, ia, ib, len(ia))

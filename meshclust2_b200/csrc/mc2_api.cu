@@ -107,6 +107,8 @@ struct CtxExtra {
 	// the last all-pairs / identity sweep: pairs the tile sweep sent through the exact epilogue, 1 if it took the coarse form
 	u64 last_exact = 0;
 	int last_coarse = 0;
+	u64 last_inline = 0; // of those, the pairs the coarse sweep refined inline because its candidate buffer was full
+	u64 sum_inline = 0;  // last_inline summed over the sweeps of the current call
 };
 
 static cudaEvent_t prof_event(CtxExtra *x)
@@ -714,6 +716,7 @@ void mc2_ctx_destroy(mc2_ctx *ctx)
 	cudaFreeHost(ctx->h_slot);
 	cudaFree(ctx->d_slot);
 	cudaFree(ctx->d_sched);
+	cudaFree(ctx->d_cand);
 	cudaEventDestroy(ctx->ev0);
 	cudaEventDestroy(ctx->ev1);
 	cudaStreamDestroy(ctx->stream);
@@ -2175,7 +2178,7 @@ static DevModel identity_model(const mc2_model *model, double min_identity)
 }
 
 // One launch of the all-pairs sweep into device buffers of capacity max_out (arguments checked by the caller): *total = all
-// survivors (may exceed max_out), the sweep's diagnostics in last_exact / last_coarse.  The device error word is fetched
+// survivors (may exceed max_out), the sweep's diagnostics in last_exact / last_coarse / last_inline.  The device error word is fetched
 // into ctx->h_err, not checked.
 static int run_sweep(mc2_ctx *ctx, const DevModel &dm, int identity, double min_identity, const mc2_hset *set_q, u64 q_begin,
 		     u64 q_end, const mc2_hset *set_d, u64 d_begin, u64 d_end, int32_t upper_only, double cutoff, u64 max_out,
@@ -2193,12 +2196,14 @@ static int run_sweep(mc2_ctx *ctx, const DevModel &dm, int identity, double min_
 	if (rc == MC2_OK) rc = fetch_err(ctx);
 	if (rc != MC2_OK) return rc;
 	cudaStream_t st = ctx->stream;
-	MC2_CUDA(cudaMemcpyAsync(ctx->h_slot, d_counters, 32, cudaMemcpyDeviceToHost, st));
+	MC2_CUDA(cudaMemcpyAsync(ctx->h_slot, d_counters, 40, cudaMemcpyDeviceToHost, st));
 	MC2_CUDA(cudaStreamSynchronize(st));
 	*total = ((u64 *)ctx->h_slot)[0];
 	if (n_scored) *n_scored = ((u64 *)ctx->h_slot)[1];
 	x->last_exact = ((u64 *)ctx->h_slot)[2];
 	x->last_coarse = ((u64 *)ctx->h_slot)[3] != 0;
+	x->last_inline = ((u64 *)ctx->h_slot)[4];
+	x->sum_inline += x->last_inline;
 	return MC2_OK;
 }
 
@@ -2222,6 +2227,7 @@ static int sweep_pairs(const char *who, mc2_ctx *ctx, const DevModel &dm, int id
 	CtxExtra *x = extra(ctx);
 	x->last_exact = 0;
 	x->last_coarse = 0;
+	x->last_inline = x->sum_inline = 0;
 	if (q_begin == q_end || d_begin == d_end) return MC2_OK;
 	int rc;
 	u64 cap = max_out ? max_out : 1;
@@ -2415,6 +2421,7 @@ int mc2_identity_pairs_both_strands(mc2_ctx *ctx, const mc2_model *model, double
 	CtxExtra *x = extra(ctx);
 	x->last_exact = 0;
 	x->last_coarse = 0;
+	x->last_inline = x->sum_inline = 0;
 	if (q_begin == q_end || d_begin == d_end) return MC2_OK;
 	const double t = min_identity;
 	const DevModel dm = identity_model(model, t);
@@ -2485,6 +2492,7 @@ int mc2_identity_pairs_both_strands(mc2_ctx *ctx, const mc2_model *model, double
 	const u64 total = ((u64 *)ctx->h_slot)[0];
 	*n_out = total;
 	x->last_exact = exact;
+	x->last_inline = x->sum_inline;
 	x->last_coarse = coarse;
 	const u64 got = std::min<u64>(total, max_out);
 	if (got) {
@@ -2536,6 +2544,7 @@ int mc2_identity_topk(mc2_ctx *ctx, const mc2_model *model, double min_identity,
 	CtxExtra *x = extra(ctx);
 	x->last_exact = 0;
 	x->last_coarse = 0;
+	x->last_inline = x->sum_inline = 0;
 	if (nq == 0) return MC2_OK;
 	if (d_begin == d_end) {
 		std::fill(out_d, out_d + nq * K, UINT64_MAX);
@@ -2578,6 +2587,7 @@ int mc2_identity_topk(mc2_ctx *ctx, const mc2_model *model, double min_identity,
 	});
 	if (rc != MC2_OK) return rc;
 	x->last_exact = exact;
+	x->last_inline = x->sum_inline;
 	x->last_coarse = coarse;
 	if (n_scored) *n_scored = ns;
 	MC2_CUDA(cudaMemcpyAsync(out_d, od, nq * K * 8, cudaMemcpyDeviceToHost, st));
@@ -2604,6 +2614,7 @@ int mc2_identity_topk_both_strands(mc2_ctx *ctx, const mc2_model *model, double 
 	CtxExtra *x = extra(ctx);
 	x->last_exact = 0;
 	x->last_coarse = 0;
+	x->last_inline = x->sum_inline = 0;
 	if (nq == 0) return MC2_OK;
 	if (d_begin == d_end) {
 		std::fill(out_d, out_d + nq * K, UINT64_MAX);
@@ -2677,6 +2688,7 @@ int mc2_identity_topk_both_strands(mc2_ctx *ctx, const mc2_model *model, double 
 	});
 	if (rc != MC2_OK) return rc;
 	x->last_exact = exact;
+	x->last_inline = x->sum_inline;
 	x->last_coarse = coarse;
 	if (n_scored) *n_scored = ns;
 	MC2_CUDA(cudaMemcpyAsync(out_d, od, nq * K * 8, cudaMemcpyDeviceToHost, st));
@@ -2688,12 +2700,13 @@ int mc2_identity_topk_both_strands(mc2_ctx *ctx, const mc2_model *model, double 
 	return MC2_OK;
 }
 
-int mc2_debug_last_sweep(mc2_ctx *ctx, uint64_t *n_exact, int32_t *coarse)
+int mc2_debug_last_sweep(mc2_ctx *ctx, uint64_t *n_exact, int32_t *coarse, uint64_t *n_inline)
 {
 	MC2_REQUIRE(ctx && n_exact && coarse, "mc2_debug_last_sweep: NULL argument");
 	const CtxExtra *x = extra(ctx);
 	*n_exact = x->last_exact;
 	*coarse = x->last_coarse;
+	if (n_inline) *n_inline = x->last_inline;
 	return MC2_OK;
 }
 

@@ -171,6 +171,7 @@ struct mc2_ctx {
 	int prof_on;      // per-kernel event timing enabled
 	int err_dirty;    // the device error word may be non-zero (set by reset_err, cleared by a clean check_err)
 	void *d_sched;    // tile schedule of the tile sweep (tile_sweep.cu), allocated on first use
+	void *d_cand;     // the coarse tile sweep's candidate buffer (tile_sweep.cu), allocated on first use
 	// resident scan server (pair_score.cu scan_server_kernel): mailbox in mapped page-locked memory, its own stream
 	mc2::ScanMailbox *mb;
 	cudaStream_t server_stream;

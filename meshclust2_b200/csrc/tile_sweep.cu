@@ -37,9 +37,10 @@
 // values at the 64 block ends s_j = 16 j + 15 (mc2_hset::cum16s, one ring stage) bound the whole sum:
 // 16 (M - T) <= sum_i m_i <= 16 M with M = sum_j m(s_j), T = m(s_63) = min(totP, totQ).  A tile streams the 8 u8 stages
 // and that single stage; the screen takes the EMD as the interval [cs - 32 M, cs - 32 (M - T)] and the candidates it
-// keeps get the exact sum min(cumP, cumQ) over the full rows from global memory (one warp per candidate; the rows are
-// prefetched into L2 when the screen keeps the pair) before the same exact epilogue, so scores and decisions are the bits
-// of the full form.
+// keeps go, as 16-byte records, to a global candidate buffer.  refine_kernel, launched after the sweep on the same stream,
+// gives them the exact sum min(cumP, cumQ) over the full rows from global memory (one warp per candidate, many warps per
+// SM) and the same exact epilogue, so scores and decisions are the bits of the full form.  Candidates beyond the buffer
+// (2^23 records) are refined inside the sweep by the warp that found them, as the full form's list is.
 // Identity search (Params::identity, mc2_identity_pairs): a regression model, clamp(sum) >= t <=> sum >= t for 0 < t <= 1,
 // so the same screen rejects on sum + bound < t - margin (DevModel::scr_thr, set per call) and the exact epilogue keeps
 // the pairs whose clamped sum is >= t.  The mode is a uniform runtime field read by the epilogue warps only.
@@ -88,7 +89,12 @@ template <int NEED, bool COARSE> struct Layout {
 	// pairs a thread of the epilogue screens at a time (query columns per tcgen05.ld): 4 where the screen's scratch
 	// (slots x pairs x NEW * 32 threads x 4 bytes) leaves room for a candidate list that is flushed once per tile, else 2
 	static constexpr int NP = scr_slots(NEED & 7) <= 7 ? 4 : 2;
-	static constexpr int LIST_CAP = NP == 4 ? 192 : 128; // candidate records per epilogue warp
+	// candidate records per epilogue warp, flushed through the exact epilogue when nearly full and at the end of the tile.
+	// The coarse form copies each ballot batch to the global candidate buffer (refine_kernel) instead; its list fills only
+	// once that buffer is full, and a batch at a time would then pay a pass of the exact epilogue over mostly idle lanes.
+	// With 16 epilogue warps the list is 176 records, which keeps the CTA within the 196 KB shared-memory carve-out
+	// (Smem::SMALL_CARVEOUT): 192 would take the 228 KB one and halve what is left of the L1 for the epilogue's row loads.
+	static constexpr int LIST_CAP = EPI_HEAVY ? 176 : NP == 4 ? 192 : 128;
 	static constexpr int STAGES = EPI_HEAVY ? 2 : 4;
 	static constexpr int REGS_LAUNCH = 72, REGS_CTRL = 24, REGS_COMPUTE = 80, REGS_EPI = 80;
 	static_assert(NCW % 4 == 0 && NEW % 4 == 0, "roles are whole warpgroups");
@@ -126,7 +132,16 @@ struct Params {
 	const u32 *sched;       // [n_super + 1] exclusive prefix of items per super-row (device)
 	// raw mode (tests): dense (q1-q0) x (d1-d0) matrices of the reductions instead of scoring
 	u32 *raw_dot, *raw_emd, *raw_sad;
+	// coarse form: the screen's candidates as records {q - q0, d - d0, dot, sad} (q - q0 = CB_EMPTY: unused slot), refined
+	// by refine_kernel after the sweep; counters[5] counts the slots reserved (whole chunks, may pass cb_cap), counters[4]
+	// the pairs refined inside the sweep because the buffer was full
+	uint4 *cbuf;
+	u32 cb_cap;             // records, a multiple of CB_CHUNK
 };
+constexpr u32 CB_CHUNK = 512;            // records a warp reserves at a time (>= one ballot batch, 32 x NP)
+constexpr u32 CB_EMPTY = 0xFFFFFFFFu;
+constexpr u32 CAND_CAP = 1u << 23;       // records of the candidate buffer (128 MiB); beyond it, candidates are refined inline
+static_assert(CAND_CAP % CB_CHUNK == 0, "a reservation either fits the buffer whole or finds it full");
 
 // ---------------------------------------------------------------------------------------------------------------
 // PTX wrappers
@@ -559,6 +574,9 @@ template <int NEED, bool COARSE> struct Smem {
 	static constexpr int TOTAL = MISC + 64 + 1024;                                    // + alignment slack
 	static_assert(2 * LY::STAGES + 8 <= 32, "mbarriers");
 	static_assert(TOTAL <= 232448, "shared memory per CTA");
+	// 196 KB carve-out less the 1 KB the system reserves per CTA
+	static constexpr bool SMALL_CARVEOUT = TOTAL + 1024 <= 196 * 1024;
+	static_assert(!LY::EPI_HEAVY || SMALL_CARVEOUT, "the epilogue-heavy layout leaves the L1 its larger share");
 };
 
 // ONE: rows of one 1 KiB slab (k = 5), stage counts known at compile time; otherwise Params::n_slabs slabs per row.
@@ -861,7 +879,9 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 		}
 		const int qc0 = (ew >> 2) * QE; // this warp's query columns: qc0 .. qc0 + QE - 1
 		u32 it = 0;
-		u64 scored_total = 0, exact_total = 0;
+		u64 scored_total = 0, exact_total = 0, inline_total = 0;
+		u32 cb_pos = 0, cb_end = 0; // coarse form: this warp's unused slots [cb_pos, cb_end) of the candidate buffer
+		bool cb_full = false;       // ... and whether a reservation found the buffer full (warp-uniform)
 		if (COARSE && blockIdx.x == 0 && etid == 0) {
 			p.counters[3] = 1;
 		}
@@ -980,10 +1000,10 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 								rec.emd = ve[k];
 								rec.sad = vs[k];
 								s_list[n_list + __popc(m & ((1u << lane) - 1))] = rec;
-								if constexpr (COARSE) {
-									// the flush refines one candidate at a time, and each reads both full cumulative
-									// rows (cum16 is larger than L2): start bringing them into L2 now, so that the
-									// flush's loads wait for L2 and not for a DRAM round trip each
+								if (COARSE && cb_full) {
+									// the inline flush refines one candidate at a time, and each reads both full
+									// cumulative rows (cum16 is larger than L2): start bringing them into L2 now, so
+									// that the flush's loads wait for L2 and not for a DRAM round trip each
 									l2_prefetch(p.cumQ + (qrow0 + qc + k) * NBINS, NBINS * 2);
 									l2_prefetch(p.cumD + d * NBINS, NBINS * 2);
 								}
@@ -991,9 +1011,46 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 							n_list += __popc(m);
 						}
 						}
+						if constexpr (COARSE) {
+							// the batch -> the candidate buffer; a reservation is one atomic per CB_CHUNK slots, and the
+							// slots a chunk cannot use are marked empty.  Once the buffer is full, the batches stay in
+							// the list and go through the exact epilogue below, as the full form's do.
+							if (n_list != 0 && !cb_full) {
+								__syncwarp();
+								if (cb_pos + n_list > cb_end) {
+									for (u32 i = cb_pos + lane; i < cb_end; i += 32) {
+										p.cbuf[i] = make_uint4(CB_EMPTY, 0, 0, 0);
+									}
+									u64 b = 0;
+									if (lane == 0) {
+										b = atomicAdd(p.counters + 5, (u64)CB_CHUNK);
+									}
+									b = __shfl_sync(0xffffffffu, b, 0);
+									cb_full = b + CB_CHUNK > p.cb_cap;
+									cb_pos = cb_full ? 0u : (u32)b;
+									cb_end = cb_full ? 0u : (u32)b + CB_CHUNK;
+								}
+								if (!cb_full) {
+									for (u32 i = lane; i < n_list; i += 32) {
+										const Cand c = s_list[i];
+										const u32 dq = (u32)(qrow0 - p.q0) + (c.pair & 63);
+										const u32 dd = (u32)(drow0 - p.d0) + ((c.pair >> 6) & 1) * 128 + quarter * 32 + ((c.pair >> 8) & 31);
+										p.cbuf[cb_pos + i] = make_uint4(dq, dd, c.dot, c.sad);
+									}
+									cb_pos += n_list;
+									exact_total += n_list;
+									n_list = 0;
+								}
+								__syncwarp();
+							}
+						}
 						if (n_list > LIST_CAP - 32 * NP || (r == 1 && qc == qc0 + QE - NP)) {
 							__syncwarp();
 							exact_total += n_list;
+							if (COARSE) {
+								inline_total += n_list;
+							}
+#pragma unroll 1
 							for (u32 base = 0; base < n_list; base += 32) {
 								const u32 e = base + (u32)lane;
 								// coarse form: the exact sum min(cumP, cumQ) of the batch's candidates, one warp per
@@ -1089,12 +1146,106 @@ tile_sweep_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ P
 			if (lane == 0 && exact_total) { // warp-uniform
 				atomicAdd(p.counters + 2, exact_total);
 			}
+			if (COARSE) {
+				for (u32 i = cb_pos + lane; i < cb_end; i += 32) { // the rest of the last chunk: empty
+					p.cbuf[i] = make_uint4(CB_EMPTY, 0, 0, 0);
+				}
+				if (lane == 0 && inline_total) {
+					atomicAdd(p.counters + 4, inline_total);
+				}
+			}
 		}
 	}
 	tc_fence_before();
 	__syncthreads();
 	if (warp == 1) {
 		asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem_base) : "memory");
+	}
+}
+
+// coarse form, after the sweep: the candidates in the buffer through the exact epilogue, with exactly the inputs of the
+// sweep's inline flush.  A warp takes 32 records; the exact sum min(cumP, cumQ) of each takes the whole warp (lane l: bins
+// 32 l .. 32 l + 31 of both full rows), two records at a time so that each warp keeps two row pairs of loads in flight; then
+// lane j scores record j.  Many resident warps per SM hide the row loads that the sweep's epilogue waited for one by one.
+__device__ __forceinline__ u32 row_min_sum(const unsigned short *a, const unsigned short *b, int lane)
+{
+	const uint4 *pa = reinterpret_cast<const uint4 *>(a) + lane * 4, *pb = reinterpret_cast<const uint4 *>(b) + lane * 4;
+	uint4 A[4], B[4];
+#pragma unroll
+	for (int i = 0; i < 4; i++) {
+		A[i] = __ldg(pa + i);
+		B[i] = __ldg(pb + i);
+	}
+	u32 acc = 0;
+#pragma unroll
+	for (int i = 0; i < 4; i++) {
+		acc = dp2a_sum(vmin2(A[i].x, B[i].x), acc);
+		acc = dp2a_sum(vmin2(A[i].y, B[i].y), acc);
+		acc = dp2a_sum(vmin2(A[i].z, B[i].z), acc);
+		acc = dp2a_sum(vmin2(A[i].w, B[i].w), acc);
+	}
+	return acc;
+}
+
+__global__ void __launch_bounds__(256) refine_kernel(const __grid_constant__ DevModel dm, const __grid_constant__ Params p)
+{
+	const bool MIN = (dm.need & NEED_MIN) != 0;
+	const int lane = threadIdx.x & 31;
+	const u64 reserved = p.counters[5];
+	const u64 n = reserved < (u64)p.cb_cap ? reserved : (u64)p.cb_cap;
+	const u64 n_warps = (u64)gridDim.x * (blockDim.x >> 5);
+	for (u64 base = ((u64)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * 32; base < n; base += n_warps * 32) {
+		const u64 e = base + (u64)lane;
+		const uint4 rec = e < n ? p.cbuf[e] : make_uint4(CB_EMPTY, 0, 0, 0);
+		const bool have = rec.x != CB_EMPTY;
+		const u64 cq = p.q0 + rec.x, cd = p.d0 + rec.y;
+		u32 smin = 0;
+#pragma unroll 1
+		for (int j = 0; j < 32; j += 2) {
+			const u32 x0 = __shfl_sync(0xffffffffu, rec.x, j), y0 = __shfl_sync(0xffffffffu, rec.y, j);
+			const u32 x1 = __shfl_sync(0xffffffffu, rec.x, j + 1), y1 = __shfl_sync(0xffffffffu, rec.y, j + 1);
+			u32 a0 = 0, a1 = 0;
+			if (x0 != CB_EMPTY) { // warp-uniform
+				a0 = row_min_sum(p.cumQ + (p.q0 + x0) * NBINS, p.cumD + (p.d0 + y0) * NBINS, lane);
+			}
+			if (x1 != CB_EMPTY) {
+				a1 = row_min_sum(p.cumQ + (p.q0 + x1) * NBINS, p.cumD + (p.d0 + y1) * NBINS, lane);
+			}
+			a0 = __reduce_add_sync(0xffffffffu, a0);
+			a1 = __reduce_add_sync(0xffffffffu, a1);
+			smin = lane == j ? a0 : lane == j + 1 ? a1 : smin;
+		}
+		int close = 0;
+		double score = 0, d0v;
+		if (have) {
+			const Side sd = load_side(p.sbD, cd), sq = load_side(p.sbQ, cq);
+			RedN rd;
+			rd.jeff = rd.js = 0;
+			rd.dot = rec.z;
+			rd.emd = p.csQ[cq] + p.csD[cd] - 2u * smin; // u32, as the full form's
+			rd.smin = MIN ? (sd.sum + sq.sum - (u64)rec.w) >> 1 : 0;
+			const int bad = eval_pair_fast(dm, (u64)NBINS, rd, sd, sq, true, score, d0v, close);
+			if (bad) {
+				atomicOr(p.err, bad & 1 ? 1 : 2);
+			}
+			if (p.identity) {
+				close = score >= p.min_identity;
+			}
+		}
+		const unsigned cm = __ballot_sync(0xffffffffu, close);
+		u64 obase = 0;
+		if (lane == 0 && cm) {
+			obase = atomicAdd(p.counters, (u64)__popc(cm));
+		}
+		obase = __shfl_sync(0xffffffffu, obase, 0);
+		if (close) {
+			const u64 idx = obase + __popc(cm & ((1u << lane) - 1));
+			if (idx < p.max_out) {
+				p.out_q[idx] = cq;
+				p.out_d[idx] = cd;
+				p.out_score[idx] = score;
+			}
+		}
 	}
 }
 
@@ -1495,6 +1646,11 @@ int launch_tile_sweep(mc2_ctx *ctx, const DevModel &dm, int need, const mc2_hset
 	// with t <= 0 among them) and wider rows take the full form.
 	const bool coarse = (need & NEED_EMD) && !raw && p.n_slabs == 1 && dm.scr_ok && q->cum16s && d->cum16s;
 	if (coarse) {
+		if (!ctx->d_cand) {
+			MC2_CUDA(cudaMalloc(&ctx->d_cand, (size_t)ts::CAND_CAP * sizeof(uint4)));
+		}
+		p.cbuf = (uint4 *)ctx->d_cand;
+		p.cb_cap = ts::CAND_CAP;
 		p.cumQ = q->cum16; p.cumD = d->cum16;
 		p.smpQ = q->cum16s; p.smpD = d->cum16s;
 		rc = make_map(&maps[0], d->cum16s, d->n, 64, 2, ts::TD);
@@ -1514,6 +1670,7 @@ int launch_tile_sweep(mc2_ctx *ctx, const DevModel &dm, int need, const mc2_hset
 		if (rc != MC2_OK) return rc;
 	}
 	const int grid = ctx->sm_count;
+	// one profiling interval for the sweep and, in the coarse form, the refinement of its candidates
 	prof_begin(ctx, 3);
 	rc = MC2_OK;
 	switch (need & 7) {
@@ -1533,6 +1690,15 @@ int launch_tile_sweep(mc2_ctx *ctx, const DevModel &dm, int need, const mc2_hset
 	default:
 		set_error("tile sweep: the model needs no reduction");
 		rc = MC2_ERR_UNSUPPORTED;
+	}
+	if (rc == MC2_OK && coarse) {
+		ctx->launches++;
+		MC2_CUDA(cudaGetLastError());
+		static int refine_blocks = 0; // resident CTAs per SM (the same kernel and block size on every device)
+		if (!refine_blocks) {
+			MC2_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&refine_blocks, ts::refine_kernel, 256, 0));
+		}
+		ts::refine_kernel<<<ctx->sm_count * refine_blocks, 256, 0, ctx->stream>>>(dm, p);
 	}
 	prof_end(ctx);
 	if (rc != MC2_OK) return rc;
