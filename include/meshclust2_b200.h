@@ -446,6 +446,40 @@ int mc2_identity_topk_both_strands(mc2_ctx *ctx, const mc2_model *model, double 
 				   double *out_identity, int8_t *out_strand, uint32_t *out_count, uint64_t *out_n_hits,
 				   uint64_t *n_scored);
 
+/* Identity clustering: single-linkage clusters (connected components) of the identity graph over rows [begin, end) of set.
+ * Vertices: the rows [begin, end).  Edges: exactly the pairs (r, c), r < c, that mc2_identity_pairs(set, [q_begin, q_end), set,
+ * [begin, end), upper_only = 1, cutoff) returns (same length window, feature order compute(database c, query r), same decision
+ * on the same bits); with both_strands != 0 exactly those mc2_identity_pairs_both_strands returns (max(id+, id-) >= t).
+ * begin <= q_begin <= q_end <= end: a query sub-range covers part of the triangle (q_begin == q_end: no edge).
+ * out_label[i - begin] = the smallest row of row i's component, as an absolute row number (a row without an edge is its own
+ * label); *n_components = the number of distinct labels.  The label is canonical: it does not depend on block sizes, on how
+ * the query rows are split over calls (join the parts with mc2_components_merge) or GPUs.  *n_scored (may be NULL) is the
+ * forward in-window pair count, equal to mc2_identity_pairs' for the same ranges.
+ * MC2_ERR_ARG: a classifier model, a NaN min_identity, a NULL set / out_label / n_components, [q_begin, q_end) not inside
+ * [begin, end), end > the set's rows, end - begin >= 2^32, and the (query row, 32-column block) and cutoff checks of
+ * mc2_identity_pairs.  MC2_ERR_FEATURE as mc2_identity_pairs returns it.
+ * How: the unchanged identity sweep runs over blocks of query rows (the first block is the whole range) into a scratch of
+ * max(end - begin, 2^24) pairs per strand (with both_strands and min_identity > 0 the block's rows are swept again on the
+ * reverse-complement set, built on first use and kept as in mc2_identity_pairs_both_strands); a block whose survivors
+ * overflow it is swept again in smaller blocks.  Each block's survivors are joined on the device into a union-find over the
+ * rows (components.cu) as soon as the block is swept, and dropped; one flatten and one copy to the host at the end.  Extra
+ * device memory: 24 bytes per scratch pair per strand, plus 12 bytes per row; it does not grow with the number of edges.
+ * min_identity <= 0 is served through the same sweeps (every in-window pair is an edge).
+ * mc2_debug_last_sweep afterwards: n_exact summed over every sweep of both strands, coarse = 1 iff every one took the coarse
+ * form (0 when there was no sweep). */
+int mc2_identity_components(mc2_ctx *ctx, const mc2_model *model, double min_identity, int32_t both_strands, const mc2_hset *set,
+			    uint64_t q_begin, uint64_t q_end, uint64_t begin, uint64_t end, double cutoff, uint64_t *out_label,
+			    uint64_t *n_components, uint64_t *n_scored);
+
+/* The union of n_parts partitions of the rows [begin, end): labels holds n_parts row-major arrays of end - begin labels in
+ * [begin, end) each (for example mc2_identity_components over disjoint query sub-ranges, or from different GPUs).  Joining
+ * the edges {i, labels_p[i]} of every part gives exactly the components of the union of the parts' edge sets; out_label and
+ * *n_components as in mc2_identity_components (the smallest row of each component).  The labels are checked on the host
+ * before the upload.  Extra device memory: 8 bytes per label plus 12 bytes per row.
+ * MC2_ERR_ARG: n_parts == 0, a label outside [begin, end), end < begin, end - begin >= 2^32, a NULL pointer. */
+int mc2_components_merge(mc2_ctx *ctx, uint64_t begin, uint64_t end, uint32_t n_parts, const uint64_t *labels,
+			 uint64_t *out_label, uint64_t *n_components);
+
 /* Measured issue rate (warp-instructions per second, whole GPU) of the tile sweep's inner instruction pair -- VIMNMX.U16x2 on
  * the ALU pipe feeding IDP.2A on the FMA pipe, register operands only, 32 resident warps per SM: the denominator of
  * bench.py's roofline for the CUDA-core EMD term (SURVEY.md section 8d: "achieved ... vs a measured ALU peak"). */
@@ -461,7 +495,7 @@ int mc2_debug_tile_reductions(mc2_ctx *ctx, const mc2_hset *set_q, uint64_t q_be
 			      uint64_t d_begin, uint64_t d_end, int32_t need, uint32_t *out_dot, uint32_t *out_emd, uint32_t *out_sad);
 
 /* Diagnostic (tests, benchmarks): of the last mc2_all_pairs / mc2_identity_pairs call on this context (for
- * mc2_identity_pairs_both_strands and the top-K searches see there), *n_exact = the pairs the tile sweep sent through the exact fp64 epilogue (those its fp32 screen could not reject; 0 for the row-streaming
+ * mc2_identity_pairs_both_strands, the top-K searches and mc2_identity_components see there), *n_exact = the pairs the tile sweep sent through the exact fp64 epilogue (those its fp32 screen could not reject; 0 for the row-streaming
  * kernels) and *coarse = 1 if it took the coarse form (the screen on 64 sampled cumulative bins), else 0.  *n_inline (may
  * be NULL) = how many of the n_exact pairs the coarse form refined inside the sweep because its candidate buffer (2^23
  * records) was full; the others were refined by the kernel that follows the sweep. */

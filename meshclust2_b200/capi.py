@@ -38,7 +38,7 @@ SYMBOLS = [
     "mc2_seqs_total_bases", "mc2_count_kmers", "mc2_count_kmers_into", "mc2_count_kmers_auto", "mc2_hset_largest_count", "mc2_hset_alloc", "mc2_count_kmers_into_rows", "mc2_hset_refresh", "mc2_width_for_count", "mc2_kmer_table_increment", "mc2_hset_from_host", "mc2_hset_from_device", "mc2_hset_update_from_device", "mc2_hset_device_sideband", "mc2_hset_free",
     "mc2_hset_count", "mc2_hset_k", "mc2_hset_elem_bytes", "mc2_hset_device_bins", "mc2_hset_download", "mc2_hset_copy_to_device",
     "mc2_hset_set_sideband", "mc2_hset_set_row", "mc2_hset_assign_rows", "mc2_hset_reverse_complement", "mc2_model_create", "mc2_model_free", "mc2_model_desc_from_file",
-    "mc2_score_pairs", "mc2_get_close", "mc2_get_close_as", "mc2_filter", "mc2_filter_as", "mc2_merge", "mc2_all_pairs", "mc2_identity_pairs", "mc2_identity_pairs_both_strands", "mc2_identity_topk", "mc2_identity_topk_both_strands", "mc2_debug_tile_reductions", "mc2_debug_last_sweep", "mc2_distance", "mc2_mean_closest", "mc2_closest",
+    "mc2_score_pairs", "mc2_get_close", "mc2_get_close_as", "mc2_filter", "mc2_filter_as", "mc2_merge", "mc2_all_pairs", "mc2_identity_pairs", "mc2_identity_pairs_both_strands", "mc2_identity_topk", "mc2_identity_topk_both_strands", "mc2_identity_components", "mc2_components_merge", "mc2_debug_tile_reductions", "mc2_debug_last_sweep", "mc2_distance", "mc2_mean_closest", "mc2_closest",
     "mc2_update_centers", "mc2_merge_centers",
     "mc2_bench_score_pairs", "mc2_bench_count_kmers", "mc2_bench_issue_rate", "mc2_encode_dna", "mc2_encode_dna_batch",
 ]
@@ -110,6 +110,11 @@ def lib():
                                         C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.mc2_identity_topk_both_strands.argtypes = (L.mc2_identity_topk.argtypes[:15] + [C.c_void_p]
                                                      + L.mc2_identity_topk.argtypes[15:])
+        L.mc2_identity_components.argtypes = [C.c_void_p, C.c_void_p, C.c_double, C.c_int32, C.c_void_p, C.c_uint64,
+                                              C.c_uint64, C.c_uint64, C.c_uint64, C.c_double, C.c_void_p, C.c_void_p,
+                                              C.c_void_p]
+        L.mc2_components_merge.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p,
+                                           C.c_void_p]
         _lib = L
     return _lib
 
@@ -472,6 +477,31 @@ class Context:
                                                     int(upper_only), int(exclude_self), cutoff, _p(od), _p(oid), _p(ostr),
                                                     _p(cnt), _p(hits), C.byref(n_scored)))
         return dict(d=od, identity=oid, strand=ostr, count=cnt, n_hits=hits, n_scored=n_scored.value)
+
+    def identity_components(self, model, hset, min_identity, cutoff, both_strands=False, q_range=None, range=None):
+        """Single-linkage clusters of the identity graph over rows range = (begin, end) (default: the whole set): an edge
+        joins r < c when identity_pairs (upper_only, queries q_range, default the whole range) keeps (r, c), or with
+        both_strands when identity_pairs_both_strands does.  Returns dict(label=uint64[end - begin] (the smallest row of each
+        row's component), n_components, n_scored)."""
+        b0, b1 = range if range else (0, len(hset))
+        q0, q1 = q_range if q_range else (b0, b1)
+        label = np.empty(max(b1 - b0, 0), dtype=np.uint64)
+        n_comp, n_scored = C.c_uint64(), C.c_uint64()
+        _check(lib().mc2_identity_components(self.h, model.h, min_identity, int(bool(both_strands)), hset.h, q0, q1, b0, b1,
+                                             cutoff, _p(label), C.byref(n_comp), C.byref(n_scored)))
+        return dict(label=label, n_components=n_comp.value, n_scored=n_scored.value)
+
+    def components_merge(self, labels_2d, begin=0):
+        """The union of the partitions given by the rows of labels_2d ([parts, n] labels in [begin, begin + n)), as
+        dict(label=uint64[n], n_components)"""
+        labels = np.ascontiguousarray(labels_2d, dtype=np.uint64)
+        if labels.ndim != 2:
+            raise ValueError("labels_2d must be [parts, n]")
+        label = np.empty(labels.shape[1], dtype=np.uint64)
+        n_comp = C.c_uint64()
+        _check(lib().mc2_components_merge(self.h, begin, begin + labels.shape[1], labels.shape[0], _p(labels), _p(label),
+                                          C.byref(n_comp)))
+        return dict(label=label, n_components=n_comp.value)
 
     def issue_rate(self, iters=100000):
         """measured warp-instructions / s of the VIMNMX.U16x2 + IDP.2A pair (roofline denominator of the tile sweep)"""

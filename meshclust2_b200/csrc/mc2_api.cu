@@ -79,6 +79,7 @@ enum { B_IA = 0, B_IB, B_SCORE, B_DIST, B_CLOSE, B_SKIP, B_CACHE, B_RAW, B_MISC,
        B_STR_Q, B_STR_D, B_STR_S, B_STR_F, B_STR_OQ, B_STR_OD, B_STR_OS, B_STR_OSTR, B_STR_CNT,
        B_TOPK_Q, B_TOPK_D, B_TOPK_S, B_TOPK_BID, B_TOPK_BD, B_TOPK_CNT, B_TOPK_OFF, B_TOPK_OD, B_TOPK_OID, B_TOPK_OCNT, B_TOPK_OHITS,
        B_TK2_RQ, B_TK2_RD, B_TK2_RS, B_TK2_X, B_TK2_SSTR, B_TK2_BSTR, B_TK2_OSTR,
+       B_CC_PARENT, B_CC_LABEL,
        B_COUNT };
 
 struct ProfRec {
@@ -2698,6 +2699,135 @@ int mc2_identity_topk_both_strands(mc2_ctx *ctx, const mc2_model *model, double 
 	if (out_n_hits) MC2_CUDA(cudaMemcpyAsync(out_n_hits, ohits, nq * 8, cudaMemcpyDeviceToHost, st));
 	MC2_CUDA(cudaStreamSynchronize(st));
 	return MC2_OK;
+}
+
+/* ---- identity clustering: connected components of the identity graph ------------------------------ */
+// survivors of one block of query rows that each strand's scratch holds: cfg3's upper triangle at t = 0.5 (12.4 M forward
+// hits) fits one block
+static const u64 kComponentsScratch = 1ull << 24;
+
+// parent array and label buffer (labels, then the component count) of a union-find over n rows, parents initialised
+static int components_begin(mc2_ctx *ctx, u64 n, u32 **parent, u64 **label)
+{
+	CtxExtra *x = extra(ctx);
+	int rc = ensure(x->d[B_CC_PARENT], n * 4, false);
+	if (rc == MC2_OK) rc = ensure(x->d[B_CC_LABEL], (n + 1) * 8, false);
+	if (rc != MC2_OK) return rc;
+	*parent = (u32 *)x->d[B_CC_PARENT].p;
+	*label = (u64 *)x->d[B_CC_LABEL].p;
+	return launch_cc_init(ctx, *parent, n);
+}
+
+// flatten, then the labels and the component count to the host
+static int components_end(mc2_ctx *ctx, u32 *parent, u64 *label, u64 n, u64 begin, uint64_t *out_label, uint64_t *n_components)
+{
+	int rc = launch_cc_flatten(ctx, parent, n, begin, label, label + n);
+	if (rc != MC2_OK) return rc;
+	cudaStream_t st = ctx->stream;
+	MC2_CUDA(cudaMemcpyAsync(out_label, label, n * 8, cudaMemcpyDeviceToHost, st));
+	MC2_CUDA(cudaMemcpyAsync(ctx->h_slot, label + n, 8, cudaMemcpyDeviceToHost, st));
+	MC2_CUDA(cudaStreamSynchronize(st));
+	*n_components = ((u64 *)ctx->h_slot)[0];
+	return MC2_OK;
+}
+
+int mc2_identity_components(mc2_ctx *ctx, const mc2_model *model, double min_identity, int32_t both_strands, const mc2_hset *set,
+			    uint64_t q_begin, uint64_t q_end, uint64_t begin, uint64_t end, double cutoff, uint64_t *out_label,
+			    uint64_t *n_components, uint64_t *n_scored)
+{
+	const std::string w("mc2_identity_components");
+	MC2_REQUIRE(ctx && model && set && out_label && n_components, w + ": NULL argument");
+	MC2_REQUIRE(!std::isnan(min_identity), w + ": min_identity is NaN");
+	MC2_REQUIRE(begin <= q_begin && q_begin <= q_end && q_end <= end && end <= set->n, w + ": row range out of bounds");
+	MC2_REQUIRE(end - begin < (1ULL << 32), w + ": the row range must hold fewer than 2^32 rows");
+	MC2_REQUIRE(cutoff > 0, w + ": cutoff must be > 0");
+	MC2_REQUIRE((q_end - q_begin) * ((end - begin + 31) / 32) < (1ULL << 32),
+		    w + ": more than 2^32 (query row, 32-column block) groups in one call; split the query range");
+	MC2_REQUIRE(model->dm.regression != 0, w + ": needs a regression model");
+	MC2_CUDA(cudaSetDevice(ctx->device));
+	*n_components = 0;
+	if (n_scored) *n_scored = 0;
+	CtxExtra *x = extra(ctx);
+	x->last_exact = 0;
+	x->last_coarse = 0;
+	x->last_inline = x->sum_inline = 0;
+	const u64 n = end - begin;
+	if (n == 0) return MC2_OK;
+	u32 *parent;
+	u64 *label;
+	int rc = components_begin(ctx, n, &parent, &label);
+	if (rc != MC2_OK) return rc;
+	if (q_begin < q_end) {
+		const double t = min_identity;
+		const DevModel dm = identity_model(model, t);
+		// an edge on either strand is an edge: no strand merge, no rescoring.  For t <= 0 every in-window pair is already a
+		// forward edge and the reverse sweep is skipped.
+		const bool rev = both_strands && t > 0;
+		const u64 scratch = std::max<u64>(n, kComponentsScratch);
+		const int bufs[] = {B_TOPK_Q, B_TOPK_D, B_TOPK_S, B_TK2_RQ, B_TK2_RD, B_TK2_RS};
+		for (int i = 0; i < (rev ? 6 : 3); i++) {
+			if ((rc = ensure(x->d[bufs[i]], scratch * 8, false)) != MC2_OK) return rc;
+		}
+		u64 *sq = (u64 *)x->d[B_TOPK_Q].p, *sd = (u64 *)x->d[B_TOPK_D].p;
+		double *ss = (double *)x->d[B_TOPK_S].p;
+		u64 *rq = rev ? (u64 *)x->d[B_TK2_RQ].p : nullptr, *rd = rev ? (u64 *)x->d[B_TK2_RD].p : nullptr;
+		double *rs = rev ? (double *)x->d[B_TK2_RS].p : nullptr;
+		const mc2_hset *rcq = nullptr;
+		if (rev) {
+			// the reverse-complement rows keep the query indices, so upper_only and the length window mean the same on
+			// both strands
+			if (!set->rc) {
+				mc2_hset *r = nullptr;
+				if ((rc = reverse_complement_set(ctx, set, &r)) != MC2_OK) return rc;
+				const_cast<mc2_hset *>(set)->rc = r;
+			}
+			rcq = set->rc;
+		}
+		// the parent array is the only state kept between blocks: each block's survivors are joined as soon as it is swept
+		u64 exact = 0;
+		uint64_t ns = 0;
+		int coarse = 1;
+		rc = sweep_row_blocks(ctx, dm, t, set, rcq, q_begin, q_end, set, begin, end, 1, cutoff, scratch, q_end - q_begin, sq, sd,
+				      ss, rq, rd, rs, &exact, &coarse, &ns, [&](u64, u64, u64 nb, u64 nb2) -> int {
+			int r = launch_cc_hook_pairs(ctx, sq, sd, nb, begin, parent);
+			if (r == MC2_OK) r = launch_cc_hook_pairs(ctx, rq, rd, nb2, begin, parent);
+			return r;
+		});
+		if (rc != MC2_OK) return rc;
+		x->last_exact = exact;
+		x->last_inline = x->sum_inline;
+		x->last_coarse = coarse;
+		if (n_scored) *n_scored = ns;
+	}
+	return components_end(ctx, parent, label, n, begin, out_label, n_components);
+}
+
+int mc2_components_merge(mc2_ctx *ctx, uint64_t begin, uint64_t end, uint32_t n_parts, const uint64_t *labels, uint64_t *out_label,
+			 uint64_t *n_components)
+{
+	const std::string w("mc2_components_merge");
+	MC2_REQUIRE(ctx && out_label && n_components, w + ": NULL argument");
+	MC2_REQUIRE(n_parts >= 1, w + ": n_parts must be >= 1");
+	MC2_REQUIRE(begin <= end && end - begin < (1ULL << 32), w + ": the row range must hold fewer than 2^32 rows");
+	const u64 n = end - begin, m = (u64)n_parts * n;
+	MC2_REQUIRE(n == 0 || labels, w + ": NULL argument");
+	MC2_REQUIRE(m <= UINT64_MAX / 8, w + ": n_parts x (end - begin) overflows");
+	for (u64 i = 0; i < m; i++) {
+		MC2_REQUIRE(labels[i] >= begin && labels[i] < end, w + ": a label outside [begin, end)");
+	}
+	MC2_CUDA(cudaSetDevice(ctx->device));
+	*n_components = 0;
+	if (n == 0) return MC2_OK;
+	CtxExtra *x = extra(ctx);
+	int rc = ensure(x->d[B_TOPK_Q], m * 8, false);
+	if (rc != MC2_OK) return rc;
+	u64 *d_labels = (u64 *)x->d[B_TOPK_Q].p;
+	MC2_CUDA(cudaMemcpyAsync(d_labels, labels, m * 8, cudaMemcpyHostToDevice, ctx->stream));
+	u32 *parent;
+	u64 *label;
+	if ((rc = components_begin(ctx, n, &parent, &label)) != MC2_OK) return rc;
+	if ((rc = launch_cc_hook_labels(ctx, d_labels, n_parts, n, begin, parent)) != MC2_OK) return rc;
+	return components_end(ctx, parent, label, n, begin, out_label, n_components);
 }
 
 int mc2_debug_last_sweep(mc2_ctx *ctx, uint64_t *n_exact, int32_t *coarse, uint64_t *n_inline)

@@ -327,6 +327,13 @@ int launch_topk_scatter_strand(mc2_ctx *ctx, const u64 *sq, const u64 *sd, const
 int launch_topk_select_strand(mc2_ctx *ctx, const u64 *off, const double *bid, const u64 *bd, const int8_t *bstr, u64 rows,
 			      u32 k_best, u64 d_begin, u64 *out_d, double *out_id, int8_t *out_str, u32 *out_cnt,
 			      u64 *out_hits);
+// components.cu: union-find over rows [begin, begin + n) in a uint32 parent array relative to begin; init sets parent[i] = i,
+// the hooks join the edges {q[i], d[i]} (absolute rows) or {i mod n, labels[i]} of n_parts stacked label arrays, flatten
+// writes out[i] = begin + the smallest row of i's component and *n_roots = the number of components
+int launch_cc_init(mc2_ctx *ctx, u32 *parent, u64 n);
+int launch_cc_hook_pairs(mc2_ctx *ctx, const u64 *q, const u64 *d, u64 n, u64 begin, u32 *parent);
+int launch_cc_hook_labels(mc2_ctx *ctx, const u64 *labels, u64 n_parts, u64 n, u64 begin, u32 *parent);
+int launch_cc_flatten(mc2_ctx *ctx, u32 *parent, u64 n, u64 begin, u64 *out, u64 *n_roots);
 int launch_merge_batch(mc2_ctx *ctx, const double *d_dist, const uint8_t *d_skipped, const uint8_t *d_close, const u64 *d_off,
 		       u64 n_centers, long long *d_out);
 

@@ -148,7 +148,7 @@ class Comm:
 
 
 def all_pairs_step(engine, comm, torch, n_total, cutoff, upper_only=True, blocks_per_rank=1, max_out=1 << 20, identity=None,
-                   top_k=None):
+                   top_k=None, components=False):
     """One pass of the hot path over a batch: local K1 -> all-gather -> row-block K2 sweep.
 
     identity: None sweeps with the engine's classifier; (regression model, min_identity) makes it an identity search
@@ -161,6 +161,11 @@ def all_pairs_step(engine, comm, torch, n_total, cutoff, upper_only=True, blocks
     it; a both-strand search ranks each pair's better strand (engine.topk_both_strands) and its tables add
     strand [q1-q0, top_k].  A query lives in exactly one block of one rank, so the tables are complete per query and
     nothing but the counters is reduced; n_close is the total hit count.
+    components: with an identity search over the upper triangle, the single-linkage clusters of the identity graph (an edge
+    is a pair the search keeps, on either strand with (model, t, True)) instead of the survivor list.  Each rank labels its
+    blocks (engine.components) and joins them (engine.merge_components); the per-rank label arrays are all-gathered and
+    joined again, so every rank holds `components` = dict(label [n_total] = the smallest row of each row's component,
+    n_components).  A label is canonical, so the result does not depend on the number of ranks; n_close is 0.
 
     engine.count()                  K1 over this rank's shard
     engine.export_local()           -> (bins [per, N] tensor, length [per] int64 tensor, mag [per] int64 tensor) padded
@@ -172,8 +177,14 @@ def all_pairs_step(engine, comm, torch, n_total, cutoff, upper_only=True, blocks
     engine.topk(q0, q1, upper_only, cutoff, (model, min_identity), top_k) -> (n_hits, n_scored, table)
     engine.topk_both_strands(q0, q1, upper_only, cutoff, (model, min_identity), top_k) -> (n_hits, n_scored, table)
                                     (optional: an engine without it takes no both-strand top_k)
-    Returns dict(n_scored, n_close, survivors (this rank's), topk (this rank's, [] without top_k), blocks)."""
+    engine.components(q0, q1, cutoff, identity) -> dict(label [n_total], n_components, n_scored)   (optional)
+    engine.merge_components(labels [parts, n_total]) -> dict(label [n_total], n_components)
+    Returns dict(n_scored, n_close, survivors (this rank's), topk (this rank's, [] without top_k), blocks, components (None
+    without components))."""
     both_strands = identity is not None and len(identity) > 2 and bool(identity[2])
+    if components and (identity is None or not upper_only or top_k is not None or not hasattr(engine, "components")):
+        raise ValueError("components needs an identity search over the upper triangle (identity=(regression model, "
+                         "min_identity[, both_strands]), upper_only=True), no top_k, and an engine with components")
     if top_k is not None and (identity is None or (both_strands and not hasattr(engine, "topk_both_strands"))):
         raise ValueError("top_k needs a one-strand identity search: identity=(regression model, min_identity), or an "
                          "engine with topk_both_strands for identity=(regression model, min_identity, True)")
@@ -202,7 +213,12 @@ def all_pairs_step(engine, comm, torch, n_total, cutoff, upper_only=True, blocks
     n_scored = n_close = 0
     surv = Survivors()
     tables = []
+    parts = []
     for q0, q1 in blocks:
+        if components:
+            parts.append(engine.components(q0, q1, cutoff, identity))
+            n_scored += int(parts[-1]["n_scored"])
+            continue
         if top_k is not None:
             if both_strands:
                 ns, sc, table = engine.topk_both_strands(q0, q1, upper_only, cutoff, identity[:2], top_k)
@@ -219,9 +235,21 @@ def all_pairs_step(engine, comm, torch, n_total, cutoff, upper_only=True, blocks
         n_close += ns
         n_scored += sc
         surv.add(pairs)
+    comp = None
+    if components:
+        if not parts:                               # no block on this rank: every row is its own component
+            comp = dict(label=np.arange(n_total, dtype=np.uint64), n_components=n_total)
+        elif len(parts) == 1:
+            comp = parts[0]
+        else:
+            comp = engine.merge_components(np.stack([p["label"] for p in parts]))
+        if comm.dist is not None:
+            local = torch.as_tensor(np.asarray(comp["label"], dtype=np.int64), device=engine.device)
+            comp = engine.merge_components(comm.all_gather_rows(local, torch).cpu().numpy().reshape(comm.world, n_total))
+        comp = dict(label=comp["label"], n_components=comp["n_components"])
     tot_scored, tot_close = comm.all_reduce_sum([n_scored, n_close], torch, engine.device)
     return dict(n_scored=tot_scored, n_close=tot_close, local_scored=n_scored, local_close=n_close, survivors=surv, topk=tables,
-                blocks=blocks)
+                blocks=blocks, components=comp)
 
 
 def candidate_scan(engine, comm, torch, q_global, n_total, cutoff):
@@ -532,6 +560,18 @@ class GpuEngine:
         r = self.ctx.identity_topk_both_strands(model, self.full, self.full, t, top_k, cutoff, q_range=(q0, q1),
                                                 d_range=(0, nd), upper_only=upper_only)
         return int(r["n_hits"].sum()), r["n_scored"], r
+
+    def components(self, q0, q1, cutoff, identity):
+        """single-linkage clusters of the identity graph over the whole set, edges from query rows [q0, q1) of the upper
+        triangle (Context.identity_components) -> dict(label, n_components, n_scored)"""
+        model, t = identity[:2]
+        nd = min(len(self.full), getattr(self, "n_total", None) or len(self.full))   # rows past n_total are shard padding
+        return self.ctx.identity_components(model, self.full, t, cutoff, both_strands=len(identity) > 2 and bool(identity[2]),
+                                            q_range=(q0, q1), range=(0, nd))
+
+    def merge_components(self, labels):
+        """the union of the partitions in the rows of labels (Context.components_merge) -> dict(label, n_components)"""
+        return self.ctx.components_merge(labels, 0)
 
     def sweep(self, q0, q1, upper_only, cutoff, max_out, identity=None):
         """identity: None = the engine's classifier (all_pairs), else (regression model, min_identity) (identity_pairs) or
