@@ -471,6 +471,39 @@ int mc2_identity_components(mc2_ctx *ctx, const mc2_model *model, double min_ide
 			    uint64_t q_begin, uint64_t q_end, uint64_t begin, uint64_t end, double cutoff, uint64_t *out_label,
 			    uint64_t *n_components, uint64_t *n_scored);
 
+/* Identity clustering: greedy representative clusters of the identity graph over rows [begin, end) of set, as CD-HIT and
+ * UCLUST build them (CD-HIT's -g 1, "most similar" assignment).  Single linkage (mc2_identity_components) chains; here no
+ * member is further than min_identity from its representative.
+ * Graph: the vertices are the rows [begin, end); the edges are exactly the pairs (r, c), r < c, that mc2_identity_pairs(set,
+ * [begin, end), set, [begin, end), upper_only = 1, cutoff) returns (same length window, feature order compute(database c,
+ * query r), so the earlier row is the query, same decision on the same bits), or with both_strands != 0 exactly those
+ * mc2_identity_pairs_both_strands returns.  Edge weight w(r, c): the identity that call reports, bit for bit (on both strands
+ * max(id+, id-), with the strand it reports).
+ * Representatives: c = begin .. end - 1 is visited in ascending order, and row c is a representative iff no representative
+ * r < c has an edge (r, c) (the lexicographically first maximal independent set in row order).  ROW ORDER IS THE VISITING
+ * ORDER: for CD-HIT's longest-first order, build the set with its rows in that order.
+ * Assignment: every other row c goes to the representative r < c with an edge (r, c) of the largest w; on a numeric tie
+ * (-0.0 equals +0.0) the smallest r.  Only earlier representatives count, as in CD-HIT.
+ * Outputs, indexed by i - begin: out_rep = the representative as an absolute row (a representative is its own);
+ * out_identity (may be NULL) = w(rep, i), the same bits the flat call reports for that pair, -1.0 for a representative;
+ * out_strand (may be NULL) = 0 or 1 (always 0 without both_strands), -1 for a representative.  *n_clusters = the number of
+ * representatives; *n_scored (may be NULL) = the forward in-window pair count, equal to mc2_identity_pairs' for the same
+ * ranges.  The result does not depend on block sizes.
+ * MC2_ERR_ARG: a classifier model, a NaN min_identity, a NULL set / out_rep / n_clusters, begin > end or end > the set's
+ * rows, end - begin >= 2^32, cutoff <= 0, more than 2^32 (query row, 32-column block) groups.  MC2_ERR_FEATURE as
+ * mc2_identity_pairs returns it.  min_identity <= 0 is served through the same sweeps (every in-window pair is an edge).
+ * How: the unchanged identity sweep runs over blocks of query rows in row order (the first block is the whole range) into
+ * the scratch of mc2_identity_components, max(end - begin, 2^24) pairs per strand; with both_strands the block's pairs are
+ * merged over the strands as in mc2_identity_topk_both_strands.  An edge arrives with the block of its smaller row, so when
+ * a block arrives every earlier row is final.  Each block's edges are bucketed by their larger row; one cooperative launch
+ * decides the block's rows in rounds, with no host round trip (greedy.cu), and one more brings every later row's best
+ * in-edge from a representative up to date.  Extra device memory: 40 bytes per scratch pair on one strand (91 on both),
+ * plus 50 bytes per row; it does not grow with the number of edges.
+ * mc2_debug_last_sweep afterwards: as for mc2_identity_components. */
+int mc2_identity_greedy_clusters(mc2_ctx *ctx, const mc2_model *model, double min_identity, int32_t both_strands,
+				 const mc2_hset *set, uint64_t begin, uint64_t end, double cutoff, uint64_t *out_rep,
+				 double *out_identity, int8_t *out_strand, uint64_t *n_clusters, uint64_t *n_scored);
+
 /* The union of n_parts partitions of the rows [begin, end): labels holds n_parts row-major arrays of end - begin labels in
  * [begin, end) each (for example mc2_identity_components over disjoint query sub-ranges, or from different GPUs).  Joining
  * the edges {i, labels_p[i]} of every part gives exactly the components of the union of the parts' edge sets; out_label and

@@ -38,7 +38,7 @@ SYMBOLS = [
     "mc2_seqs_total_bases", "mc2_count_kmers", "mc2_count_kmers_into", "mc2_count_kmers_auto", "mc2_hset_largest_count", "mc2_hset_alloc", "mc2_count_kmers_into_rows", "mc2_hset_refresh", "mc2_width_for_count", "mc2_kmer_table_increment", "mc2_hset_from_host", "mc2_hset_from_device", "mc2_hset_update_from_device", "mc2_hset_device_sideband", "mc2_hset_free",
     "mc2_hset_count", "mc2_hset_k", "mc2_hset_elem_bytes", "mc2_hset_device_bins", "mc2_hset_download", "mc2_hset_copy_to_device",
     "mc2_hset_set_sideband", "mc2_hset_set_row", "mc2_hset_assign_rows", "mc2_hset_reverse_complement", "mc2_model_create", "mc2_model_free", "mc2_model_desc_from_file",
-    "mc2_score_pairs", "mc2_get_close", "mc2_get_close_as", "mc2_filter", "mc2_filter_as", "mc2_merge", "mc2_all_pairs", "mc2_identity_pairs", "mc2_identity_pairs_both_strands", "mc2_identity_topk", "mc2_identity_topk_both_strands", "mc2_identity_components", "mc2_components_merge", "mc2_debug_tile_reductions", "mc2_debug_last_sweep", "mc2_distance", "mc2_mean_closest", "mc2_closest",
+    "mc2_score_pairs", "mc2_get_close", "mc2_get_close_as", "mc2_filter", "mc2_filter_as", "mc2_merge", "mc2_all_pairs", "mc2_identity_pairs", "mc2_identity_pairs_both_strands", "mc2_identity_topk", "mc2_identity_topk_both_strands", "mc2_identity_components", "mc2_components_merge", "mc2_identity_greedy_clusters", "mc2_debug_tile_reductions", "mc2_debug_last_sweep", "mc2_distance", "mc2_mean_closest", "mc2_closest",
     "mc2_update_centers", "mc2_merge_centers",
     "mc2_bench_score_pairs", "mc2_bench_count_kmers", "mc2_bench_issue_rate", "mc2_encode_dna", "mc2_encode_dna_batch",
 ]
@@ -113,6 +113,9 @@ def lib():
         L.mc2_identity_components.argtypes = [C.c_void_p, C.c_void_p, C.c_double, C.c_int32, C.c_void_p, C.c_uint64,
                                               C.c_uint64, C.c_uint64, C.c_uint64, C.c_double, C.c_void_p, C.c_void_p,
                                               C.c_void_p]
+        L.mc2_identity_greedy_clusters.argtypes = [C.c_void_p, C.c_void_p, C.c_double, C.c_int32, C.c_void_p, C.c_uint64,
+                                                   C.c_uint64, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                   C.c_void_p]
         L.mc2_components_merge.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p,
                                            C.c_void_p]
         _lib = L
@@ -490,6 +493,23 @@ class Context:
         _check(lib().mc2_identity_components(self.h, model.h, min_identity, int(bool(both_strands)), hset.h, q0, q1, b0, b1,
                                              cutoff, _p(label), C.byref(n_comp), C.byref(n_scored)))
         return dict(label=label, n_components=n_comp.value, n_scored=n_scored.value)
+
+    def identity_greedy_clusters(self, model, hset, min_identity, cutoff, both_strands=False, range=None):
+        """Greedy representative clusters (CD-HIT / UCLUST style) of the identity graph over rows range = (begin, end)
+        (default: the whole set), with the edges of identity_components.  Rows are visited in row order, which is the
+        visiting order: for longest-first, build the set in that order.  A row is a representative unless an earlier
+        representative has an edge to it; every other row goes to the earlier representative of its heaviest edge (ties:
+        the smallest row).  Returns dict(rep=uint64[end - begin] (absolute rows; a representative is its own),
+        identity=float64 (-1.0 for a representative), strand=int8 (0 / 1, -1 for a representative), n_clusters, n_scored)."""
+        b0, b1 = range if range else (0, len(hset))
+        m = max(b1 - b0, 0)
+        rep = np.empty(m, dtype=np.uint64)
+        ident = np.empty(m)
+        strand = np.empty(m, dtype=np.int8)
+        n_cl, n_scored = C.c_uint64(), C.c_uint64()
+        _check(lib().mc2_identity_greedy_clusters(self.h, model.h, min_identity, int(bool(both_strands)), hset.h, b0, b1, cutoff,
+                                                  _p(rep), _p(ident), _p(strand), C.byref(n_cl), C.byref(n_scored)))
+        return dict(rep=rep, identity=ident, strand=strand, n_clusters=n_cl.value, n_scored=n_scored.value)
 
     def components_merge(self, labels_2d, begin=0):
         """The union of the partitions given by the rows of labels_2d ([parts, n] labels in [begin, begin + n)), as

@@ -79,7 +79,7 @@ enum { B_IA = 0, B_IB, B_SCORE, B_DIST, B_CLOSE, B_SKIP, B_CACHE, B_RAW, B_MISC,
        B_STR_Q, B_STR_D, B_STR_S, B_STR_F, B_STR_OQ, B_STR_OD, B_STR_OS, B_STR_OSTR, B_STR_CNT,
        B_TOPK_Q, B_TOPK_D, B_TOPK_S, B_TOPK_BID, B_TOPK_BD, B_TOPK_CNT, B_TOPK_OFF, B_TOPK_OD, B_TOPK_OID, B_TOPK_OCNT, B_TOPK_OHITS,
        B_TK2_RQ, B_TK2_RD, B_TK2_RS, B_TK2_X, B_TK2_SSTR, B_TK2_BSTR, B_TK2_OSTR,
-       B_CC_PARENT, B_CC_LABEL,
+       B_CC_PARENT, B_CC_LABEL, B_GR_ROWS, B_GR_OUT,
        B_COUNT };
 
 struct ProfRec {
@@ -2506,6 +2506,45 @@ int mc2_identity_pairs_both_strands(mc2_ctx *ctx, const mc2_model *model, double
 	return MC2_OK;
 }
 
+// One block of both strands' survivors: F = (sq, sd, ss)[0..nb) and R = (rq, rd, rs)[0..nb2) (R empty for t <= 0), sx the
+// other strand's identity of one of them at a time.
+struct StrandBlock {
+	const u64 *sq, *sd;
+	double *ss;
+	int8_t *sstr;
+	u64 nb;
+	const u64 *rq, *rd;
+	const double *rs;
+	u64 nb2;
+	double *sx;
+};
+
+// The strand merge and bucketing of one block on both strands (mc2_identity_topk_both_strands, mc2_identity_greedy_clusters):
+// F keeps max(id+, id-) with its strand (a tie stays forward), R adds the pairs the forward sweep rejected, !(id+ >= t) on
+// the same bits, on strand 1.  A (q, d) pair is then in at most one of the two, with the bits and strand
+// mc2_identity_pairs_both_strands reports.  Both lists go into `rows` buckets (identity bid, row bd, strand bstr) at the
+// exclusive scan off of their counts: keyed by query q - base with bd = d, or with by_d by database row d - base with bd = q.
+static int bucket_both_strands(mc2_ctx *ctx, const DevModel &dm, const mc2_hset *set_q, const mc2_hset *rcq, const mc2_hset *set_d,
+			       double t, const StrandBlock &b, bool by_d, u64 base, u64 rows, int exclude_self, u32 *cnt, u64 *off,
+			       double *bid, u64 *bd, int8_t *bstr)
+{
+	cudaStream_t st = ctx->stream;
+	int r = score_device_lists(ctx, dm, set_d, rcq, b.sd, b.sq, b.nb, b.sx);
+	if (r == MC2_OK) r = launch_strand_pick(ctx, b.ss, b.sx, b.sstr, b.nb);
+	if (r != MC2_OK) return r;
+	MC2_CUDA(cudaMemsetAsync(cnt, 0, rows * 4, st));
+	r = launch_topk_count_strand(ctx, b.sq, b.sd, nullptr, t, b.nb, base, exclude_self, by_d, cnt);
+	if (r == MC2_OK) r = score_device_lists(ctx, dm, set_d, set_q, b.rd, b.rq, b.nb2, b.sx); // id+ of R, after F's pick used sx
+	if (r == MC2_OK) r = launch_topk_count_strand(ctx, b.rq, b.rd, b.sx, t, b.nb2, base, exclude_self, by_d, cnt);
+	if (r == MC2_OK) r = launch_seg_scan(ctx, cnt, rows, off);
+	if (r != MC2_OK) return r;
+	MC2_CUDA(cudaMemsetAsync(cnt, 0, rows * 4, st)); // now the scatter's cursors
+	r = launch_topk_scatter_strand(ctx, b.sq, b.sd, b.ss, b.sstr, nullptr, t, b.nb, base, exclude_self, by_d, off, cnt, bid, bd, bstr);
+	if (r == MC2_OK) r = launch_topk_scatter_strand(ctx, b.rq, b.rd, b.rs, nullptr, b.sx, t, b.nb2, base, exclude_self, by_d, off, cnt,
+							bid, bd, bstr);
+	return r;
+}
+
 /* ---- top-K identity search ---------------------------------------------------------------------- */
 // survivors of one block of query rows that the scratch holds; a query row has at most d_end - d_begin of them
 static const u64 kTopkScratch = 1ull << 22;
@@ -2578,11 +2617,11 @@ int mc2_identity_topk(mc2_ctx *ctx, const mc2_model *model, double min_identity,
 			      nq, sq, sd, ss, nullptr, nullptr, nullptr, &exact, &coarse, &ns, [&](u64 qb, u64 qe, u64 nb, u64) -> int {
 		const u64 rows = qe - qb, r0 = qb - q_begin;
 		MC2_CUDA(cudaMemsetAsync(cnt, 0, rows * 4, st));
-		int r = launch_topk_count(ctx, sq, sd, nb, qb, exclude_self, cnt);
+		int r = launch_topk_count(ctx, sq, sd, nb, qb, exclude_self, false, cnt);
 		if (r == MC2_OK) r = launch_seg_scan(ctx, cnt, rows, off);
 		if (r != MC2_OK) return r;
 		MC2_CUDA(cudaMemsetAsync(cnt, 0, rows * 4, st)); // now the scatter's cursors
-		r = launch_topk_scatter(ctx, sq, sd, ss, nb, qb, exclude_self, off, cnt, bid, bd);
+		r = launch_topk_scatter(ctx, sq, sd, ss, nb, qb, exclude_self, false, off, cnt, bid, bd);
 		if (r == MC2_OK) r = launch_topk_select(ctx, off, bid, bd, rows, k_best, d_begin, od + r0 * K, oid + r0 * K, ocnt + r0, ohits + r0);
 		return r;
 	});
@@ -2668,18 +2707,8 @@ int mc2_identity_topk_both_strands(mc2_ctx *ctx, const mc2_model *model, double 
 			      nq, sq, sd, ss, rq, rd, rs, &exact, &coarse, &ns, [&](u64 qb, u64 qe, u64 nb, u64 nb2) -> int {
 		const u64 rows = qe - qb, r0 = qb - q_begin;
 		int r = reset_err(ctx);
-		if (r == MC2_OK) r = score_device_lists(ctx, dm, set_d, rcq, sd, sq, nb, sx);
-		if (r == MC2_OK) r = launch_strand_pick(ctx, ss, sx, sstr, nb);
-		if (r != MC2_OK) return r;
-		MC2_CUDA(cudaMemsetAsync(cnt, 0, rows * 4, st));
-		r = launch_topk_count_strand(ctx, sq, sd, nullptr, t, nb, qb, exclude_self, cnt);
-		if (r == MC2_OK) r = score_device_lists(ctx, dm, set_d, set_q, rd, rq, nb2, sx); // id+ of R, after F's pick used sx
-		if (r == MC2_OK) r = launch_topk_count_strand(ctx, rq, rd, sx, t, nb2, qb, exclude_self, cnt);
-		if (r == MC2_OK) r = launch_seg_scan(ctx, cnt, rows, off);
-		if (r != MC2_OK) return r;
-		MC2_CUDA(cudaMemsetAsync(cnt, 0, rows * 4, st)); // now the scatter's cursors
-		r = launch_topk_scatter_strand(ctx, sq, sd, ss, sstr, nullptr, t, nb, qb, exclude_self, off, cnt, bid, bd, bstr);
-		if (r == MC2_OK) r = launch_topk_scatter_strand(ctx, rq, rd, rs, nullptr, sx, t, nb2, qb, exclude_self, off, cnt, bid, bd, bstr);
+		if (r == MC2_OK) r = bucket_both_strands(ctx, dm, set_q, rcq, set_d, t, StrandBlock{sq, sd, ss, sstr, nb, rq, rd, rs, nb2, sx},
+							 false, qb, rows, exclude_self, cnt, off, bid, bd, bstr);
 		if (r == MC2_OK) r = launch_topk_select_strand(ctx, off, bid, bd, bstr, rows, k_best, d_begin, od + r0 * K, oid + r0 * K,
 								ostr + r0 * K, ocnt + r0, ohits + r0);
 		if (r == MC2_OK) r = fetch_err(ctx);
@@ -2828,6 +2857,121 @@ int mc2_components_merge(mc2_ctx *ctx, uint64_t begin, uint64_t end, uint32_t n_
 	if ((rc = components_begin(ctx, n, &parent, &label)) != MC2_OK) return rc;
 	if ((rc = launch_cc_hook_labels(ctx, d_labels, n_parts, n, begin, parent)) != MC2_OK) return rc;
 	return components_end(ctx, parent, label, n, begin, out_label, n_components);
+}
+
+/* ---- identity clustering: greedy representatives in row order ------------------------------------ */
+int mc2_identity_greedy_clusters(mc2_ctx *ctx, const mc2_model *model, double min_identity, int32_t both_strands, const mc2_hset *set,
+				 uint64_t begin, uint64_t end, double cutoff, uint64_t *out_rep, double *out_identity, int8_t *out_strand,
+				 uint64_t *n_clusters, uint64_t *n_scored)
+{
+	const std::string w("mc2_identity_greedy_clusters");
+	MC2_REQUIRE(ctx && model && set && out_rep && n_clusters, w + ": NULL argument");
+	MC2_REQUIRE(!std::isnan(min_identity), w + ": min_identity is NaN");
+	MC2_REQUIRE(begin <= end && end <= set->n, w + ": row range out of bounds");
+	MC2_REQUIRE(end - begin < (1ULL << 32), w + ": the row range must hold fewer than 2^32 rows");
+	MC2_REQUIRE(cutoff > 0, w + ": cutoff must be > 0");
+	MC2_REQUIRE((end - begin) * ((end - begin + 31) / 32) < (1ULL << 32),
+		    w + ": more than 2^32 (query row, 32-column block) groups in one call; split the row range");
+	MC2_REQUIRE(model->dm.regression != 0, w + ": needs a regression model");
+	MC2_CUDA(cudaSetDevice(ctx->device));
+	*n_clusters = 0;
+	if (n_scored) *n_scored = 0;
+	CtxExtra *x = extra(ctx);
+	x->last_exact = 0;
+	x->last_coarse = 0;
+	x->last_inline = x->sum_inline = 0;
+	const u64 n = end - begin;
+	if (n == 0) return MC2_OK;
+	const double t = min_identity;
+	const DevModel dm = identity_model(model, t);
+	// Both strands: every forward survivor's id- is scored for the strand merge, so the reverse-complement set is needed for
+	// any t; for t <= 0 every in-window pair is already a forward edge and the reverse sweep is skipped.
+	const bool both = both_strands != 0, rev = both && t > 0;
+	const u64 scratch = std::max<u64>(n, kComponentsScratch), bucket = both ? 2 * scratch : scratch;
+	// per row: the state kept across blocks (identity 8, status 4, cursor 4, rep 4, strand 1 bytes; three round flags after
+	// rep), the outputs (rep 8, identity 8, strand 1; the representative count after the identities), bucket counts and
+	// offsets
+	const int bufs[] = {B_GR_ROWS, B_GR_OUT, B_TOPK_CNT, B_TOPK_OFF, B_TOPK_Q, B_TOPK_D, B_TOPK_S, B_TOPK_BID, B_TOPK_BD,
+			    B_TK2_SSTR, B_TK2_X, B_TK2_BSTR, B_TK2_RQ, B_TK2_RD, B_TK2_RS};
+	const u64 sizes[] = {21 * n + 16, 17 * n + 8, n * 4, (n + 1) * 8, scratch * 8, scratch * 8, scratch * 8, bucket * 8, bucket * 8,
+			     scratch, scratch * 8, bucket, scratch * 8, scratch * 8, scratch * 8};
+	int rc;
+	for (int i = 0; i < (rev ? 15 : both ? 12 : 9); i++) {
+		if ((rc = ensure(x->d[bufs[i]], sizes[i], false)) != MC2_OK) return rc;
+	}
+	char *rows_p = (char *)x->d[B_GR_ROWS].p, *out_p = (char *)x->d[B_GR_OUT].p;
+	GreedyRows g;
+	g.id = (double *)rows_p;
+	g.status = (u32 *)(rows_p + 8 * n);
+	g.cursor = (u32 *)(rows_p + 12 * n);
+	g.rep = (u32 *)(rows_p + 16 * n);
+	u32 *remain = (u32 *)(rows_p + 20 * n);
+	g.str = (int8_t *)(rows_p + 20 * n + 16);
+	u64 *d_rep = (u64 *)out_p, *d_reps = (u64 *)(out_p + 16 * n);
+	double *d_id = (double *)(out_p + 8 * n);
+	int8_t *d_str = (int8_t *)(out_p + 16 * n + 8);
+	u32 *cnt = (u32 *)x->d[B_TOPK_CNT].p;
+	u64 *off = (u64 *)x->d[B_TOPK_OFF].p, *sq = (u64 *)x->d[B_TOPK_Q].p, *sd = (u64 *)x->d[B_TOPK_D].p, *bd = (u64 *)x->d[B_TOPK_BD].p;
+	double *ss = (double *)x->d[B_TOPK_S].p, *bid = (double *)x->d[B_TOPK_BID].p;
+	double *sx = both ? (double *)x->d[B_TK2_X].p : nullptr;
+	int8_t *sstr = both ? (int8_t *)x->d[B_TK2_SSTR].p : nullptr, *bstr = both ? (int8_t *)x->d[B_TK2_BSTR].p : nullptr;
+	u64 *rq = rev ? (u64 *)x->d[B_TK2_RQ].p : nullptr, *rd = rev ? (u64 *)x->d[B_TK2_RD].p : nullptr;
+	double *rs = rev ? (double *)x->d[B_TK2_RS].p : nullptr;
+	cudaStream_t st = ctx->stream;
+	if ((rc = launch_greedy_init(ctx, g, n)) != MC2_OK) return rc;
+	const mc2_hset *rcq = nullptr;
+	if (both) {
+		// the reverse-complement rows keep the query indices, so upper_only and the length window mean the same on both
+		// strands
+		if (!set->rc) {
+			mc2_hset *r = nullptr;
+			if ((rc = reverse_complement_set(ctx, set, &r)) != MC2_OK) return rc;
+			const_cast<mc2_hset *>(set)->rc = r;
+		}
+		rcq = set->rc;
+	}
+	// Blocks arrive in row order and an edge with the block of its smaller row, so when [qb, qe) arrives every row below qb is
+	// final: the block's edges are bucketed by their larger row (qb .. end - 1), the block's rows are decided, and every
+	// later row's best in-edge from a representative is brought up to date.
+	u64 exact = 0;
+	uint64_t ns = 0;
+	int coarse = 1;
+	rc = sweep_row_blocks(ctx, dm, t, set, rev ? rcq : nullptr, begin, end, set, begin, end, 1, cutoff, scratch, n, sq, sd, ss, rq, rd,
+			      rs, &exact, &coarse, &ns, [&](u64 qb, u64 qe, u64 nb, u64 nb2) -> int {
+		const u64 rows = end - qb;
+		int r = MC2_OK;
+		if (both) {
+			r = reset_err(ctx);
+			if (r == MC2_OK) r = bucket_both_strands(ctx, dm, set, rcq, set, t, StrandBlock{sq, sd, ss, sstr, nb, rq, rd, rs, nb2, sx},
+								 true, qb, rows, 0, cnt, off, bid, bd, bstr);
+		} else {
+			MC2_CUDA(cudaMemsetAsync(cnt, 0, rows * 4, st));
+			r = launch_topk_count(ctx, sq, sd, nb, qb, 0, true, cnt);
+			if (r == MC2_OK) r = launch_seg_scan(ctx, cnt, rows, off);
+			if (r != MC2_OK) return r;
+			MC2_CUDA(cudaMemsetAsync(cnt, 0, rows * 4, st)); // now the scatter's cursors
+			r = launch_topk_scatter(ctx, sq, sd, ss, nb, qb, 0, true, off, cnt, bid, bd);
+		}
+		if (r == MC2_OK) r = launch_greedy_resolve(ctx, off, bd, qb, qe - qb, begin, g, remain);
+		if (r == MC2_OK) r = launch_greedy_assign(ctx, off, bid, bd, bstr, qb, rows, begin, g);
+		if (r != MC2_OK || !both) return r;
+		if ((r = fetch_err(ctx)) != MC2_OK) return r;
+		MC2_CUDA(cudaStreamSynchronize(st));
+		return check_err(ctx);
+	});
+	if (rc != MC2_OK) return rc;
+	x->last_exact = exact;
+	x->last_inline = x->sum_inline;
+	x->last_coarse = coarse;
+	if (n_scored) *n_scored = ns;
+	if ((rc = launch_greedy_finish(ctx, g, n, begin, d_rep, d_id, d_str, d_reps)) != MC2_OK) return rc;
+	MC2_CUDA(cudaMemcpyAsync(out_rep, d_rep, n * 8, cudaMemcpyDeviceToHost, st));
+	if (out_identity) MC2_CUDA(cudaMemcpyAsync(out_identity, d_id, n * 8, cudaMemcpyDeviceToHost, st));
+	if (out_strand) MC2_CUDA(cudaMemcpyAsync(out_strand, d_str, n, cudaMemcpyDeviceToHost, st));
+	MC2_CUDA(cudaMemcpyAsync(ctx->h_slot, d_reps, 8, cudaMemcpyDeviceToHost, st));
+	MC2_CUDA(cudaStreamSynchronize(st));
+	*n_clusters = ((u64 *)ctx->h_slot)[0];
+	return MC2_OK;
 }
 
 int mc2_debug_last_sweep(mc2_ctx *ctx, uint64_t *n_exact, int32_t *coarse, uint64_t *n_inline)

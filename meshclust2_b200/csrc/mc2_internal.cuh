@@ -312,17 +312,18 @@ int launch_strand_pick(mc2_ctx *ctx, double *score, const double *rev, int8_t *s
 int launch_strand_append(mc2_ctx *ctx, const u64 *bq, const u64 *bd, const double *bs, const double *fwd, u64 n, double t,
 			 u64 *counter, u64 max_out, u64 *oq, u64 *od, double *os, int8_t *ostr);
 // topk.cu: survivors (sq, sd, ss)[0..n) of query rows [qb, ...) -> per-query counts, buckets at the counts' exclusive scan
-// off, and each query's first k_best (1..1024) entries by (identity desc, d asc) into its output row
-int launch_topk_count(mc2_ctx *ctx, const u64 *sq, const u64 *sd, u64 n, u64 qb, int exclude_self, u32 *cnt);
-int launch_topk_scatter(mc2_ctx *ctx, const u64 *sq, const u64 *sd, const double *ss, u64 n, u64 qb, int exclude_self,
+// off, and each query's first k_best (1..1024) entries by (identity desc, d asc) into its output row.  by_d: the count and
+// scatter bucket by database row d - qb instead, and the bucket holds (identity, q); no self pair is dropped.
+int launch_topk_count(mc2_ctx *ctx, const u64 *sq, const u64 *sd, u64 n, u64 qb, int exclude_self, bool by_d, u32 *cnt);
+int launch_topk_scatter(mc2_ctx *ctx, const u64 *sq, const u64 *sd, const double *ss, u64 n, u64 qb, int exclude_self, bool by_d,
 			const u64 *off, u32 *cur, double *bid, u64 *bd);
 int launch_topk_select(mc2_ctx *ctx, const u64 *off, const double *bid, const u64 *bd, u64 rows, u32 k_best, u64 d_begin,
 		       u64 *out_d, double *out_id, u32 *out_cnt, u64 *out_hits);
 // the same with a strand per entry: a list with fwd != NULL keeps only its entries with !(fwd[i] >= t); sstr NULL = strand 1
 int launch_topk_count_strand(mc2_ctx *ctx, const u64 *sq, const u64 *sd, const double *fwd, double t, u64 n, u64 qb,
-			     int exclude_self, u32 *cnt);
+			     int exclude_self, bool by_d, u32 *cnt);
 int launch_topk_scatter_strand(mc2_ctx *ctx, const u64 *sq, const u64 *sd, const double *ss, const int8_t *sstr,
-			       const double *fwd, double t, u64 n, u64 qb, int exclude_self, const u64 *off, u32 *cur,
+			       const double *fwd, double t, u64 n, u64 qb, int exclude_self, bool by_d, const u64 *off, u32 *cur,
 			       double *bid, u64 *bd, int8_t *bstr);
 int launch_topk_select_strand(mc2_ctx *ctx, const u64 *off, const double *bid, const u64 *bd, const int8_t *bstr, u64 rows,
 			      u32 k_best, u64 d_begin, u64 *out_d, double *out_id, int8_t *out_str, u32 *out_cnt,
@@ -334,6 +335,24 @@ int launch_cc_init(mc2_ctx *ctx, u32 *parent, u64 n);
 int launch_cc_hook_pairs(mc2_ctx *ctx, const u64 *q, const u64 *d, u64 n, u64 begin, u32 *parent);
 int launch_cc_hook_labels(mc2_ctx *ctx, const u64 *labels, u64 n_parts, u64 n, u64 begin, u32 *parent);
 int launch_cc_flatten(mc2_ctx *ctx, u32 *parent, u64 n, u64 begin, u64 *out, u64 *n_roots);
+// greedy.cu: greedy representative clustering over rows [begin, begin + n), state relative to begin.  Per row: status
+// (undecided 0, representative 1, member 2), the bucket cursor of the resolve rounds, and the best in-edge from a
+// representative so far (rep relative to begin, 0xffffffff none; its identity and strand).  A block of query rows [qb, qb +
+// rows) is resolved from the buckets of its edges keyed by database row - qb (off, br: query rows); assign merges each
+// bucket of (qb, qb + rows) (here rows = end - qb) into the best in-edges; finish writes out_rep (absolute), out_id
+// (-1.0 for a representative), out_str (-1) and *n_reps.
+struct GreedyRows {
+	u32 *status, *cursor, *rep;
+	double *id;
+	int8_t *str;
+};
+int launch_greedy_init(mc2_ctx *ctx, const GreedyRows &g, u64 n);
+int launch_greedy_resolve(mc2_ctx *ctx, const u64 *off, const u64 *br, u64 qb, u64 rows, u64 begin, const GreedyRows &g,
+			  u32 *remain);
+int launch_greedy_assign(mc2_ctx *ctx, const u64 *off, const double *bid, const u64 *br, const int8_t *bstr, u64 qb, u64 rows,
+			 u64 begin, const GreedyRows &g);
+int launch_greedy_finish(mc2_ctx *ctx, const GreedyRows &g, u64 n, u64 begin, u64 *out_rep, double *out_id, int8_t *out_str,
+			 u64 *n_reps);
 int launch_merge_batch(mc2_ctx *ctx, const double *d_dist, const uint8_t *d_skipped, const uint8_t *d_close, const u64 *d_off,
 		       u64 n_centers, long long *d_out);
 

@@ -19,6 +19,9 @@
 // identity, and the reverse survivors that the forward sweep rejected (fwd = id+, kept when !(id+ >= t), strand 1).  The
 // strand travels with each entry as payload, in its own shared array; it never takes part in the order.  The one-strand
 // instantiation (STRAND = false) does the work it did before the strand existed.
+//
+// The count and scatter kernels also serve greedy clustering (greedy.cu), which buckets a block's edges by database row
+// (BY_D = true) and keeps the query row in the bucket; the top-K instantiations (BY_D = false) are unchanged.
 #include "mc2_internal.cuh"
 
 namespace mc2 {
@@ -26,8 +29,9 @@ namespace mc2 {
 static constexpr int kTopkThreads = 256;
 static constexpr u32 kTopkMaxK = 1024;
 
-// survivors per block query (self pairs dropped when asked); STRAND with fwd != NULL: only those with !(fwd[i] >= t)
-template <bool STRAND>
+// survivors per bucket (self pairs dropped when asked); STRAND with fwd != NULL: only those with !(fwd[i] >= t).  The bucket
+// is the query row minus qb, or with BY_D (greedy.cu) the database row minus qb.
+template <bool STRAND, bool BY_D>
 __global__ void __launch_bounds__(256) topk_count_kernel(const u64 *__restrict__ sq, const u64 *__restrict__ sd, u64 n, u64 qb,
 							  int exclude_self, const double *__restrict__ fwd, double t, u32 *__restrict__ cnt)
 {
@@ -36,15 +40,18 @@ __global__ void __launch_bounds__(256) topk_count_kernel(const u64 *__restrict__
 		if (STRAND && fwd && fwd[i] >= t) {
 			continue;
 		}
-		if (!(exclude_self && sd[i] == q)) {
+		if (BY_D) {
+			atomicAdd(cnt + (sd[i] - qb), 1u);
+		} else if (!(exclude_self && sd[i] == q)) {
 			atomicAdd(cnt + (q - qb), 1u);
 		}
 	}
 }
 
 // (identity, d) of each kept survivor into its query's bucket [off[q - qb], off[q - qb + 1]); cur (zeroed) is the fill cursor.
-// STRAND: also its strand into bstr, sstr[i] (sstr NULL: 1), with the filter of topk_count_kernel
-template <bool STRAND>
+// BY_D: (identity, q) into the bucket of d (no self pair to drop).  STRAND: also its strand into bstr, sstr[i] (sstr NULL: 1),
+// with the filter of topk_count_kernel
+template <bool STRAND, bool BY_D>
 __global__ void __launch_bounds__(256) topk_scatter_kernel(const u64 *__restrict__ sq, const u64 *__restrict__ sd,
 							    const double *__restrict__ ss, const int8_t *__restrict__ sstr,
 							    const double *__restrict__ fwd, double t, u64 n, u64 qb, int exclude_self,
@@ -56,12 +63,13 @@ __global__ void __launch_bounds__(256) topk_scatter_kernel(const u64 *__restrict
 		if (STRAND && fwd && fwd[i] >= t) {
 			continue;
 		}
-		if (exclude_self && d == q) {
+		if (!BY_D && exclude_self && d == q) {
 			continue;
 		}
-		const u64 pos = off[q - qb] + atomicAdd(cur + (q - qb), 1u);
+		const u64 key = BY_D ? d : q;
+		const u64 pos = off[key - qb] + atomicAdd(cur + (key - qb), 1u);
 		bid[pos] = ss[i];
-		bd[pos] = d;
+		bd[pos] = BY_D ? q : d;
 		if (STRAND) {
 			bstr[pos] = sstr ? sstr[i] : (int8_t)1;
 		}
@@ -258,25 +266,36 @@ static int grid_for(mc2_ctx *ctx, u64 work, u64 per_cta, u64 ctas_per_sm)
 	return (int)(want < cap ? want : cap);
 }
 
-int launch_topk_count(mc2_ctx *ctx, const u64 *sq, const u64 *sd, u64 n, u64 qb, int exclude_self, u32 *cnt)
+int launch_topk_count(mc2_ctx *ctx, const u64 *sq, const u64 *sd, u64 n, u64 qb, int exclude_self, bool by_d, u32 *cnt)
 {
 	if (n == 0) {
 		return MC2_OK;
 	}
-	topk_count_kernel<false><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, n, qb, exclude_self, nullptr, 0.0, cnt);
+	if (by_d) {
+		topk_count_kernel<false, true><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, n, qb, 0, nullptr, 0.0, cnt);
+	} else {
+		topk_count_kernel<false, false><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, n, qb, exclude_self, nullptr,
+												    0.0, cnt);
+	}
 	ctx->launches++;
 	MC2_CUDA(cudaGetLastError());
 	return MC2_OK;
 }
 
-int launch_topk_scatter(mc2_ctx *ctx, const u64 *sq, const u64 *sd, const double *ss, u64 n, u64 qb, int exclude_self,
+int launch_topk_scatter(mc2_ctx *ctx, const u64 *sq, const u64 *sd, const double *ss, u64 n, u64 qb, int exclude_self, bool by_d,
 			const u64 *off, u32 *cur, double *bid, u64 *bd)
 {
 	if (n == 0) {
 		return MC2_OK;
 	}
-	topk_scatter_kernel<false><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, ss, nullptr, nullptr, 0.0, n, qb,
-											 exclude_self, off, cur, bid, bd, nullptr);
+	if (by_d) {
+		topk_scatter_kernel<false, true><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, ss, nullptr, nullptr, 0.0, n,
+												      qb, 0, off, cur, bid, bd, nullptr);
+	} else {
+		topk_scatter_kernel<false, false><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, ss, nullptr, nullptr, 0.0, n,
+												       qb, exclude_self, off, cur, bid, bd,
+												       nullptr);
+	}
 	ctx->launches++;
 	MC2_CUDA(cudaGetLastError());
 	return MC2_OK;
@@ -297,26 +316,36 @@ int launch_topk_select(mc2_ctx *ctx, const u64 *off, const double *bid, const u6
 }
 
 int launch_topk_count_strand(mc2_ctx *ctx, const u64 *sq, const u64 *sd, const double *fwd, double t, u64 n, u64 qb,
-			     int exclude_self, u32 *cnt)
+			     int exclude_self, bool by_d, u32 *cnt)
 {
 	if (n == 0) {
 		return MC2_OK;
 	}
-	topk_count_kernel<true><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, n, qb, exclude_self, fwd, t, cnt);
+	if (by_d) {
+		topk_count_kernel<true, true><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, n, qb, 0, fwd, t, cnt);
+	} else {
+		topk_count_kernel<true, false><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, n, qb, exclude_self, fwd, t,
+												   cnt);
+	}
 	ctx->launches++;
 	MC2_CUDA(cudaGetLastError());
 	return MC2_OK;
 }
 
 int launch_topk_scatter_strand(mc2_ctx *ctx, const u64 *sq, const u64 *sd, const double *ss, const int8_t *sstr,
-			       const double *fwd, double t, u64 n, u64 qb, int exclude_self, const u64 *off, u32 *cur,
+			       const double *fwd, double t, u64 n, u64 qb, int exclude_self, bool by_d, const u64 *off, u32 *cur,
 			       double *bid, u64 *bd, int8_t *bstr)
 {
 	if (n == 0) {
 		return MC2_OK;
 	}
-	topk_scatter_kernel<true><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, ss, sstr, fwd, t, n, qb, exclude_self,
-											off, cur, bid, bd, bstr);
+	if (by_d) {
+		topk_scatter_kernel<true, true><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, ss, sstr, fwd, t, n, qb, 0,
+												     off, cur, bid, bd, bstr);
+	} else {
+		topk_scatter_kernel<true, false><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, ss, sstr, fwd, t, n, qb,
+												      exclude_self, off, cur, bid, bd, bstr);
+	}
 	ctx->launches++;
 	MC2_CUDA(cudaGetLastError());
 	return MC2_OK;
