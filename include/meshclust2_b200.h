@@ -504,6 +504,49 @@ int mc2_identity_greedy_clusters(mc2_ctx *ctx, const mc2_model *model, double mi
 				 const mc2_hset *set, uint64_t begin, uint64_t end, double cutoff, uint64_t *out_rep,
 				 double *out_identity, int8_t *out_strand, uint64_t *n_clusters, uint64_t *n_scored);
 
+/* Staged greedy clustering: mc2_identity_greedy_clusters split into stages that a caller can spread over calls and GPUs.
+ * The result of mc2_greedy_end is bit for bit that of mc2_identity_greedy_clusters with the same model, min_identity,
+ * both_strands, set, [begin, end) and cutoff (out_rep, out_identity, out_strand, *n_clusters; the n_scored of the sweeps of
+ * the blocks added sum to its *n_scored), whatever the block tiling, the split of each block into parts, the order of the
+ * sweeps and the calls made between stages: the result depends only on the edge set and the row order.
+ * The object sweeps query-row blocks [qb, qe) in row order, starting at the next undecided row (begin at first):
+ *   1. mc2_greedy_sweep_part(part p, [q_begin, q_end)) sweeps those query rows against the columns (r, end) into slot p: its
+ *      records are exactly the edges (r, c), r in [q_begin, q_end), that mc2_identity_greedy_clusters takes, with the same
+ *      identity bits and strand.  *n_edges = how many (may exceed the capacity; the slot's contents are then unspecified and
+ *      the caller sweeps a smaller block), *n_scored = the forward in-window pair count.  Returns once the slot is written.
+ *   2. The caller may copy slots between objects (one per GPU, each with n_parts = the number of GPUs): a slot is
+ *      mc2_greedy_part_buffers' *capacity records of 16 bytes {uint32 r - begin, uint32 c - begin, float64 identity} at
+ *      *d_records (device memory) and, with both_strands, *capacity strand bytes at *d_strand (NULL on one strand); only the
+ *      first n_edges of each are read.
+ *   3. mc2_greedy_add_block(qb, qe, part ranges, part edge counts) decides the rows of [qb, qe) from every slot's records.
+ *      The part ranges tile [qb, qe) in part order (empty ranges allowed).  Every record is checked on the device first (r
+ *      in its part's range, c in (r, end)); a bad one gives MC2_ERR_ARG and leaves the object unchanged.  Returns once the
+ *      slots have been read.
+ * mc2_greedy_end writes the outputs once every row up to end has been added.  The set (and its reverse complement) must not
+ * change or be freed while the object lives; the object keeps its own copy of the model.  Calls on other objects and any
+ * other call may run between stages on the same context.
+ * part_capacity: records per slot; 0 = max(end - begin, ceil(2^24 / n_parts)).  One query row has at most end - begin - 1
+ * edges, so a one-row block always fits.
+ * Extra device memory of the object, n = end - begin, E = n_parts x part_capacity: 50 n + 32 E bytes on one strand, 50 n +
+ * 34 E on both, plus 24 n_parts + 44.  A sweep uses the context's scratch: 24 part_capacity bytes on one strand, 56 on
+ * both.  None of it grows with the number of edges.
+ * MC2_ERR_ARG: the checks of mc2_identity_greedy_clusters (at begin); n_parts == 0; part_capacity below end - begin; a part
+ * index >= n_parts; a sweep range outside [next undecided row, end); a block that does not start at the next undecided row
+ * or ends past end; part ranges that do not tile the block; a count above part_capacity; a bad record; mc2_greedy_end before
+ * every row was added; a NULL argument.
+ * mc2_debug_last_sweep after mc2_greedy_sweep_part: as for the flat identity calls. */
+typedef struct mc2_greedy mc2_greedy;
+int mc2_greedy_begin(mc2_ctx *ctx, const mc2_model *model, double min_identity, int32_t both_strands, const mc2_hset *set,
+		     uint64_t begin, uint64_t end, double cutoff, uint32_t n_parts, uint64_t part_capacity, mc2_greedy **out);
+int mc2_greedy_sweep_part(mc2_ctx *ctx, mc2_greedy *g, uint32_t part, uint64_t q_begin, uint64_t q_end, uint64_t *n_edges,
+			  uint64_t *n_scored);
+int mc2_greedy_part_buffers(const mc2_greedy *g, uint32_t part, void **d_records, int8_t **d_strand, uint64_t *capacity);
+int mc2_greedy_add_block(mc2_ctx *ctx, mc2_greedy *g, uint64_t qb, uint64_t qe, const uint64_t *part_q_begin,
+			 const uint64_t *part_q_end, const uint64_t *part_edges);
+int mc2_greedy_end(mc2_ctx *ctx, mc2_greedy *g, uint64_t *out_rep, double *out_identity, int8_t *out_strand,
+		   uint64_t *n_clusters);
+void mc2_greedy_free(mc2_greedy *g);
+
 /* The union of n_parts partitions of the rows [begin, end): labels holds n_parts row-major arrays of end - begin labels in
  * [begin, end) each (for example mc2_identity_components over disjoint query sub-ranges, or from different GPUs).  Joining
  * the edges {i, labels_p[i]} of every part gives exactly the components of the union of the parts' edge sets; out_label and

@@ -38,7 +38,7 @@ SYMBOLS = [
     "mc2_seqs_total_bases", "mc2_count_kmers", "mc2_count_kmers_into", "mc2_count_kmers_auto", "mc2_hset_largest_count", "mc2_hset_alloc", "mc2_count_kmers_into_rows", "mc2_hset_refresh", "mc2_width_for_count", "mc2_kmer_table_increment", "mc2_hset_from_host", "mc2_hset_from_device", "mc2_hset_update_from_device", "mc2_hset_device_sideband", "mc2_hset_free",
     "mc2_hset_count", "mc2_hset_k", "mc2_hset_elem_bytes", "mc2_hset_device_bins", "mc2_hset_download", "mc2_hset_copy_to_device",
     "mc2_hset_set_sideband", "mc2_hset_set_row", "mc2_hset_assign_rows", "mc2_hset_reverse_complement", "mc2_model_create", "mc2_model_free", "mc2_model_desc_from_file",
-    "mc2_score_pairs", "mc2_get_close", "mc2_get_close_as", "mc2_filter", "mc2_filter_as", "mc2_merge", "mc2_all_pairs", "mc2_identity_pairs", "mc2_identity_pairs_both_strands", "mc2_identity_topk", "mc2_identity_topk_both_strands", "mc2_identity_components", "mc2_components_merge", "mc2_identity_greedy_clusters", "mc2_debug_tile_reductions", "mc2_debug_last_sweep", "mc2_distance", "mc2_mean_closest", "mc2_closest",
+    "mc2_score_pairs", "mc2_get_close", "mc2_get_close_as", "mc2_filter", "mc2_filter_as", "mc2_merge", "mc2_all_pairs", "mc2_identity_pairs", "mc2_identity_pairs_both_strands", "mc2_identity_topk", "mc2_identity_topk_both_strands", "mc2_identity_components", "mc2_components_merge", "mc2_identity_greedy_clusters", "mc2_greedy_begin", "mc2_greedy_sweep_part", "mc2_greedy_part_buffers", "mc2_greedy_add_block", "mc2_greedy_end", "mc2_greedy_free", "mc2_debug_tile_reductions", "mc2_debug_last_sweep", "mc2_distance", "mc2_mean_closest", "mc2_closest",
     "mc2_update_centers", "mc2_merge_centers",
     "mc2_bench_score_pairs", "mc2_bench_count_kmers", "mc2_bench_issue_rate", "mc2_encode_dna", "mc2_encode_dna_batch",
 ]
@@ -116,6 +116,14 @@ def lib():
         L.mc2_identity_greedy_clusters.argtypes = [C.c_void_p, C.c_void_p, C.c_double, C.c_int32, C.c_void_p, C.c_uint64,
                                                    C.c_uint64, C.c_double, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                                    C.c_void_p]
+        L.mc2_greedy_begin.argtypes = [C.c_void_p, C.c_void_p, C.c_double, C.c_int32, C.c_void_p, C.c_uint64, C.c_uint64,
+                                       C.c_double, C.c_uint32, C.c_uint64, C.c_void_p]
+        L.mc2_greedy_sweep_part.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p]
+        L.mc2_greedy_part_buffers.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.mc2_greedy_add_block.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.mc2_greedy_end.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.mc2_greedy_free.argtypes = [C.c_void_p]
+        L.mc2_greedy_free.restype = None
         L.mc2_components_merge.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p,
                                            C.c_void_p]
         _lib = L
@@ -511,6 +519,17 @@ class Context:
                                                   _p(rep), _p(ident), _p(strand), C.byref(n_cl), C.byref(n_scored)))
         return dict(rep=rep, identity=ident, strand=strand, n_clusters=n_cl.value, n_scored=n_scored.value)
 
+    def greedy_begin(self, model, hset, min_identity, cutoff, both_strands=False, range=None, n_parts=1, part_capacity=0):
+        """A staged identity_greedy_clusters over rows range = (begin, end) (default: the whole set), as a GreedyClustering:
+        query-row blocks are swept part by part into n_parts slots of part_capacity edges (0: the library's default),
+        the slots may be exchanged between GPUs, and each block is added in row order.  The result equals
+        identity_greedy_clusters' whatever the blocks and parts.  hset must stay alive and unchanged meanwhile."""
+        b0, b1 = range if range else (0, len(hset))
+        h = C.c_void_p()
+        _check(lib().mc2_greedy_begin(self.h, model.h, min_identity, int(bool(both_strands)), hset.h, b0, b1, cutoff, n_parts,
+                                      part_capacity, C.byref(h)))
+        return GreedyClustering(self, h, b0, b1, n_parts, hset)
+
     def components_merge(self, labels_2d, begin=0):
         """The union of the partitions given by the rows of labels_2d ([parts, n] labels in [begin, begin + n)), as
         dict(label=uint64[n], n_components)"""
@@ -602,6 +621,64 @@ class Context:
         ms = C.c_float()
         _check(lib().mc2_bench_count_kmers(self.h, seqs.h, k, elem_bytes, iters, int(flush_l2), C.byref(ms)))
         return ms.value
+
+
+class GreedyClustering:
+    """A staged greedy clustering (Context.greedy_begin; mc2_greedy_* in include/meshclust2_b200.h)."""
+
+    def __init__(self, ctx, h, begin, end, n_parts, hset):
+        self.ctx, self.h, self.range, self.n_parts = ctx, h, (begin, end), n_parts
+        self._hset = hset           # the set must outlive the object
+
+    def sweep_part(self, part, q0, q1):
+        """sweep query rows [q0, q1) into slot `part` -> (n_edges, n_scored); n_edges > capacity: the slot overflowed"""
+        ne, ns = C.c_uint64(), C.c_uint64()
+        _check(lib().mc2_greedy_sweep_part(self.ctx.h, self.h, part, q0, q1, C.byref(ne), C.byref(ns)))
+        return ne.value, ns.value
+
+    def part_arrays(self, part):
+        """dict(records, strand, capacity): device pointers of slot `part` as __cuda_array_interface__ objects
+        (records: uint8 [capacity, 16] of {uint32 r - begin, uint32 c - begin, float64 identity}; strand: int8 [capacity],
+        None on one strand), which torch.as_tensor wraps without a copy"""
+        rec, st, cap = C.c_void_p(), C.c_void_p(), C.c_uint64()
+        _check(lib().mc2_greedy_part_buffers(self.h, part, C.byref(rec), C.byref(st), C.byref(cap)))
+        n = cap.value
+
+        def dev(ptr, shape, typestr):
+            return type("DevArray", (), {"__cuda_array_interface__": {"shape": shape, "typestr": typestr,
+                                                                       "data": (int(ptr), False), "version": 2}})()
+        return dict(records=dev(rec.value, (n, 16), "|u1"), strand=dev(st.value, (n,), "|i1") if st.value else None,
+                    capacity=n)
+
+    def add_block(self, qb, qe, shares, counts):
+        """decide rows [qb, qe) from the slots: shares = [(q0, q1)] per part tiling [qb, qe), counts = edges per part"""
+        q0 = np.ascontiguousarray([a for a, _ in shares], dtype=np.uint64)
+        q1 = np.ascontiguousarray([b for _, b in shares], dtype=np.uint64)
+        cnt = np.ascontiguousarray(counts, dtype=np.uint64)
+        if len(q0) != self.n_parts or len(q1) != self.n_parts or len(cnt) != self.n_parts:
+            raise ValueError("add_block needs one share and one count per part")
+        _check(lib().mc2_greedy_add_block(self.ctx.h, self.h, qb, qe, _p(q0), _p(q1), _p(cnt)))
+
+    def end(self):
+        """dict(rep, identity, strand, n_clusters) as Context.identity_greedy_clusters returns them"""
+        m = self.range[1] - self.range[0]
+        rep = np.empty(m, dtype=np.uint64)
+        ident = np.empty(m)
+        strand = np.empty(m, dtype=np.int8)
+        n_cl = C.c_uint64()
+        _check(lib().mc2_greedy_end(self.ctx.h, self.h, _p(rep), _p(ident), _p(strand), C.byref(n_cl)))
+        return dict(rep=rep, identity=ident, strand=strand, n_clusters=n_cl.value)
+
+    def free(self):
+        if self.h:
+            lib().mc2_greedy_free(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.free()
+        except Exception:
+            pass
 
 
 def host_register(arr):

@@ -189,6 +189,15 @@ __global__ void __launch_bounds__(kGrThreads) greedy_finish_kernel(GreedyRows g,
 	}
 }
 
+// the part slot records of a staged clustering (mc2_greedy_sweep_part): 16 bytes per edge instead of the sweep's 24
+__global__ void __launch_bounds__(kGrThreads) greedy_pack_kernel(const u64 *__restrict__ sq, const u64 *__restrict__ sd,
+								  const double *__restrict__ ss, u64 n, u64 begin, GreedyEdge *__restrict__ out)
+{
+	for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (u64)gridDim.x * blockDim.x) {
+		out[i] = GreedyEdge{(u32)(sq[i] - begin), (u32)(sd[i] - begin), ss[i]};
+	}
+}
+
 static int gr_grid(mc2_ctx *ctx, u64 work)
 {
 	const u64 want = (work + kGrThreads - 1) / kGrThreads, cap = (u64)ctx->sm_count * 8;
@@ -246,6 +255,17 @@ int launch_greedy_finish(mc2_ctx *ctx, const GreedyRows &g, u64 n, u64 begin, u6
 	}
 	greedy_finish_kernel<<<gr_grid(ctx, n), kGrThreads, 0, ctx->stream>>>(g, n, begin, out_rep, out_id, out_str,
 									     (unsigned long long *)n_reps);
+	ctx->launches++;
+	MC2_CUDA(cudaGetLastError());
+	return MC2_OK;
+}
+
+int launch_greedy_pack(mc2_ctx *ctx, const u64 *sq, const u64 *sd, const double *ss, u64 n, u64 begin, GreedyEdge *out)
+{
+	if (n == 0) {
+		return MC2_OK;
+	}
+	greedy_pack_kernel<<<gr_grid(ctx, n), kGrThreads, 0, ctx->stream>>>(sq, sd, ss, n, begin, out);
 	ctx->launches++;
 	MC2_CUDA(cudaGetLastError());
 	return MC2_OK;

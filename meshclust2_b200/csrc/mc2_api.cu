@@ -2402,40 +2402,22 @@ static int sweep_row_blocks(mc2_ctx *ctx, const DevModel &dm, double t, const mc
 // survivors of one reverse-strand block that the scratch holds; a query row has at most d_end - d_begin of them
 static const u64 kStrandScratch = 1ull << 20;
 
-int mc2_identity_pairs_both_strands(mc2_ctx *ctx, const mc2_model *model, double min_identity, const mc2_hset *set_q,
-				    uint64_t q_begin, uint64_t q_end, const mc2_hset *set_d, uint64_t d_begin, uint64_t d_end,
-				    int32_t upper_only, double cutoff, uint64_t max_out, uint64_t *out_q, uint64_t *out_d,
-				    double *out_identity, int8_t *out_strand, uint64_t *n_out, uint64_t *n_scored)
+// The device stages of mc2_identity_pairs_both_strands: its first max_out pairs (q, d, identity, strand) into (oq, od, os,
+// ostr), *total = all of them; the query set's reverse complement is made and kept when missing.  The reverse strand is
+// swept in blocks whose survivors fit `scratch` pairs (>= d_end - d_begin).  Sets the sweep diagnostics.
+static int sweep_both_strands(mc2_ctx *ctx, const DevModel &dm, double t, const mc2_hset *set_q, u64 q_begin, u64 q_end,
+			      const mc2_hset *set_d, u64 d_begin, u64 d_end, int32_t upper_only, double cutoff, u64 max_out, u64 *oq,
+			      u64 *od, double *os, int8_t *ostr, u64 scratch, u64 *total, uint64_t *n_scored)
 {
-	const std::string w("mc2_identity_pairs_both_strands");
-	MC2_REQUIRE(ctx && model && set_q && set_d && n_out, w + ": NULL argument");
-	MC2_REQUIRE(!std::isnan(min_identity), w + ": min_identity is NaN");
-	MC2_REQUIRE(q_begin <= q_end && q_end <= set_q->n && d_begin <= d_end && d_end <= set_d->n, w + ": row range out of bounds");
-	MC2_REQUIRE(set_q->k == set_d->k && set_q->eb == set_d->eb, w + ": the two sets differ in k or histogram width");
-	MC2_REQUIRE(cutoff > 0, w + ": cutoff must be > 0");
-	MC2_REQUIRE((q_end - q_begin) * ((d_end - d_begin + 31) / 32) < (1ULL << 32),
-		    w + ": more than 2^32 (query row, 32-column block) groups in one call; split the query range");
-	MC2_REQUIRE(model->dm.regression != 0, w + ": needs a regression model");
-	MC2_CUDA(cudaSetDevice(ctx->device));
-	*n_out = 0;
-	if (n_scored) *n_scored = 0;
 	CtxExtra *x = extra(ctx);
-	x->last_exact = 0;
-	x->last_coarse = 0;
-	x->last_inline = x->sum_inline = 0;
-	if (q_begin == q_end || d_begin == d_end) return MC2_OK;
-	const double t = min_identity;
-	const DevModel dm = identity_model(model, t);
-	const u64 cap = max_out ? max_out : 1, scratch = std::max<u64>(d_end - d_begin, kStrandScratch);
 	int rc;
-	const int bufs[] = {B_STR_Q, B_STR_D, B_STR_S, B_STR_F, B_STR_OQ, B_STR_OD, B_STR_OS, B_STR_OSTR, B_STR_CNT};
-	const u64 sizes[] = {scratch * 8, scratch * 8, scratch * 8, scratch * 8, cap * 8, cap * 8, cap * 8, cap, 8};
-	for (int i = 0; i < 9; i++) {
+	const int bufs[] = {B_STR_Q, B_STR_D, B_STR_S, B_STR_F, B_STR_CNT};
+	const u64 sizes[] = {scratch * 8, scratch * 8, scratch * 8, scratch * 8, 8};
+	for (int i = 0; i < 5; i++) {
 		if ((rc = ensure(x->d[bufs[i]], sizes[i], false)) != MC2_OK) return rc;
 	}
-	u64 *sq = (u64 *)x->d[B_STR_Q].p, *sd = (u64 *)x->d[B_STR_D].p, *oq = (u64 *)x->d[B_STR_OQ].p, *od = (u64 *)x->d[B_STR_OD].p;
-	double *ss = (double *)x->d[B_STR_S].p, *sf = (double *)x->d[B_STR_F].p, *os = (double *)x->d[B_STR_OS].p;
-	int8_t *ostr = (int8_t *)x->d[B_STR_OSTR].p;
+	u64 *sq = (u64 *)x->d[B_STR_Q].p, *sd = (u64 *)x->d[B_STR_D].p;
+	double *ss = (double *)x->d[B_STR_S].p, *sf = (double *)x->d[B_STR_F].p;
 	u64 *cnt = (u64 *)x->d[B_STR_CNT].p;
 	cudaStream_t st = ctx->stream;
 
@@ -2490,11 +2472,53 @@ int mc2_identity_pairs_both_strands(mc2_ctx *ctx, const mc2_model *model, double
 	}
 	MC2_CUDA(cudaMemcpyAsync(ctx->h_slot, cnt, 8, cudaMemcpyDeviceToHost, st));
 	MC2_CUDA(cudaStreamSynchronize(st));
-	const u64 total = ((u64 *)ctx->h_slot)[0];
-	*n_out = total;
+	*total = ((u64 *)ctx->h_slot)[0];
 	x->last_exact = exact;
 	x->last_inline = x->sum_inline;
 	x->last_coarse = coarse;
+	return MC2_OK;
+}
+
+int mc2_identity_pairs_both_strands(mc2_ctx *ctx, const mc2_model *model, double min_identity, const mc2_hset *set_q,
+				    uint64_t q_begin, uint64_t q_end, const mc2_hset *set_d, uint64_t d_begin, uint64_t d_end,
+				    int32_t upper_only, double cutoff, uint64_t max_out, uint64_t *out_q, uint64_t *out_d,
+				    double *out_identity, int8_t *out_strand, uint64_t *n_out, uint64_t *n_scored)
+{
+	const std::string w("mc2_identity_pairs_both_strands");
+	MC2_REQUIRE(ctx && model && set_q && set_d && n_out, w + ": NULL argument");
+	MC2_REQUIRE(!std::isnan(min_identity), w + ": min_identity is NaN");
+	MC2_REQUIRE(q_begin <= q_end && q_end <= set_q->n && d_begin <= d_end && d_end <= set_d->n, w + ": row range out of bounds");
+	MC2_REQUIRE(set_q->k == set_d->k && set_q->eb == set_d->eb, w + ": the two sets differ in k or histogram width");
+	MC2_REQUIRE(cutoff > 0, w + ": cutoff must be > 0");
+	MC2_REQUIRE((q_end - q_begin) * ((d_end - d_begin + 31) / 32) < (1ULL << 32),
+		    w + ": more than 2^32 (query row, 32-column block) groups in one call; split the query range");
+	MC2_REQUIRE(model->dm.regression != 0, w + ": needs a regression model");
+	MC2_CUDA(cudaSetDevice(ctx->device));
+	*n_out = 0;
+	if (n_scored) *n_scored = 0;
+	CtxExtra *x = extra(ctx);
+	x->last_exact = 0;
+	x->last_coarse = 0;
+	x->last_inline = x->sum_inline = 0;
+	if (q_begin == q_end || d_begin == d_end) return MC2_OK;
+	const double t = min_identity;
+	const DevModel dm = identity_model(model, t);
+	const u64 cap = max_out ? max_out : 1;
+	int rc;
+	const int bufs[] = {B_STR_OQ, B_STR_OD, B_STR_OS, B_STR_OSTR};
+	const u64 sizes[] = {cap * 8, cap * 8, cap * 8, cap};
+	for (int i = 0; i < 4; i++) {
+		if ((rc = ensure(x->d[bufs[i]], sizes[i], false)) != MC2_OK) return rc;
+	}
+	u64 *oq = (u64 *)x->d[B_STR_OQ].p, *od = (u64 *)x->d[B_STR_OD].p;
+	double *os = (double *)x->d[B_STR_OS].p;
+	int8_t *ostr = (int8_t *)x->d[B_STR_OSTR].p;
+	cudaStream_t st = ctx->stream;
+	u64 total = 0;
+	rc = sweep_both_strands(ctx, dm, t, set_q, q_begin, q_end, set_d, d_begin, d_end, upper_only, cutoff, max_out, oq, od, os, ostr,
+				std::max<u64>(d_end - d_begin, kStrandScratch), &total, n_scored);
+	if (rc != MC2_OK) return rc;
+	*n_out = total;
 	const u64 got = std::min<u64>(total, max_out);
 	if (got) {
 		if (out_q) MC2_CUDA(cudaMemcpyAsync(out_q, oq, got * 8, cudaMemcpyDeviceToHost, st));
@@ -2860,12 +2884,10 @@ int mc2_components_merge(mc2_ctx *ctx, uint64_t begin, uint64_t end, uint32_t n_
 }
 
 /* ---- identity clustering: greedy representatives in row order ------------------------------------ */
-int mc2_identity_greedy_clusters(mc2_ctx *ctx, const mc2_model *model, double min_identity, int32_t both_strands, const mc2_hset *set,
-				 uint64_t begin, uint64_t end, double cutoff, uint64_t *out_rep, double *out_identity, int8_t *out_strand,
-				 uint64_t *n_clusters, uint64_t *n_scored)
+// the argument checks of mc2_identity_greedy_clusters and mc2_greedy_begin (`w` names the caller in error messages)
+static int greedy_check(const std::string &w, const mc2_model *model, double min_identity, const mc2_hset *set, uint64_t begin,
+			uint64_t end, double cutoff)
 {
-	const std::string w("mc2_identity_greedy_clusters");
-	MC2_REQUIRE(ctx && model && set && out_rep && n_clusters, w + ": NULL argument");
 	MC2_REQUIRE(!std::isnan(min_identity), w + ": min_identity is NaN");
 	MC2_REQUIRE(begin <= end && end <= set->n, w + ": row range out of bounds");
 	MC2_REQUIRE(end - begin < (1ULL << 32), w + ": the row range must hold fewer than 2^32 rows");
@@ -2873,6 +2895,73 @@ int mc2_identity_greedy_clusters(mc2_ctx *ctx, const mc2_model *model, double mi
 	MC2_REQUIRE((end - begin) * ((end - begin + 31) / 32) < (1ULL << 32),
 		    w + ": more than 2^32 (query row, 32-column block) groups in one call; split the row range");
 	MC2_REQUIRE(model->dm.regression != 0, w + ": needs a regression model");
+	return MC2_OK;
+}
+
+// The device state of a greedy clustering over rows [begin, end): the rows (GreedyRows and the resolve's three round flags,
+// carved from 21 n + 16 bytes), and the buckets of one block (counts / cursors, offsets, identity, query row, strand).
+struct GreedyBlock {
+	GreedyRows g;
+	u32 *remain, *cnt;
+	u64 *off, *bd;
+	double *bid;
+	int8_t *bstr;
+	u64 begin, end;
+};
+
+// per row: identity 8, status 4, cursor 4, rep 4 bytes, the three round flags after rep, then strand 1
+static void greedy_rows(char *p, u64 n, GreedyBlock *b)
+{
+	b->g.id = (double *)p;
+	b->g.status = (u32 *)(p + 8 * n);
+	b->g.cursor = (u32 *)(p + 12 * n);
+	b->g.rep = (u32 *)(p + 16 * n);
+	b->remain = (u32 *)(p + 20 * n);
+	b->g.str = (int8_t *)(p + 20 * n + 16);
+}
+
+// One block [qb, qe) of query rows, every row below qb final: bucket(rows) puts the block's edges into the buckets of their
+// larger row - qb (rows = end - qb buckets); then one cooperative launch decides the block's rows and one more brings every
+// later row's best in-edge from a representative up to date.
+extern "C++" {
+template <typename F>
+static int greedy_block(mc2_ctx *ctx, const GreedyBlock &b, u64 qb, u64 qe, F &&bucket)
+{
+	int r = bucket(b.end - qb);
+	if (r == MC2_OK) r = launch_greedy_resolve(ctx, b.off, b.bd, qb, qe - qb, b.begin, b.g, b.remain);
+	if (r == MC2_OK) r = launch_greedy_assign(ctx, b.off, b.bid, b.bd, b.bstr, qb, b.end - qb, b.begin, b.g);
+	return r;
+}
+}
+
+// the outputs of a finished clustering over n rows from the rows' state, through d_out (17 n + 8 bytes: rep 8, identity 8,
+// strand 1 per row; the representative count after the identities)
+static int greedy_outputs(mc2_ctx *ctx, const GreedyRows &g, u64 n, u64 begin, char *d_out, uint64_t *out_rep, double *out_identity,
+			  int8_t *out_strand, uint64_t *n_clusters)
+{
+	u64 *d_rep = (u64 *)d_out, *d_reps = (u64 *)(d_out + 16 * n);
+	double *d_id = (double *)(d_out + 8 * n);
+	int8_t *d_str = (int8_t *)(d_out + 16 * n + 8);
+	cudaStream_t st = ctx->stream;
+	int rc = launch_greedy_finish(ctx, g, n, begin, d_rep, d_id, d_str, d_reps);
+	if (rc != MC2_OK) return rc;
+	MC2_CUDA(cudaMemcpyAsync(out_rep, d_rep, n * 8, cudaMemcpyDeviceToHost, st));
+	if (out_identity) MC2_CUDA(cudaMemcpyAsync(out_identity, d_id, n * 8, cudaMemcpyDeviceToHost, st));
+	if (out_strand) MC2_CUDA(cudaMemcpyAsync(out_strand, d_str, n, cudaMemcpyDeviceToHost, st));
+	MC2_CUDA(cudaMemcpyAsync(ctx->h_slot, d_reps, 8, cudaMemcpyDeviceToHost, st));
+	MC2_CUDA(cudaStreamSynchronize(st));
+	*n_clusters = ((u64 *)ctx->h_slot)[0];
+	return MC2_OK;
+}
+
+int mc2_identity_greedy_clusters(mc2_ctx *ctx, const mc2_model *model, double min_identity, int32_t both_strands, const mc2_hset *set,
+				 uint64_t begin, uint64_t end, double cutoff, uint64_t *out_rep, double *out_identity, int8_t *out_strand,
+				 uint64_t *n_clusters, uint64_t *n_scored)
+{
+	const std::string w("mc2_identity_greedy_clusters");
+	MC2_REQUIRE(ctx && model && set && out_rep && n_clusters, w + ": NULL argument");
+	int rc = greedy_check(w, model, min_identity, set, begin, end, cutoff);
+	if (rc != MC2_OK) return rc;
 	MC2_CUDA(cudaSetDevice(ctx->device));
 	*n_clusters = 0;
 	if (n_scored) *n_scored = 0;
@@ -2888,37 +2977,32 @@ int mc2_identity_greedy_clusters(mc2_ctx *ctx, const mc2_model *model, double mi
 	// any t; for t <= 0 every in-window pair is already a forward edge and the reverse sweep is skipped.
 	const bool both = both_strands != 0, rev = both && t > 0;
 	const u64 scratch = std::max<u64>(n, kComponentsScratch), bucket = both ? 2 * scratch : scratch;
-	// per row: the state kept across blocks (identity 8, status 4, cursor 4, rep 4, strand 1 bytes; three round flags after
-	// rep), the outputs (rep 8, identity 8, strand 1; the representative count after the identities), bucket counts and
-	// offsets
+	// per row: the state kept across blocks, the outputs, bucket counts and offsets
 	const int bufs[] = {B_GR_ROWS, B_GR_OUT, B_TOPK_CNT, B_TOPK_OFF, B_TOPK_Q, B_TOPK_D, B_TOPK_S, B_TOPK_BID, B_TOPK_BD,
 			    B_TK2_SSTR, B_TK2_X, B_TK2_BSTR, B_TK2_RQ, B_TK2_RD, B_TK2_RS};
 	const u64 sizes[] = {21 * n + 16, 17 * n + 8, n * 4, (n + 1) * 8, scratch * 8, scratch * 8, scratch * 8, bucket * 8, bucket * 8,
 			     scratch, scratch * 8, bucket, scratch * 8, scratch * 8, scratch * 8};
-	int rc;
 	for (int i = 0; i < (rev ? 15 : both ? 12 : 9); i++) {
 		if ((rc = ensure(x->d[bufs[i]], sizes[i], false)) != MC2_OK) return rc;
 	}
-	char *rows_p = (char *)x->d[B_GR_ROWS].p, *out_p = (char *)x->d[B_GR_OUT].p;
-	GreedyRows g;
-	g.id = (double *)rows_p;
-	g.status = (u32 *)(rows_p + 8 * n);
-	g.cursor = (u32 *)(rows_p + 12 * n);
-	g.rep = (u32 *)(rows_p + 16 * n);
-	u32 *remain = (u32 *)(rows_p + 20 * n);
-	g.str = (int8_t *)(rows_p + 20 * n + 16);
-	u64 *d_rep = (u64 *)out_p, *d_reps = (u64 *)(out_p + 16 * n);
-	double *d_id = (double *)(out_p + 8 * n);
-	int8_t *d_str = (int8_t *)(out_p + 16 * n + 8);
-	u32 *cnt = (u32 *)x->d[B_TOPK_CNT].p;
-	u64 *off = (u64 *)x->d[B_TOPK_OFF].p, *sq = (u64 *)x->d[B_TOPK_Q].p, *sd = (u64 *)x->d[B_TOPK_D].p, *bd = (u64 *)x->d[B_TOPK_BD].p;
-	double *ss = (double *)x->d[B_TOPK_S].p, *bid = (double *)x->d[B_TOPK_BID].p;
+	GreedyBlock gb;
+	greedy_rows((char *)x->d[B_GR_ROWS].p, n, &gb);
+	gb.cnt = (u32 *)x->d[B_TOPK_CNT].p;
+	gb.off = (u64 *)x->d[B_TOPK_OFF].p;
+	gb.bd = (u64 *)x->d[B_TOPK_BD].p;
+	gb.bid = (double *)x->d[B_TOPK_BID].p;
+	gb.bstr = both ? (int8_t *)x->d[B_TK2_BSTR].p : nullptr;
+	gb.begin = begin;
+	gb.end = end;
+	u32 *cnt = gb.cnt;
+	u64 *off = gb.off, *sq = (u64 *)x->d[B_TOPK_Q].p, *sd = (u64 *)x->d[B_TOPK_D].p, *bd = gb.bd;
+	double *ss = (double *)x->d[B_TOPK_S].p, *bid = gb.bid;
 	double *sx = both ? (double *)x->d[B_TK2_X].p : nullptr;
-	int8_t *sstr = both ? (int8_t *)x->d[B_TK2_SSTR].p : nullptr, *bstr = both ? (int8_t *)x->d[B_TK2_BSTR].p : nullptr;
+	int8_t *sstr = both ? (int8_t *)x->d[B_TK2_SSTR].p : nullptr, *bstr = gb.bstr;
 	u64 *rq = rev ? (u64 *)x->d[B_TK2_RQ].p : nullptr, *rd = rev ? (u64 *)x->d[B_TK2_RD].p : nullptr;
 	double *rs = rev ? (double *)x->d[B_TK2_RS].p : nullptr;
 	cudaStream_t st = ctx->stream;
-	if ((rc = launch_greedy_init(ctx, g, n)) != MC2_OK) return rc;
+	if ((rc = launch_greedy_init(ctx, gb.g, n)) != MC2_OK) return rc;
 	const mc2_hset *rcq = nullptr;
 	if (both) {
 		// the reverse-complement rows keep the query indices, so upper_only and the length window mean the same on both
@@ -2931,29 +3015,26 @@ int mc2_identity_greedy_clusters(mc2_ctx *ctx, const mc2_model *model, double mi
 		rcq = set->rc;
 	}
 	// Blocks arrive in row order and an edge with the block of its smaller row, so when [qb, qe) arrives every row below qb is
-	// final: the block's edges are bucketed by their larger row (qb .. end - 1), the block's rows are decided, and every
-	// later row's best in-edge from a representative is brought up to date.
+	// final.
 	u64 exact = 0;
 	uint64_t ns = 0;
 	int coarse = 1;
 	rc = sweep_row_blocks(ctx, dm, t, set, rev ? rcq : nullptr, begin, end, set, begin, end, 1, cutoff, scratch, n, sq, sd, ss, rq, rd,
 			      rs, &exact, &coarse, &ns, [&](u64 qb, u64 qe, u64 nb, u64 nb2) -> int {
-		const u64 rows = end - qb;
-		int r = MC2_OK;
-		if (both) {
-			r = reset_err(ctx);
-			if (r == MC2_OK) r = bucket_both_strands(ctx, dm, set, rcq, set, t, StrandBlock{sq, sd, ss, sstr, nb, rq, rd, rs, nb2, sx},
-								 true, qb, rows, 0, cnt, off, bid, bd, bstr);
-		} else {
+		int r = greedy_block(ctx, gb, qb, qe, [&](u64 rows) -> int {
+			if (both) {
+				int r2 = reset_err(ctx);
+				if (r2 == MC2_OK) r2 = bucket_both_strands(ctx, dm, set, rcq, set, t, StrandBlock{sq, sd, ss, sstr, nb, rq, rd, rs, nb2, sx},
+									   true, qb, rows, 0, cnt, off, bid, bd, bstr);
+				return r2;
+			}
 			MC2_CUDA(cudaMemsetAsync(cnt, 0, rows * 4, st));
-			r = launch_topk_count(ctx, sq, sd, nb, qb, 0, true, cnt);
-			if (r == MC2_OK) r = launch_seg_scan(ctx, cnt, rows, off);
-			if (r != MC2_OK) return r;
+			int r2 = launch_topk_count(ctx, sq, sd, nb, qb, 0, true, cnt);
+			if (r2 == MC2_OK) r2 = launch_seg_scan(ctx, cnt, rows, off);
+			if (r2 != MC2_OK) return r2;
 			MC2_CUDA(cudaMemsetAsync(cnt, 0, rows * 4, st)); // now the scatter's cursors
-			r = launch_topk_scatter(ctx, sq, sd, ss, nb, qb, 0, true, off, cnt, bid, bd);
-		}
-		if (r == MC2_OK) r = launch_greedy_resolve(ctx, off, bd, qb, qe - qb, begin, g, remain);
-		if (r == MC2_OK) r = launch_greedy_assign(ctx, off, bid, bd, bstr, qb, rows, begin, g);
+			return launch_topk_scatter(ctx, sq, sd, ss, nb, qb, 0, true, off, cnt, bid, bd);
+		});
 		if (r != MC2_OK || !both) return r;
 		if ((r = fetch_err(ctx)) != MC2_OK) return r;
 		MC2_CUDA(cudaStreamSynchronize(st));
@@ -2964,14 +3045,221 @@ int mc2_identity_greedy_clusters(mc2_ctx *ctx, const mc2_model *model, double mi
 	x->last_inline = x->sum_inline;
 	x->last_coarse = coarse;
 	if (n_scored) *n_scored = ns;
-	if ((rc = launch_greedy_finish(ctx, g, n, begin, d_rep, d_id, d_str, d_reps)) != MC2_OK) return rc;
-	MC2_CUDA(cudaMemcpyAsync(out_rep, d_rep, n * 8, cudaMemcpyDeviceToHost, st));
-	if (out_identity) MC2_CUDA(cudaMemcpyAsync(out_identity, d_id, n * 8, cudaMemcpyDeviceToHost, st));
-	if (out_strand) MC2_CUDA(cudaMemcpyAsync(out_strand, d_str, n, cudaMemcpyDeviceToHost, st));
-	MC2_CUDA(cudaMemcpyAsync(ctx->h_slot, d_reps, 8, cudaMemcpyDeviceToHost, st));
-	MC2_CUDA(cudaStreamSynchronize(st));
-	*n_clusters = ((u64 *)ctx->h_slot)[0];
+	return greedy_outputs(ctx, gb.g, n, begin, (char *)x->d[B_GR_OUT].p, out_rep, out_identity, out_strand, n_clusters);
+}
+
+} // extern "C"
+
+// A staged greedy clustering (mc2_greedy_begin .. mc2_greedy_end): the rows' state, n_parts part slots of cap records (and
+// strand bytes), buckets for n_parts * cap edges, and the parts' ranges and counts (3 words each, then the bad-record flag),
+// all owned by the object so that other calls may run between its stages.
+struct mc2_greedy {
+	DevModel dm;
+	double t, cutoff;
+	bool both;
+	const mc2_hset *set;
+	u64 begin, end, next, cap;
+	u32 n_parts;
+	Buf rows, out, cnt, off, bid, bd, bstr, rec, str, part;
+	GreedyBlock b;
+};
+
+extern "C" {
+
+// the default part capacity: every part of a whole-range block of cfg3's shape at t = 0.5 (12.4 M forward edges) fits
+static const u64 kGreedyPartEdges = 1ull << 24;
+
+void mc2_greedy_free(mc2_greedy *g)
+{
+	if (!g) return;
+	Buf *bufs[] = {&g->rows, &g->out, &g->cnt, &g->off, &g->bid, &g->bd, &g->bstr, &g->rec, &g->str, &g->part};
+	for (Buf *b : bufs) release(*b);
+	delete g;
+}
+
+int mc2_greedy_begin(mc2_ctx *ctx, const mc2_model *model, double min_identity, int32_t both_strands, const mc2_hset *set,
+		     uint64_t begin, uint64_t end, double cutoff, uint32_t n_parts, uint64_t part_capacity, mc2_greedy **out)
+{
+	const std::string w("mc2_greedy_begin");
+	MC2_REQUIRE(ctx && model && set && out, w + ": NULL argument");
+	*out = nullptr;
+	int rc = greedy_check(w, model, min_identity, set, begin, end, cutoff);
+	if (rc != MC2_OK) return rc;
+	MC2_REQUIRE(n_parts >= 1, w + ": n_parts must be >= 1");
+	const u64 n = end - begin, P = n_parts;
+	const u64 cap = part_capacity ? part_capacity : std::max<u64>(n, (kGreedyPartEdges + P - 1) / P);
+	MC2_REQUIRE(cap >= n, w + ": part_capacity must be >= end - begin (one query row's edges)");
+	MC2_REQUIRE(cap <= UINT64_MAX / 32 / P, w + ": n_parts x part_capacity overflows");
+	MC2_CUDA(cudaSetDevice(ctx->device));
+	mc2_greedy *g = new (std::nothrow) mc2_greedy();
+	MC2_REQUIRE(g, w + ": out of host memory");
+	g->dm = identity_model(model, min_identity);
+	g->t = min_identity;
+	g->cutoff = cutoff;
+	g->both = both_strands != 0;
+	g->set = set;
+	g->begin = g->next = begin;
+	g->end = end;
+	g->cap = cap;
+	g->n_parts = n_parts;
+	const u64 edges = P * cap;
+	Buf *bufs[] = {&g->rows, &g->out, &g->cnt, &g->off, &g->bid, &g->bd, &g->rec, &g->part, &g->bstr, &g->str};
+	const u64 sizes[] = {21 * n + 16, 17 * n + 8, n * 4 + 4, (n + 1) * 8, edges * 8, edges * 8, edges * 16, P * 24 + 8, edges, edges};
+	for (int i = 0; i < (g->both ? 10 : 8) && rc == MC2_OK; i++) {
+		// sized once, exactly: the object never grows
+		const cudaError_t e = cudaMalloc(&bufs[i]->p, sizes[i]);
+		if (e != cudaSuccess) {
+			bufs[i]->p = nullptr;
+			rc = cuda_fail(e, "mc2_greedy_begin: device memory", __FILE__, __LINE__);
+		}
+		bufs[i]->cap = sizes[i];
+	}
+	if (rc == MC2_OK) {
+		greedy_rows((char *)g->rows.p, n, &g->b);
+		g->b.cnt = (u32 *)g->cnt.p;
+		g->b.off = (u64 *)g->off.p;
+		g->b.bd = (u64 *)g->bd.p;
+		g->b.bid = (double *)g->bid.p;
+		g->b.bstr = g->both ? (int8_t *)g->bstr.p : nullptr;
+		g->b.begin = begin;
+		g->b.end = end;
+		rc = launch_greedy_init(ctx, g->b.g, n);
+	}
+	if (rc == MC2_OK) {
+		const cudaError_t e = cudaStreamSynchronize(ctx->stream);
+		if (e != cudaSuccess) rc = cuda_fail(e, "mc2_greedy_begin", __FILE__, __LINE__);
+	}
+	if (rc != MC2_OK) {
+		mc2_greedy_free(g);
+		return rc;
+	}
+	*out = g;
 	return MC2_OK;
+}
+
+int mc2_greedy_part_buffers(const mc2_greedy *g, uint32_t part, void **d_records, int8_t **d_strand, uint64_t *capacity)
+{
+	const std::string w("mc2_greedy_part_buffers");
+	MC2_REQUIRE(g && d_records && capacity, w + ": NULL argument");
+	MC2_REQUIRE(part < g->n_parts, w + ": part must be < n_parts");
+	*d_records = (char *)g->rec.p + (u64)part * g->cap * 16;
+	if (d_strand) *d_strand = g->both ? (int8_t *)g->str.p + (u64)part * g->cap : nullptr;
+	*capacity = g->cap;
+	return MC2_OK;
+}
+
+int mc2_greedy_sweep_part(mc2_ctx *ctx, mc2_greedy *g, uint32_t part, uint64_t q_begin, uint64_t q_end, uint64_t *n_edges,
+			  uint64_t *n_scored)
+{
+	const std::string w("mc2_greedy_sweep_part");
+	MC2_REQUIRE(ctx && g && n_edges, w + ": NULL argument");
+	MC2_REQUIRE(part < g->n_parts, w + ": part must be < n_parts");
+	MC2_REQUIRE(g->next <= q_begin && q_begin <= q_end && q_end <= g->end,
+		    w + ": the query rows must lie in [the next undecided row, end)");
+	MC2_CUDA(cudaSetDevice(ctx->device));
+	*n_edges = 0;
+	if (n_scored) *n_scored = 0;
+	CtxExtra *x = extra(ctx);
+	x->last_exact = 0;
+	x->last_coarse = 0;
+	x->last_inline = x->sum_inline = 0;
+	cudaStream_t st = ctx->stream;
+	if (q_begin == q_end) {
+		// a slot is free once the stream is idle: the caller may write the next block's records into it
+		MC2_CUDA(cudaStreamSynchronize(st));
+		return MC2_OK;
+	}
+	const u64 cap = g->cap;
+	int rc;
+	const int bufs[] = {B_TOPK_Q, B_TOPK_D, B_TOPK_S};
+	for (int i = 0; i < 3; i++) {
+		if ((rc = ensure(x->d[bufs[i]], cap * 8, false)) != MC2_OK) return rc;
+	}
+	u64 *sq = (u64 *)x->d[B_TOPK_Q].p, *sd = (u64 *)x->d[B_TOPK_D].p;
+	double *ss = (double *)x->d[B_TOPK_S].p;
+	u64 total = 0;
+	if (g->both) {
+		// the reverse survivors of a part fit a scratch of a slot's size, as the forward ones fit the slot: the reverse sweep
+		// then takes one or two blocks, as in the single call, rather than one per 2^20 survivors
+		rc = sweep_both_strands(ctx, g->dm, g->t, g->set, q_begin, q_end, g->set, g->begin, g->end, 1, g->cutoff, cap, sq, sd, ss,
+					(int8_t *)g->str.p + (u64)part * cap, cap, &total, n_scored);
+	} else {
+		rc = run_sweep(ctx, g->dm, 1, g->t, g->set, q_begin, q_end, g->set, g->begin, g->end, 1, g->cutoff, cap, sq, sd, ss, &total,
+			       n_scored);
+		if (rc == MC2_OK) rc = check_err(ctx);
+	}
+	if (rc != MC2_OK) return rc;
+	*n_edges = total;
+	if (total <= cap) {
+		if ((rc = launch_greedy_pack(ctx, sq, sd, ss, total, g->begin, (GreedyEdge *)g->rec.p + (u64)part * cap)) != MC2_OK) return rc;
+	}
+	MC2_CUDA(cudaStreamSynchronize(st));
+	return MC2_OK;
+}
+
+int mc2_greedy_add_block(mc2_ctx *ctx, mc2_greedy *g, uint64_t qb, uint64_t qe, const uint64_t *part_q_begin,
+			 const uint64_t *part_q_end, const uint64_t *part_edges)
+{
+	const std::string w("mc2_greedy_add_block");
+	MC2_REQUIRE(ctx && g && part_q_begin && part_q_end && part_edges, w + ": NULL argument");
+	MC2_REQUIRE(qb == g->next, w + ": the block must start at the next undecided row");
+	MC2_REQUIRE(qb <= qe && qe <= g->end, w + ": the block must end at or before end");
+	const u64 P = g->n_parts;
+	std::vector<u64> h(3 * P);
+	u64 at = qb, stride = 0;
+	for (u64 p = 0; p < P; p++) {
+		MC2_REQUIRE(part_q_begin[p] == at && part_q_begin[p] <= part_q_end[p], w + ": the part ranges must tile [qb, qe) in part order");
+		MC2_REQUIRE(part_edges[p] <= g->cap, w + ": a part's edge count exceeds the part capacity");
+		at = part_q_end[p];
+		h[3 * p] = part_q_begin[p];
+		h[3 * p + 1] = part_q_end[p];
+		h[3 * p + 2] = part_edges[p];
+		stride = std::max<u64>(stride, part_edges[p]);
+	}
+	MC2_REQUIRE(at == qe, w + ": the part ranges must tile [qb, qe) in part order");
+	MC2_CUDA(cudaSetDevice(ctx->device));
+	if (qb == qe) return MC2_OK;
+	cudaStream_t st = ctx->stream;
+	u64 *d_part = (u64 *)g->part.p;
+	u32 *bad = (u32 *)(d_part + 3 * P);
+	GreedyParts src{(const GreedyEdge *)g->rec.p, g->both ? (const int8_t *)g->str.p : nullptr, d_part, P, stride, g->cap, g->begin,
+			g->end, bad};
+	const GreedyBlock &b = g->b;
+	const u64 rows = g->end - qb;
+	// The records came through the caller's exchange: the count pass checks every one before anything else is written, and
+	// a bad one leaves the object as it was.
+	MC2_CUDA(cudaMemcpyAsync(d_part, h.data(), P * 24, cudaMemcpyHostToDevice, st));
+	MC2_CUDA(cudaMemsetAsync(bad, 0, 4, st));
+	MC2_CUDA(cudaMemsetAsync(b.cnt, 0, rows * 4, st));
+	int rc = launch_greedy_parts_count(ctx, src, qb, b.cnt);
+	if (rc != MC2_OK) return rc;
+	MC2_CUDA(cudaMemcpyAsync(ctx->h_slot, bad, 4, cudaMemcpyDeviceToHost, st));
+	MC2_CUDA(cudaStreamSynchronize(st));
+	MC2_REQUIRE(*(u32 *)ctx->h_slot == 0, w + ": a part slot holds a record outside its part's query range or outside (r, end)");
+	src.bad = nullptr;
+	rc = greedy_block(ctx, b, qb, qe, [&](u64 n_rows) -> int {
+		int r = launch_seg_scan(ctx, b.cnt, n_rows, b.off);
+		if (r != MC2_OK) return r;
+		MC2_CUDA(cudaMemsetAsync(b.cnt, 0, n_rows * 4, st)); // now the scatter's cursors
+		return launch_greedy_parts_scatter(ctx, src, qb, b.off, b.cnt, b.bid, b.bd, b.bstr);
+	});
+	if (rc != MC2_OK) return rc;
+	// the slots are read: the caller may write the next block's records once this returns
+	MC2_CUDA(cudaStreamSynchronize(st));
+	g->next = qe;
+	return MC2_OK;
+}
+
+int mc2_greedy_end(mc2_ctx *ctx, mc2_greedy *g, uint64_t *out_rep, double *out_identity, int8_t *out_strand, uint64_t *n_clusters)
+{
+	const std::string w("mc2_greedy_end");
+	MC2_REQUIRE(ctx && g && out_rep && n_clusters, w + ": NULL argument");
+	MC2_REQUIRE(g->next == g->end, w + ": rows remain undecided: add the blocks up to end first");
+	MC2_CUDA(cudaSetDevice(ctx->device));
+	*n_clusters = 0;
+	const u64 n = g->end - g->begin;
+	if (n == 0) return MC2_OK;
+	return greedy_outputs(ctx, g->b.g, n, g->begin, (char *)g->out.p, out_rep, out_identity, out_strand, n_clusters);
 }
 
 int mc2_debug_last_sweep(mc2_ctx *ctx, uint64_t *n_exact, int32_t *coarse, uint64_t *n_inline)

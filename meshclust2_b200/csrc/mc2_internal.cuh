@@ -353,6 +353,26 @@ int launch_greedy_assign(mc2_ctx *ctx, const u64 *off, const double *bid, const 
 			 u64 begin, const GreedyRows &g);
 int launch_greedy_finish(mc2_ctx *ctx, const GreedyRows &g, u64 n, u64 begin, u64 *out_rep, double *out_id, int8_t *out_str,
 			 u64 *n_reps);
+// the part slots of a staged greedy clustering (mc2_greedy_*): slot p holds records rec[p * cap + j], j < its count, of edges
+// (begin + r, begin + c) with their identity, and with both strands a strand byte str[p * cap + j] (str NULL: one strand).
+// part[3 p .. 3 p + 2] = (query range begin, end, count) of part p; stride = the largest count.  bad (the count pass; NULL
+// in the scatter) is raised by a record with r outside its part's range or c outside (r, end).
+struct GreedyEdge {
+	u32 r, c;
+	double id;
+};
+struct GreedyParts {
+	const GreedyEdge *rec;
+	const int8_t *str;
+	const u64 *part;
+	u64 n_parts, stride, cap, begin, end;
+	u32 *bad;
+};
+int launch_greedy_parts_count(mc2_ctx *ctx, const GreedyParts &parts, u64 qb, u32 *cnt);
+int launch_greedy_parts_scatter(mc2_ctx *ctx, const GreedyParts &parts, u64 qb, const u64 *off, u32 *cur, double *bid, u64 *bd,
+				int8_t *bstr);
+// the first n survivors (sq, sd, ss) as records relative to begin
+int launch_greedy_pack(mc2_ctx *ctx, const u64 *sq, const u64 *sd, const double *ss, u64 n, u64 begin, GreedyEdge *out);
 int launch_merge_batch(mc2_ctx *ctx, const double *d_dist, const uint8_t *d_skipped, const uint8_t *d_close, const u64 *d_off,
 		       u64 n_centers, long long *d_out);
 

@@ -21,7 +21,9 @@
 // instantiation (STRAND = false) does the work it did before the strand existed.
 //
 // The count and scatter kernels also serve greedy clustering (greedy.cu), which buckets a block's edges by database row
-// (BY_D = true) and keeps the query row in the bucket; the top-K instantiations (BY_D = false) are unchanged.
+// (BY_D = true) and keeps the query row in the bucket; the top-K instantiations (BY_D = false) are unchanged.  Their edge
+// source is a template parameter: the sweep's flat survivor arrays, or the part slots of a staged greedy clustering, read
+// in place by one launch over every part.
 #include "mc2_internal.cuh"
 
 namespace mc2 {
@@ -29,37 +31,95 @@ namespace mc2 {
 static constexpr int kTopkThreads = 256;
 static constexpr u32 kTopkMaxK = 1024;
 
+// Edge sources of the count and scatter kernels: index i in [0, n) is an edge or nothing (has), with its query row q,
+// database row d, identity and strand (absolute rows).
+// the identity sweep's flat survivor arrays (count)
+struct FlatKeys {
+	const u64 *__restrict__ sq, *__restrict__ sd;
+	__device__ __forceinline__ bool has(u64) const { return true; }
+	__device__ __forceinline__ u64 q(u64 i) const { return sq[i]; }
+	__device__ __forceinline__ u64 d(u64 i) const { return sd[i]; }
+};
+
+// the same with identities and strands (scatter; sstr NULL: strand 1)
+struct FlatEdges {
+	const u64 *__restrict__ sq, *__restrict__ sd;
+	const double *__restrict__ ss;
+	const int8_t *__restrict__ sstr;
+	__device__ __forceinline__ bool has(u64) const { return true; }
+	__device__ __forceinline__ u64 q(u64 i) const { return sq[i]; }
+	__device__ __forceinline__ u64 d(u64 i) const { return sd[i]; }
+	__device__ __forceinline__ double id(u64 i) const { return ss[i]; }
+	__device__ __forceinline__ int8_t str(u64 i) const { return sstr ? sstr[i] : (int8_t)1; }
+};
+
+// the part slots of a staged greedy clustering (GreedyParts): i = p * stride + j is record j of slot p when j < its count.
+// With bad != NULL (the count pass) a record must have r in its part's query range and c in (r, end): any other raises *bad
+// and is skipped, so it never indexes a bucket.
+struct PartEdges {
+	GreedyParts s;
+	__device__ __forceinline__ u64 at(u64 i) const
+	{
+		const u64 p = i / s.stride;
+		return p * s.cap + (i - p * s.stride);
+	}
+	__device__ __forceinline__ bool has(u64 i) const
+	{
+		const u64 p = i / s.stride, j = i - p * s.stride;
+		const u64 *pp = s.part + 3 * p;
+		if (j >= pp[2]) {
+			return false;
+		}
+		if (s.bad) {
+			const u64 r = q(i), c = d(i);
+			if (!(r >= pp[0] && r < pp[1] && c > r && c < s.end)) {
+				*s.bad = 1;
+				return false;
+			}
+		}
+		return true;
+	}
+	__device__ __forceinline__ u64 q(u64 i) const { return s.begin + s.rec[at(i)].r; }
+	__device__ __forceinline__ u64 d(u64 i) const { return s.begin + s.rec[at(i)].c; }
+	__device__ __forceinline__ double id(u64 i) const { return s.rec[at(i)].id; }
+	__device__ __forceinline__ int8_t str(u64 i) const { return s.str[at(i)]; }
+};
+
 // survivors per bucket (self pairs dropped when asked); STRAND with fwd != NULL: only those with !(fwd[i] >= t).  The bucket
 // is the query row minus qb, or with BY_D (greedy.cu) the database row minus qb.
-template <bool STRAND, bool BY_D>
-__global__ void __launch_bounds__(256) topk_count_kernel(const u64 *__restrict__ sq, const u64 *__restrict__ sd, u64 n, u64 qb,
-							  int exclude_self, const double *__restrict__ fwd, double t, u32 *__restrict__ cnt)
+template <bool STRAND, bool BY_D, typename Src>
+__global__ void __launch_bounds__(256) topk_count_kernel(Src src, u64 n, u64 qb, int exclude_self, const double *__restrict__ fwd,
+							  double t, u32 *__restrict__ cnt)
 {
 	for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (u64)gridDim.x * blockDim.x) {
-		const u64 q = sq[i];
+		if (!src.has(i)) {
+			continue;
+		}
+		const u64 q = src.q(i);
 		if (STRAND && fwd && fwd[i] >= t) {
 			continue;
 		}
 		if (BY_D) {
-			atomicAdd(cnt + (sd[i] - qb), 1u);
-		} else if (!(exclude_self && sd[i] == q)) {
+			atomicAdd(cnt + (src.d(i) - qb), 1u);
+		} else if (!(exclude_self && src.d(i) == q)) {
 			atomicAdd(cnt + (q - qb), 1u);
 		}
 	}
 }
 
 // (identity, d) of each kept survivor into its query's bucket [off[q - qb], off[q - qb + 1]); cur (zeroed) is the fill cursor.
-// BY_D: (identity, q) into the bucket of d (no self pair to drop).  STRAND: also its strand into bstr, sstr[i] (sstr NULL: 1),
-// with the filter of topk_count_kernel
-template <bool STRAND, bool BY_D>
-__global__ void __launch_bounds__(256) topk_scatter_kernel(const u64 *__restrict__ sq, const u64 *__restrict__ sd,
-							    const double *__restrict__ ss, const int8_t *__restrict__ sstr,
-							    const double *__restrict__ fwd, double t, u64 n, u64 qb, int exclude_self,
-							    const u64 *__restrict__ off, u32 *__restrict__ cur, double *__restrict__ bid,
-							    u64 *__restrict__ bd, int8_t *__restrict__ bstr)
+// BY_D: (identity, q) into the bucket of d (no self pair to drop).  STRAND: also its strand into bstr, with the filter of
+// topk_count_kernel
+template <bool STRAND, bool BY_D, typename Src>
+__global__ void __launch_bounds__(256) topk_scatter_kernel(Src src, const double *__restrict__ fwd, double t, u64 n, u64 qb,
+							    int exclude_self, const u64 *__restrict__ off, u32 *__restrict__ cur,
+							    double *__restrict__ bid, u64 *__restrict__ bd, int8_t *__restrict__ bstr)
 {
 	for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (u64)gridDim.x * blockDim.x) {
-		const u64 q = sq[i], d = sd[i];
+		if (!src.has(i)) {
+			continue;
+		}
+		const u64 q = src.q(i), d = src.d(i);
 		if (STRAND && fwd && fwd[i] >= t) {
 			continue;
 		}
@@ -68,10 +128,10 @@ __global__ void __launch_bounds__(256) topk_scatter_kernel(const u64 *__restrict
 		}
 		const u64 key = BY_D ? d : q;
 		const u64 pos = off[key - qb] + atomicAdd(cur + (key - qb), 1u);
-		bid[pos] = ss[i];
+		bid[pos] = src.id(i);
 		bd[pos] = BY_D ? q : d;
 		if (STRAND) {
-			bstr[pos] = sstr ? sstr[i] : (int8_t)1;
+			bstr[pos] = src.str(i);
 		}
 	}
 }
@@ -272,9 +332,9 @@ int launch_topk_count(mc2_ctx *ctx, const u64 *sq, const u64 *sd, u64 n, u64 qb,
 		return MC2_OK;
 	}
 	if (by_d) {
-		topk_count_kernel<false, true><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, n, qb, 0, nullptr, 0.0, cnt);
+		topk_count_kernel<false, true><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(FlatKeys{sq, sd}, n, qb, 0, nullptr, 0.0, cnt);
 	} else {
-		topk_count_kernel<false, false><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, n, qb, exclude_self, nullptr,
+		topk_count_kernel<false, false><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(FlatKeys{sq, sd}, n, qb, exclude_self, nullptr,
 												    0.0, cnt);
 	}
 	ctx->launches++;
@@ -289,10 +349,10 @@ int launch_topk_scatter(mc2_ctx *ctx, const u64 *sq, const u64 *sd, const double
 		return MC2_OK;
 	}
 	if (by_d) {
-		topk_scatter_kernel<false, true><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, ss, nullptr, nullptr, 0.0, n,
+		topk_scatter_kernel<false, true><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(FlatEdges{sq, sd, ss, nullptr}, nullptr, 0.0, n,
 												      qb, 0, off, cur, bid, bd, nullptr);
 	} else {
-		topk_scatter_kernel<false, false><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, ss, nullptr, nullptr, 0.0, n,
+		topk_scatter_kernel<false, false><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(FlatEdges{sq, sd, ss, nullptr}, nullptr, 0.0, n,
 												       qb, exclude_self, off, cur, bid, bd,
 												       nullptr);
 	}
@@ -322,9 +382,9 @@ int launch_topk_count_strand(mc2_ctx *ctx, const u64 *sq, const u64 *sd, const d
 		return MC2_OK;
 	}
 	if (by_d) {
-		topk_count_kernel<true, true><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, n, qb, 0, fwd, t, cnt);
+		topk_count_kernel<true, true><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(FlatKeys{sq, sd}, n, qb, 0, fwd, t, cnt);
 	} else {
-		topk_count_kernel<true, false><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, n, qb, exclude_self, fwd, t,
+		topk_count_kernel<true, false><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(FlatKeys{sq, sd}, n, qb, exclude_self, fwd, t,
 												   cnt);
 	}
 	ctx->launches++;
@@ -340,10 +400,10 @@ int launch_topk_scatter_strand(mc2_ctx *ctx, const u64 *sq, const u64 *sd, const
 		return MC2_OK;
 	}
 	if (by_d) {
-		topk_scatter_kernel<true, true><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, ss, sstr, fwd, t, n, qb, 0,
+		topk_scatter_kernel<true, true><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(FlatEdges{sq, sd, ss, sstr}, fwd, t, n, qb, 0,
 												     off, cur, bid, bd, bstr);
 	} else {
-		topk_scatter_kernel<true, false><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(sq, sd, ss, sstr, fwd, t, n, qb,
+		topk_scatter_kernel<true, false><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(FlatEdges{sq, sd, ss, sstr}, fwd, t, n, qb,
 												      exclude_self, off, cur, bid, bd, bstr);
 	}
 	ctx->launches++;
@@ -361,6 +421,37 @@ int launch_topk_select_strand(mc2_ctx *ctx, const u64 *off, const double *bid, c
 	topk_select_kernel<true><<<grid_for(ctx, rows, 1, 8), kTopkThreads, 0, ctx->stream>>>(off, bid, bd, bstr, rows, k_best,
 												  d_begin, out_d, out_id, out_str,
 												  out_cnt, out_hits);
+	ctx->launches++;
+	MC2_CUDA(cudaGetLastError());
+	return MC2_OK;
+}
+
+int launch_greedy_parts_count(mc2_ctx *ctx, const GreedyParts &parts, u64 qb, u32 *cnt)
+{
+	const u64 n = parts.n_parts * parts.stride;
+	if (n == 0) {
+		return MC2_OK;
+	}
+	topk_count_kernel<false, true><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(PartEdges{parts}, n, qb, 0, nullptr, 0.0, cnt);
+	ctx->launches++;
+	MC2_CUDA(cudaGetLastError());
+	return MC2_OK;
+}
+
+int launch_greedy_parts_scatter(mc2_ctx *ctx, const GreedyParts &parts, u64 qb, const u64 *off, u32 *cur, double *bid, u64 *bd,
+				int8_t *bstr)
+{
+	const u64 n = parts.n_parts * parts.stride;
+	if (n == 0) {
+		return MC2_OK;
+	}
+	if (parts.str) {
+		topk_scatter_kernel<true, true><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(PartEdges{parts}, nullptr, 0.0, n, qb, 0,
+												     off, cur, bid, bd, bstr);
+	} else {
+		topk_scatter_kernel<false, true><<<grid_for(ctx, n, 256, 8), 256, 0, ctx->stream>>>(PartEdges{parts}, nullptr, 0.0, n, qb,
+												      0, off, cur, bid, bd, nullptr);
+	}
 	ctx->launches++;
 	MC2_CUDA(cudaGetLastError());
 	return MC2_OK;

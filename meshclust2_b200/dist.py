@@ -32,22 +32,19 @@ def folded_row_blocks(n, world, rank, blocks_per_rank=8):
     return sorted(out)
 
 
-def triangle_row_blocks(n, world, rank, blocks_per_rank=1, row_overhead=160):
-    """Query-row blocks of an upper-triangular sweep for `rank`: CONTIGUOUS row ranges of equal cost (so they get longer
-    towards the end of the set), `blocks_per_rank` of them per rank.  Row q costs its n - 1 - q pairs plus `row_overhead`
-    pair slots: the tile kernel pays whole 64 x 256 tiles along the diagonal (about half a tile width + half a tile height
-    of unused slots per query row), which would otherwise make the last rank, whose range is mostly diagonal, the slowest.
-    One range per rank means one sweep launch per rank and step: every launch pays a tail of up to one tile per SM."""
-    B = max(1, world * blocks_per_rank)
+def block_shares(qb, qe, end, world, row_overhead=160):
+    """`world` CONTIGUOUS shares of query rows [qb, qe) of an upper-triangular sweep over columns up to `end`, of equal
+    cost, in row order; they tile [qb, qe) and may be empty.  Row q costs its end - 1 - q pairs plus `row_overhead` pair
+    slots: the tile kernel pays whole 64 x 256 tiles along the diagonal (about half a tile width + half a tile height of
+    unused slots per query row), which would otherwise make the share that is mostly diagonal the slowest."""
+    def cost(x):                                    # rows [qb, x)
+        return (x - qb) * (end - 1 + row_overhead) - (x * (x - 1) - qb * (qb - 1)) // 2
 
-    def cost(x):                                    # rows [0, x)
-        return x * (n - 1) - x * (x - 1) // 2 + row_overhead * x
-
-    total = cost(n)
-    edges = [0]
-    for j in range(1, B):
-        target = total * j // B
-        lo, hi = edges[-1], n
+    total = cost(qe)
+    edges = [qb]
+    for j in range(1, world):
+        target = total * j // world
+        lo, hi = edges[-1], qe
         while lo < hi:                              # smallest x with cost(rows < x) >= target
             mid = (lo + hi) // 2
             if cost(mid) >= target:
@@ -55,13 +52,16 @@ def triangle_row_blocks(n, world, rank, blocks_per_rank=1, row_overhead=160):
             else:
                 lo = mid + 1
         edges.append(lo)
-    edges.append(n)
-    out = []
-    for b in range(rank * blocks_per_rank, (rank + 1) * blocks_per_rank):
-        q0, q1 = edges[b], edges[b + 1]
-        if q1 > q0:
-            out.append((q0, q1))
-    return out
+    edges.append(qe)
+    return [(edges[p], edges[p + 1]) for p in range(world)]
+
+
+def triangle_row_blocks(n, world, rank, blocks_per_rank=1, row_overhead=160):
+    """Query-row blocks of an upper-triangular sweep for `rank`: CONTIGUOUS row ranges of equal cost (block_shares of the
+    whole set, so they get longer towards the end of the set), `blocks_per_rank` of them per rank.  One range per rank
+    means one sweep launch per rank and step: every launch pays a tail of up to one tile per SM."""
+    shares = block_shares(0, n, n, max(1, world * blocks_per_rank), row_overhead)
+    return [(q0, q1) for q0, q1 in shares[rank * blocks_per_rank:(rank + 1) * blocks_per_rank] if q1 > q0]
 
 
 def rect_row_blocks(n, world, rank):
@@ -148,7 +148,7 @@ class Comm:
 
 
 def all_pairs_step(engine, comm, torch, n_total, cutoff, upper_only=True, blocks_per_rank=1, max_out=1 << 20, identity=None,
-                   top_k=None, components=False):
+                   top_k=None, components=False, greedy=False):
     """One pass of the hot path over a batch: local K1 -> all-gather -> row-block K2 sweep.
 
     identity: None sweeps with the engine's classifier; (regression model, min_identity) makes it an identity search
@@ -179,12 +179,22 @@ def all_pairs_step(engine, comm, torch, n_total, cutoff, upper_only=True, blocks
                                     (optional: an engine without it takes no both-strand top_k)
     engine.components(q0, q1, cutoff, identity) -> dict(label [n_total], n_components, n_scored)   (optional)
     engine.merge_components(labels [parts, n_total]) -> dict(label [n_total], n_components)
+    engine.greedy_begin(cutoff, identity, n_parts) -> part capacity (edges per slot)    (optional, as the four below)
+    engine.greedy_sweep_part(part, q0, q1) -> (n_edges, n_scored)   slot `part` holds the edges when n_edges <= capacity
+    engine.greedy_gather(comm, most)    every rank's slot `rank` into slot `rank` of every rank (first `most` edges)
+    engine.greedy_add_block(qb, qe, shares, counts)
+    engine.greedy_end() -> dict(rep [n_total], identity, strand, n_clusters)
     Returns dict(n_scored, n_close, survivors (this rank's), topk (this rank's, [] without top_k), blocks, components (None
-    without components))."""
+    without components), greedy (None without greedy))."""
     both_strands = identity is not None and len(identity) > 2 and bool(identity[2])
     if components and (identity is None or not upper_only or top_k is not None or not hasattr(engine, "components")):
         raise ValueError("components needs an identity search over the upper triangle (identity=(regression model, "
                          "min_identity[, both_strands]), upper_only=True), no top_k, and an engine with components")
+    if greedy and (identity is None or not upper_only or top_k is not None or components
+                   or not hasattr(engine, "greedy_begin")):
+        raise ValueError("greedy needs an identity search over the upper triangle (identity=(regression model, "
+                         "min_identity[, both_strands]), upper_only=True), no top_k, no components, and an engine with "
+                         "greedy_begin")
     if top_k is not None and (identity is None or (both_strands and not hasattr(engine, "topk_both_strands"))):
         raise ValueError("top_k needs a one-strand identity search: identity=(regression model, min_identity), or an "
                          "engine with topk_both_strands for identity=(regression model, min_identity, True)")
@@ -208,6 +218,11 @@ def all_pairs_step(engine, comm, torch, n_total, cutoff, upper_only=True, blocks
             idx = torch.as_tensor(keep, device=bins.device)
             bins, length, mag = bins[idx].contiguous(), length[idx].contiguous(), mag[idx].contiguous()
         engine.install_full(bins, length, mag, n_total)
+    if greedy:
+        gr, blocks, n_scored, n_close = _greedy_blocks(engine, comm, torch, n_total, cutoff, identity)
+        tot_scored, = comm.all_reduce_sum([n_scored], torch, engine.device)
+        return dict(n_scored=tot_scored, n_close=n_close, local_scored=n_scored, local_close=n_close, survivors=Survivors(),
+                    topk=[], blocks=blocks, components=None, greedy=gr)
     blocks = (triangle_row_blocks(n_total, comm.world, comm.rank, blocks_per_rank) if upper_only
               else rect_row_blocks(n_total, comm.world, comm.rank))
     n_scored = n_close = 0
@@ -249,7 +264,40 @@ def all_pairs_step(engine, comm, torch, n_total, cutoff, upper_only=True, blocks
         comp = dict(label=comp["label"], n_components=comp["n_components"])
     tot_scored, tot_close = comm.all_reduce_sum([n_scored, n_close], torch, engine.device)
     return dict(n_scored=tot_scored, n_close=tot_close, local_scored=n_scored, local_close=n_close, survivors=surv, topk=tables,
-                blocks=blocks, components=comp)
+                blocks=blocks, components=comp, greedy=None)
+
+
+def _greedy_blocks(engine, comm, torch, n_total, cutoff, identity):
+    """The block-synchronous greedy clustering of all_pairs_step(greedy=True) -> (result, blocks, this rank's n_scored,
+    edge count).  Blocks grow and shrink as the single-GPU call's do: the first is the whole set, a block that overflows a
+    slot is swept again at about half a slot's worth of edges, and a block whose fullest slot is under a quarter full
+    doubles the next one."""
+    world, rank = comm.world, comm.rank
+    cap = engine.greedy_begin(cutoff, identity, world)
+    qb, rows = 0, n_total
+    n_scored = n_close = 0
+    blocks = []
+    while qb < n_total:
+        qe = qb + min(rows, n_total - qb)
+        shares = block_shares(qb, qe, n_total, world)
+        ne, ns = engine.greedy_sweep_part(rank, *shares[rank])
+        mine = [0] * world
+        mine[rank] = ne
+        counts = comm.all_reduce_sum(mine, torch, engine.device)
+        most = max(counts)
+        if most > cap:                              # one row always fits: cap >= n_total
+            span = qe - qb
+            rows = max(1, min(span // 2, int(float(span) * float(cap // 2) / float(most))))
+            continue
+        engine.greedy_gather(comm, most)
+        engine.greedy_add_block(qb, qe, shares, counts)
+        n_scored += ns
+        n_close += sum(counts)
+        blocks.append((qb, qe))
+        qb = qe
+        if most < cap // 4:
+            rows = min(rows * 2, n_total)
+    return engine.greedy_end(), blocks, n_scored, n_close
 
 
 def candidate_scan(engine, comm, torch, q_global, n_total, cutoff):
@@ -572,6 +620,49 @@ class GpuEngine:
     def merge_components(self, labels):
         """the union of the partitions in the rows of labels (Context.components_merge) -> dict(label, n_components)"""
         return self.ctx.components_merge(labels, 0)
+
+    # ---- staged greedy clustering (all_pairs_step(greedy=True)) ----
+    def greedy_begin(self, cutoff, identity, n_parts):
+        """a staged greedy clustering of the whole set with n_parts slots (Context.greedy_begin) -> slot capacity"""
+        torch = self.torch
+        self.greedy_free()
+        model, t = identity[:2]
+        nd = min(len(self.full), getattr(self, "n_total", None) or len(self.full))   # rows past n_total are shard padding
+        g = self._greedy = self.ctx.greedy_begin(model, self.full, t, cutoff, both_strands=len(identity) > 2 and bool(identity[2]),
+                                                 range=(0, nd), n_parts=n_parts)
+        arrays = [g.part_arrays(p) for p in range(n_parts)]
+        self._greedy_rec = [torch.as_tensor(a["records"], device=self.device) for a in arrays]
+        self._greedy_str = [torch.as_tensor(a["strand"], device=self.device) for a in arrays if a["strand"] is not None]
+        return arrays[0]["capacity"]
+
+    def greedy_sweep_part(self, part, q0, q1):
+        """returns after the context's stream has written the slot, so a collective may read it"""
+        return self._greedy.sweep_part(part, q0, q1)
+
+    def greedy_gather(self, comm, most):
+        """slot r of every rank <- slot r of rank r, the first `most` records (and strand bytes)"""
+        if comm.dist is None or most == 0:
+            return
+        for slots in (self._greedy_rec, self._greedy_str):
+            if slots:
+                views = [s[:most] for s in slots]
+                comm.dist.all_gather(views, views[comm.rank])
+
+    def greedy_add_block(self, qb, qe, shares, counts):
+        self.torch.cuda.synchronize(self.device)        # the gather ran on torch's streams; the resolve's CTAs must all be resident
+        self._greedy.add_block(qb, qe, shares, counts)
+
+    def greedy_end(self):
+        r = self._greedy.end()
+        self.greedy_free()
+        return r
+
+    def greedy_free(self):
+        g = getattr(self, "_greedy", None)
+        if g is not None:
+            self._greedy_rec = self._greedy_str = None
+            g.free()
+            self._greedy = None
 
     def sweep(self, q0, q1, upper_only, cutoff, max_out, identity=None):
         """identity: None = the engine's classifier (all_pairs), else (regression model, min_identity) (identity_pairs) or
